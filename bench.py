@@ -3,6 +3,7 @@
 recombined per second, N -> n at d = 10).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling weak|strong]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one full pass of the hot path over one batch of synthetic candidates: Nystrom basis of
@@ -19,6 +20,9 @@ host<->device copies; `iteration` times one BASQ iteration with the candidates d
 `extra` (N = 1 only) times the other BASELINE configurations and the config-5 acquisition pass.
 `--impl reference` times the CPU oracle port of the reference's algorithm on a bounded sample (the
 reference is pure Python over gpytorch and does not ship to the GPU box).
+`--dump-outputs DIR` writes the quadrature rule the last timed `value` step returned (global candidate
+indices and weights) as DIR/indices.npy and DIR/weights.npy, both float64; the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -59,7 +63,21 @@ def parse():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-extra", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the last timed step's rule as DIR/indices.npy and DIR/weights.npy (float64)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
+
+
+def dump_outputs(out_dir, idx, w):
+    """The rule a caller of the timed path receives: candidate indices (exact in float64) and weights."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "indices.npy"), idx.cpu().to(torch.float64).numpy())
+    np.save(os.path.join(out_dir, "weights.npy"), w.cpu().to(torch.float64).numpy())
 
 
 # ------------------------------------------------------------------------------------------ workload
@@ -527,6 +545,8 @@ def run_ours(a, rank, world, local_rank):
     idx, w = out
     assert 1 <= len(idx) <= a.n and bool((w > 0).all()), "invalid quadrature rule"
     assert abs(float(w.sum()) - 1.0) < 1e-9, float(w.sum())
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, idx, w)
     value = N_glob / (ms_step * 1e-3)
 
     e2e = None

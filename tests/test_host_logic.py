@@ -192,3 +192,14 @@ def test_bench_reference_arm_uses_all_threads_under_torchrun_env():
     env["RANK"] = "1"
     out = subprocess.run(args, capture_output=True, text=True, timeout=300, cwd=root, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_bench_rejects_zero_steps():
+    """--steps is the number of timed steps: zero would leave nothing to time."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=300, cwd=root)
+    assert out.returncode == 2 and "--steps" in out.stderr
