@@ -57,6 +57,8 @@ def _load():
         "basq_ctx_profile_read": (I, [P, C.POINTER(D), C.POINTER(L), I]),
         "basq_gram": (I, [P, KD, P, L, P, L, P]),
         "basq_gp_predict": (I, [P, KD, P, L, I, D, P, P]),
+        "basq_kernel_quadform": (I, [P, KD, P, L, P, C.POINTER(D)]),
+        "basq_kernel_bilinear": (I, [P, KD, P, L, P, P, L, P, C.POINTER(D)]),
         "basq_ctx_stage_candidates": (I, [P, P, L, I, I, P]),
         "basq_session_create_staged": (I, [P, KD, L, L, L, P, L, P, I, C.POINTER(P)]),
         "basq_nystrom_basis_sharded": (I, [P, KD, P, L, I, P, I, I, I, P, P, P, P, P]),

@@ -116,6 +116,24 @@ __global__ void row_l1_max_kernel(const double* __restrict__ A, int rows, int co
   if (threadIdx.x == 0) atomicMax(out, (unsigned long long)__double_as_longlong(sh[0]));
 }
 
+}  // namespace
+
+int narrow_f64(basq_ctx* ctx, const double* in, int64_t n, float* out) {
+  f64_to_f32_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(in, n, out);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+int widen_f32(basq_ctx* ctx, const float* in, int64_t n, double* out) {
+  f32_to_f64_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(in, n, out);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+namespace {
+
 int check_finite_host(const double* v, int64_t n, const char* what) {
   for (int64_t i = 0; i < n; ++i)
     BASQ_CHECK(isfinite(v[i]), BASQ_ERR_NUMERIC, "%s contains a non-finite value at %lld", what, (long long)i);
@@ -161,13 +179,10 @@ struct basq_session {
   DevBuf raw[2];    // [n, S] unscaled local columns of the current / previous level
   int raw_cur = 0;
   DevBuf lnode, lppos, lfpar;  // device copies of a level's node ids, parent positions, parent factors
-  DevBuf V, corrT;  // chunk buffers of the non-linear modes
-  int64_t chunkP = 0;
+  NlSweep nls;      // set sums of the non-linear modes (tensor-core operands or chunk buffers)
   // fp32 inputs whose posterior correction would amplify the fp32 kernel noise beyond tolerance are
   // promoted to the all-fp64 path (session_create_impl): fp64 copies of the inputs live here
   DevBuf X64, Z64, Xobs64;
-  NlOperands nlop;  // tensor-core path of the non-linear modes (fp32 records)
-  bool use_nls = false;
   bool promoted = false;
   double kappa = 0.0;
   int64_t idx_base = 0;
@@ -204,28 +219,92 @@ int session_set_sums(basq_session* s, int64_t off, int S, int64_t p_lo, int64_t 
     a.accumulate = false;
     return set_sums(ctx, s->kp, a);
   }
-  if (s->use_nls)
-    return nls_set_sums(ctx, s->kp, s->nl, &s->nlop, s->pool, s->lm.view(), s->lmobs.view(), off, S, p_lo, p_hi, G, ldg);
-  // non-linear kernels need C_h(z_m, x_p) = k(z_m, x_p) - (K_ZX W) k(Xobs, x_p) per pair: build the
-  // correction for a chunk of points with two GEMM-shaped steps, then accumulate.
-  const int n_obs = s->desc.n_obs;
-  BASQ_CUDA(cudaMemsetAsync(G, 0, sizeof(double) * (size_t)s->Mtot * ldg, ctx->stream));
-  for (int64_t c0 = p_lo; c0 < p_hi; c0 += s->chunkP) {
-    const int64_t c1 = std::min(p_hi, c0 + s->chunkP);
-    const int64_t cnt = c1 - c0;
-    BASQ_TRY(base_gram_records(ctx, s->kp, s->lmobs.view(), s->pool, c0, c1, s->V.as<double>(), s->chunkP));
-    // corrT[p, m] = sum_o V[o, p] * Az[m, o]
-    BASQ_TRY(dgemm(ctx, true, true, (int)cnt, s->M, n_obs, 1.0, s->V.as<double>(), s->chunkP, s->Az.as<double>(),
-                   n_obs, 0.0, s->corrT.as<double>(), s->M));
-    a.p_lo = c0;
-    a.p_hi = c1;
-    a.corrT = s->corrT.as<double>();
-    a.ld_corr = s->M;
-    a.accumulate = true;
-    BASQ_TRY(set_sums(ctx, s->kp, a));
+  return nl_sweep_sums(ctx, s->kp, s->nl, &s->nls, s->pool, s->lm.view(), s->lmobs.view(), off, S, p_lo, p_hi, G, ldg,
+                       &a);
+}
+
+}  // namespace
+
+// Az = K(Z, Xobs) W   (BASQ/_gp.py:270-273: KxX @ woodbury_inv) and the conditioning guard's measure.  The
+// correction K_ZX W k(Xobs, x) multiplies the kernel values by the rows of Az, so an evaluation error eps_k of
+// k (fp32: ~2e-7 relative) reaches the covariance as eps_k |Az_m|_1 sigma_f^2.  kappa = max_m |Az_m|_1 is
+// O(10) for well-separated observations even at the reference's default noise 1e-10 (BASQ/_parameters.py:30),
+// but grows like sigma_f / sigma_n for clustered ones; beyond kappa_max the fp32 inputs are promoted to the
+// all-fp64 path.
+int posterior_az(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const LmView& lmz, double* Az,
+                 double* kappa) {
+  const int M = lmz.count, n_obs = desc->n_obs;
+  DevBuf KzX, kap;
+  BASQ_TRY(KzX.alloc(ctx, sizeof(double) * (size_t)M * n_obs));
+  BASQ_TRY(base_gram(ctx, kp, lmz, desc->Xobs, n_obs, KzX.as<double>(), n_obs));
+  BASQ_TRY(dgemm(ctx, false, false, M, n_obs, n_obs, 1.0, KzX.as<double>(), n_obs, desc->W, n_obs, 0.0, Az, n_obs));
+  BASQ_TRY(kap.alloc(ctx, sizeof(unsigned long long)));
+  BASQ_CUDA(cudaMemsetAsync(kap.p, 0, sizeof(unsigned long long), ctx->stream));
+  row_l1_max_kernel<<<(unsigned)M, 256, 0, ctx->stream>>>(Az, M, n_obs, kap.as<unsigned long long>());
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  BASQ_CUDA(cudaMemcpyAsync(kappa, kap.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));  // also: KzX goes out of scope
+  BASQ_CHECK(isfinite(*kappa), BASQ_ERR_NUMERIC, "the GP caches contain non-finite values (K_ZX W)");
+  ctx->last_kappa = *kappa;
+  return BASQ_OK;
+}
+
+// Non-linear modes: fp32 records run on the tensor cores (nlsum.cuh, operands from Az); otherwise the
+// correction is built per chunk of points, whose size is chosen here for N_loc points.  Az stays the caller's
+// and must outlive the sweeps on the chunked path.
+int nl_sweep_prepare(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const double* Az, int M,
+                     const double* sz, int64_t N_loc, NlSweep* w) {
+  const int n_obs = desc->n_obs;
+  { const char* t = getenv("BASQ_NLSUM"); ctx->no_nlsum = t && t[0] == '0'; }  // read per call (A/B tests toggle it)
+  w->M = M;
+  w->Az = Az;
+  w->use_nls = desc->dtype == BASQ_F32 && !ctx->no_nlsum;
+  if (w->use_nls) {
+    // fp32 records: the pairwise correction runs on the tensor cores (nlsum.cuh)
+    BASQ_TRY(nls_prepare(ctx, kp, Az, M, n_obs, sz, &w->nlop));
+    w->Az = nullptr;
+  } else {
+    // points per chunk of the pairwise correction: corrT [P, M] may take up to 2 GB, so that a chunk
+    // spans many cells of a refined pass (every chunk re-reads the G columns it touches)
+    int64_t P = (int64_t)(2048ll << 20) / (8ll * std::max<int64_t>(M, n_obs));
+    P = std::max<int64_t>(1024, std::min<int64_t>(P, 131072));
+    P = std::min<int64_t>(P, std::max<int64_t>(N_loc, 1024));
+    w->chunkP = P;
+    BASQ_TRY(w->V.alloc(ctx, sizeof(double) * (size_t)n_obs * P));
+    BASQ_TRY(w->corrT.alloc(ctx, sizeof(double) * (size_t)M * P));
   }
   return BASQ_OK;
 }
+
+// G[:, 0..S) of the non-linear set sums of local records [p_lo, p_hi); a = the set-sum arguments of the linear
+// fields (pool, landmarks, offset, sets, G, sz), completed here per chunk.
+int nl_sweep_sums(basq_ctx* ctx, const KParams& kp, int nl, NlSweep* w, const RecPool& pool, const LmView& lmz,
+                  const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg,
+                  SetSumArgs* a) {
+  if (w->use_nls) return nls_set_sums(ctx, kp, nl, &w->nlop, pool, lmz, lmobs, off, S, p_lo, p_hi, G, ldg);
+  // non-linear kernels need C_h(z_m, x_p) = k(z_m, x_p) - (K_ZX W) k(Xobs, x_p) per pair: build the
+  // correction for a chunk of points with two GEMM-shaped steps, then accumulate.
+  const int n_obs = lmobs.count;
+  BASQ_CUDA(cudaMemsetAsync(G, 0, sizeof(double) * (size_t)lmz.count * ldg, ctx->stream));
+  for (int64_t c0 = p_lo; c0 < p_hi; c0 += w->chunkP) {
+    const int64_t c1 = std::min(p_hi, c0 + w->chunkP);
+    const int64_t cnt = c1 - c0;
+    BASQ_TRY(base_gram_records(ctx, kp, lmobs, pool, c0, c1, w->V.as<double>(), w->chunkP));
+    // corrT[p, m] = sum_o V[o, p] * Az[m, o]
+    BASQ_TRY(dgemm(ctx, true, true, (int)cnt, w->M, n_obs, 1.0, w->V.as<double>(), w->chunkP, w->Az, n_obs, 0.0,
+                   w->corrT.as<double>(), w->M));
+    a->p_lo = c0;
+    a->p_hi = c1;
+    a->corrT = w->corrT.as<double>();
+    a->ld_corr = w->M;
+    a->accumulate = true;
+    BASQ_TRY(set_sums(ctx, kp, *a));
+  }
+  return BASQ_OK;
+}
+
+namespace {
 
 int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N_loc, int64_t N_glob,
                         int64_t idx_base, const void* Z, int64_t M, const double* U, int q, const double* mu,
@@ -243,12 +322,7 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
     const int d = desc->d;
     auto narrow = [&](const void* src, int64_t rows, DevBuf* dst) -> int {
       BASQ_TRY(dst->alloc(ctx, sizeof(float) * (size_t)std::max<int64_t>(rows, 1) * d));
-      if (rows > 0) {
-        f64_to_f32_kernel<<<(unsigned)ceil_div64(rows * d, 256), 256, 0, ctx->stream>>>((const double*)src, rows * d,
-                                                                                         dst->as<float>());
-        ctx->launches++;
-        BASQ_CUDA(cudaGetLastError());
-      }
+      if (rows > 0) BASQ_TRY(narrow_f64(ctx, (const double*)src, rows * d, dst->as<float>()));
       return BASQ_OK;
     };
     BASQ_TRY(narrow(X, N_loc, &s->X32));
@@ -286,39 +360,14 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
   s->Mtot = s->lm.count;
 
   if (mode != BASQ_PLAIN) {
-    // Az = K(Z, Xobs) W   (BASQ/_gp.py:270-273: KxX @ woodbury_inv)
-    DevBuf KzX, kap;
-    BASQ_TRY(KzX.alloc(ctx, sizeof(double) * (size_t)M * n_obs));
     BASQ_TRY(s->Az.alloc(ctx, sizeof(double) * (size_t)M * n_obs));
-    BASQ_TRY(base_gram(ctx, s->kp, s->lm.view(0, (int)M), desc->Xobs, n_obs, KzX.as<double>(), n_obs));
-    BASQ_TRY(dgemm(ctx, false, false, (int)M, n_obs, n_obs, 1.0, KzX.as<double>(), n_obs, desc->W, n_obs, 0.0,
-                   s->Az.as<double>(), n_obs));
-    // Conditioning guard.  The correction K_ZX W k(Xobs, x) multiplies the kernel values by the rows of
-    // Az, so an evaluation error eps_k of k (fp32: ~2e-7 relative) reaches the covariance as
-    // eps_k |Az_m|_1 sigma_f^2.  kappa = max_m |Az_m|_1 is O(10) for well-separated observations even at
-    // the reference's default noise 1e-10 (BASQ/_parameters.py:30), but grows like sigma_f / sigma_n for
-    // clustered ones; beyond kappa_max the fp32 inputs are promoted to the all-fp64 path.
-    BASQ_TRY(kap.alloc(ctx, sizeof(unsigned long long)));
-    BASQ_CUDA(cudaMemsetAsync(kap.p, 0, sizeof(unsigned long long), ctx->stream));
-    row_l1_max_kernel<<<(unsigned)M, 256, 0, ctx->stream>>>(s->Az.as<double>(), (int)M, n_obs,
-                                                            kap.as<unsigned long long>());
-    ctx->launches++;
-    BASQ_CUDA(cudaGetLastError());
-    BASQ_CUDA(cudaMemcpyAsync(&s->kappa, kap.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    BASQ_CUDA(cudaStreamSynchronize(ctx->stream));  // also: KzX goes out of scope
-    BASQ_CHECK(isfinite(s->kappa), BASQ_ERR_NUMERIC, "the GP caches contain non-finite values (K_ZX W)");
-    ctx->last_kappa = s->kappa;
+    BASQ_TRY(posterior_az(ctx, desc, s->kp, s->lm.view(0, (int)M), s->Az.as<double>(), &s->kappa));
     if (desc->dtype == BASQ_F32 && ctx->kappa_max > 0.0 && s->kappa > ctx->kappa_max) {
       // promote: fp64 copies of X, Z, Xobs, then the same construction with dtype = F64
       const int d = desc->d;
       auto widen = [&](const void* src, int64_t rows, DevBuf* dst) -> int {
         BASQ_TRY(dst->alloc(ctx, sizeof(double) * (size_t)std::max<int64_t>(rows, 1) * d));
-        if (rows > 0) {
-          f32_to_f64_kernel<<<(unsigned)ceil_div64(rows * d, 256), 256, 0, ctx->stream>>>((const float*)src, rows * d,
-                                                                                           dst->as<double>());
-          ctx->launches++;
-          BASQ_CUDA(cudaGetLastError());
-        }
+        if (rows > 0) BASQ_TRY(widen_f32(ctx, (const float*)src, rows * d, dst->as<double>()));
         return BASQ_OK;
       };
       if (s->demoted) {   // the caller's arrays were fp64 to begin with: go back to them
@@ -388,21 +437,9 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
                          !nonlin, &s->pool));
 
   s->ldg = 0;  // G and the rank table are sized by the first pass (session_reserve_cells)
-  { const char* t = getenv("BASQ_NLSUM"); ctx->no_nlsum = t && t[0] == '0'; }  // read per session (A/B tests toggle it)
-  s->use_nls = nonlin && desc->dtype == BASQ_F32 && !ctx->no_nlsum;
-  if (s->use_nls) {
-    // fp32 records: the pairwise correction runs on the tensor cores (nlsum.cuh)
-    BASQ_TRY(nls_prepare(ctx, s->kp, s->Az.as<double>(), (int)M, n_obs, s->sz.as<double>(), &s->nlop));
-    s->Az.release();
-  } else if (nonlin) {
-    // points per chunk of the pairwise correction: corrT [P, M] may take up to 2 GB, so that a chunk
-    // spans many cells of a refined pass (every chunk re-reads the G columns it touches)
-    int64_t P = (int64_t)(2048ll << 20) / (8ll * std::max<int64_t>(M, n_obs));
-    P = std::max<int64_t>(1024, std::min<int64_t>(P, 131072));
-    P = std::min<int64_t>(P, std::max<int64_t>(N_loc, 1024));
-    s->chunkP = P;
-    BASQ_TRY(s->V.alloc(ctx, sizeof(double) * (size_t)n_obs * P));
-    BASQ_TRY(s->corrT.alloc(ctx, sizeof(double) * (size_t)M * P));
+  if (nonlin) {
+    BASQ_TRY(nl_sweep_prepare(ctx, desc, s->kp, s->Az.as<double>(), (int)M, s->sz.as<double>(), N_loc, &s->nls));
+    if (s->nls.use_nls) s->Az.release();
   }
   BASQ_CUDA(cudaStreamSynchronize(ctx->stream));  // sx goes out of scope
   return BASQ_OK;

@@ -450,6 +450,8 @@ int base_gram_records(basq_ctx* ctx, const KParams& kp, const LmView& lm, const 
 // mean_out[N] = c0 + sum_o coef[o] k(lm_o, x)   (fp64 accumulation)
 int landmark_dot(basq_ctx* ctx, const KParams& kp, const LmView& lm, const double* coef, double c0,
                  const void* P, int64_t N, double* out);
+// out[p] = c0 + sum_{j < cols} G[p, j]   (p < n; fixed order)
+int rowsum_cols(basq_ctx* ctx, const double* G, int64_t n, int cols, double c0, double* out);
 int gp_predict_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const LmView& lmobs,
                     const void* X, int64_t N, double* mean_out, double* var_out);
 // per-point / per-landmark factor of the warped kernels (m(x) or mu_g(x)); out == nullptr allowed
@@ -466,8 +468,10 @@ struct RecPool {
   int64_t count = 0;
   int64_t capacity = 0;
 };
+// round_buffer: also allocate the second buffer that apply_round compacts into (recombination only)
 int build_records(basq_ctx* ctx, const KParams& kp, int dtype, const void* X, int64_t N, double uniform_w,
-                  const double* mu, const double* factor, bool factor_in_weight, RecPool* pool);
+                  const double* mu, const double* factor, bool factor_in_weight, RecPool* pool,
+                  bool round_buffer = true);
 int set_masses(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, double* mass_out);
 int cell_objective(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, const double* obj,
                    double* out);
@@ -527,6 +531,29 @@ int caratheodory(basq_ctx* ctx, double* A, int n, int S, int lda, double* omega_
 // (noise, jitter) then sit at (i, diag_col0 + i)
 int gram_matrix(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t a, const void* Y, int64_t b,
                 double* out, bool tensor_correction, int64_t diag_col0 = 0);
+// out[n] (fp32) = in[n] (fp64), rounded to nearest
+int narrow_f64(basq_ctx* ctx, const double* in, int64_t n, float* out);
+int widen_f32(basq_ctx* ctx, const float* in, int64_t n, double* out);
+// Landmark side of the posterior modes, shared by sessions and the weighted double sums (quadform.cu):
+// Az[M, n_obs] = K(Z, Xobs) W for the prepared landmarks lmz (M = lmz.count) and the conditioning guard's
+// kappa = max_m |Az_m|_1 (also stored in ctx->last_kappa; synchronises)
+int posterior_az(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const LmView& lmz, double* Az,
+                 double* kappa);
+// set sums of the pairwise non-linear modes (WSABI-M, MMLT) against landmarks with Az and factors sz
+struct NlSweep {
+  int M = 0;
+  bool use_nls = false;   // fp32 records: tensor-core operands (nlsum.cuh); else the chunked fp64-GEMM correction
+  NlOperands nlop;
+  const double* Az = nullptr;   // chunked path: the caller's Az, alive while sweeping
+  DevBuf V, corrT;              // chunked path: k(Xobs, x) and the correction of a chunk of points
+  int64_t chunkP = 0;
+};
+int nl_sweep_prepare(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const double* Az, int M,
+                     const double* sz, int64_t N_loc, NlSweep* w);
+// G[:, 0..S) for local records [p_lo, p_hi); a carries pool, landmarks, offset, S, nl, sz, G, ldg
+int nl_sweep_sums(basq_ctx* ctx, const KParams& kp, int nl, NlSweep* w, const RecPool& pool, const LmView& lmz,
+                  const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg,
+                  SetSumArgs* a);
 
 // nystrom.cu
 // out[rows, cols] fp64 N(0, 1) draws of the Philox stream `seed` (candidates.cu)

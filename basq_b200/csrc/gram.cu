@@ -262,6 +262,13 @@ __global__ void rowsum_cols_kernel(const double* __restrict__ G, int64_t n, int 
   out[p] = c0 + s;
 }
 
+int rowsum_cols(basq_ctx* ctx, const double* G, int64_t n, int cols, double c0, double* out) {
+  rowsum_cols_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(G, n, cols, c0, out);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
 // The same sum on the tensor-core set-sum kernel (setsum_mma.cuh) with the roles swapped: the N points are the
 // "landmarks" (128 per tile row), the n_obs observations are the "records" carrying coef as their weight, spread
 // over 8 sets so that the 256-column tiles are full; the 8 partial sums per point are added afterwards.
@@ -294,9 +301,7 @@ int landmark_dot_tc(basq_ctx* ctx, const KParams& kp, const void* Xobs, int n_ob
     a.ldg = SETS;
     a.accumulate = false;
     BASQ_TRY(set_sums(ctx, kp, a));
-    rowsum_cols_kernel<<<(unsigned)ceil_div64(cnt, 256), 256, 0, ctx->stream>>>(G.as<double>(), cnt, SETS, c0, out + p0);
-    ctx->launches++;
-    BASQ_CUDA(cudaGetLastError());
+    BASQ_TRY(rowsum_cols(ctx, G.as<double>(), cnt, SETS, c0, out + p0));
   }
   return BASQ_OK;
 }

@@ -90,9 +90,11 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
   // full / empty hand-shake costs more than the halved B stream saves), so it stays opt-in.
   const bool pairs = !gram && ctx->num_sms >= 2 && ([] { const char* e = getenv("BASQ_NLS_2CTA"); return e && e[0] == '1'; }());
   const int n_jg_total = ceil_div(S, JT);
-  // tile stride: an upper bound of any group's tile count
+  // tile stride: an upper bound of any group's tile count.  The kernels start group g at
+  // e_lo = ceil((p_lo + off - (g JT + JT - 1)) / S); the last group's column n_jg_total JT - 1 may exceed
+  // S - 1 (GRAM mode with S < JT: 255), so the bound takes that column.
   const int64_t e_hi_max = (p_hi - 1 + off) / S + 1;
-  const int64_t num_lo = p_lo + off - (int64_t)(S - 1);
+  const int64_t num_lo = p_lo + off - ((int64_t)n_jg_total * JT - 1);
   const int64_t e_lo_min = num_lo <= 0 ? 0 : (num_lo + S - 1) / S;
   const int T = (int)std::max<int64_t>(1, ceil_div64(e_hi_max - e_lo_min, EC));
   const size_t b_tile_bytes = (size_t)op->KP * NLS_NT * 2;              // one of hi / lo

@@ -114,7 +114,7 @@ __global__ void build_records_kernel(KParams kp, const T* __restrict__ X, int64_
 }
 
 int build_records(basq_ctx* ctx, const KParams& kp, int dtype, const void* X, int64_t N, double uniform_w,
-                  const double* mu, const double* factor, bool factor_in_weight, RecPool* pool) {
+                  const double* mu, const double* factor, bool factor_in_weight, RecPool* pool, bool round_buffer) {
   BASQ_CHECK(N >= 0 && N < (1ll << 31) - 1024, BASQ_ERR_UNSUPPORTED,
              "at most 2^31 candidates per rank (got %lld)", (long long)N);
   pool->dtype = dtype;
@@ -126,7 +126,7 @@ int build_records(basq_ctx* ctx, const KParams& kp, int dtype, const void* X, in
   BASQ_TRY(pool->buf[0].alloc(ctx, (size_t)(N + 1) * pool->rec_bytes));
   // the second buffer only ever receives the survivors of a round (about half), but the first
   // round of a weighted run may keep more: size it for the worst case of one halving round + 1.
-  BASQ_TRY(pool->buf[1].alloc(ctx, (size_t)(N + 1) * pool->rec_bytes));
+  if (round_buffer) BASQ_TRY(pool->buf[1].alloc(ctx, (size_t)(N + 1) * pool->rec_bytes));
   if (N == 0) return BASQ_OK;
   const int nb = ceil_div(N, 256);
   DevBuf counts, offs, total;

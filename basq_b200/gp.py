@@ -92,3 +92,33 @@ def quadrature(X, w, kernel):
     K = ops.gram(kernel, X, X)
     w64 = w.to(torch.float64)
     return float(w64 @ mean), float(w64 @ K @ w64)
+
+
+def full_quadrature(X, w, kernel):
+    """SOBER's full_quadrature (SOBER/BASQ/_basq.py:48-81) at candidate scale: the formulas of ``quadrature``,
+    EZy = w . m(X) and VarZy = w^T K(X, X) w, with the variance streamed by ops.kernel_quadform instead of
+    forming K (N = 1e6 would need 8 TB)."""
+    mean, _ = ops.gp_predict(kernel, X, space=1, want_var=False)
+    w64 = w.to(device=mean.device, dtype=torch.float64)
+    return float(w64 @ mean), ops.kernel_quadform(kernel, X, w64)
+
+
+def worst_case_error(kernel, X, idx, w, mu=None):
+    """Squared worst-case error of the quadrature rule (idx, w) over the candidates X - the rule that
+    ``recombination`` returns - in the kernel's RKHS: the squared MMD (mu - w~)^T K (mu - w~) between the rule
+    and the candidate measure mu (None: uniform 1/N, as in recombination), where w~ is w scattered to idx.
+
+    It is one quadratic form of a signed measure (ops.kernel_quadform), so the cancellation between the
+    measure and the rule happens in the fp64 accumulators.  For fp32 inputs the kernel values are fp32
+    (relative error ~2^-21): a rule at that resolution floor may come out as a tiny negative number."""
+    device = X.device
+    N = len(X)
+    if mu is None:
+        a = torch.full((N,), 1.0 / N, dtype=torch.float64, device=device)
+    else:
+        a = mu.to(device=device, dtype=torch.float64).clone()
+    idx = torch.as_tensor(idx, device=device).long()
+    if idx.numel() != torch.unique(idx).numel():
+        raise ValueError("worst_case_error: the rule's indices must be distinct")
+    a[idx] -= torch.as_tensor(w, device=device).to(torch.float64)
+    return ops.kernel_quadform(kernel, X, a)

@@ -49,6 +49,40 @@ def gp_predict(kernel, X, space=0, want_var=True, device=None):
     return mean, var
 
 
+def _weights(w, n, device, what):
+    wd = _prep(torch.as_tensor(w), device, torch.float64)
+    if wd.shape != (n,):
+        raise ValueError(f"{what} must have one entry per point ({n}), not shape {tuple(wd.shape)}")
+    return wd
+
+
+def kernel_quadform(kernel, X, a, device=None) -> float:
+    """a^T kernel(X, X) a for fp64 weights a [N] (any sign) without forming the N x N matrix
+    (basq_kernel_quadform): the square Gram matrix of ``gram``, diagonal terms included, summed in fp64 in a
+    fixed order.  Every mode of ``describe_kernel``."""
+    spec, ctx, device, dtype = _common(kernel, X, device)
+    Xd = _prep(X, device, dtype)
+    ad = _weights(a, len(Xd), device, "a")
+    desc, keep = spec.to_desc(Xd.shape[1], device, dtype)
+    out = C.c_double(0.0)
+    _lib.check(_lib.lib.basq_kernel_quadform(ctx.handle, C.byref(desc), Xd.data_ptr(), len(Xd), ad.data_ptr(),
+                                             C.byref(out)))
+    return float(out.value)
+
+
+def kernel_bilinear(kernel, X, a, Y, b, device=None) -> float:
+    """sum_ij a_i b_j kernel(x_i, y_j) (basq_kernel_bilinear): the kernel function alone, without the diagonal
+    terms of the square Gram matrix even when Y is X."""
+    spec, ctx, device, dtype = _common(kernel, X, device)
+    Xd, Yd = _prep(X, device, dtype), _prep(Y, device, dtype)
+    ad, bd = _weights(a, len(Xd), device, "a"), _weights(b, len(Yd), device, "b")
+    desc, keep = spec.to_desc(Xd.shape[1], device, dtype)
+    out = C.c_double(0.0)
+    _lib.check(_lib.lib.basq_kernel_bilinear(ctx.handle, C.byref(desc), Xd.data_ptr(), len(Xd), ad.data_ptr(),
+                                             Yd.data_ptr(), len(Yd), bd.data_ptr(), C.byref(out)))
+    return float(out.value)
+
+
 def _seed_context(ctx, seed):
     """Key of the library's next Gaussian draw: the caller's, or - like every torch routine the reference
     calls - the next value of torch's global generator, so that torch.manual_seed reproduces a run."""

@@ -273,3 +273,62 @@ def _shared_seed(group, on, device):
         s = s.to(device) if dist.get_backend(group) == "nccl" else s
         dist.broadcast(s, dist.get_global_rank(group, 0) if group is not None else 0, group=group)
     return int(s.item())
+
+
+def quadform_pair_assignment(world):
+    """Cross terms of a sharded quadratic form, assigned to ranks: tasks[r] lists (i, j, half) for rank r,
+    meaning 2 B(X_i, a_i; X_j, a_j) restricted to the rows of shard i given by `half` (None: all rows, 0: the
+    first len_i // 2 rows, 1: the rest).  Every unordered pair i < j of shards is covered exactly once: rank r
+    takes the pairs (r, r + k mod G) for k = 1 .. (G - 1) // 2, and for even G the antipodal pair
+    (r, r + G / 2) is split by rows between its two ranks (B is linear in a).  Every rank gets (G - 1) / 2
+    pair-equivalents."""
+    tasks = [[] for _ in range(world)]
+    for r in range(world):
+        for k in range(1, (world - 1) // 2 + 1):
+            s = (r + k) % world
+            tasks[r].append((min(r, s), max(r, s), None))
+        if world % 2 == 0 and world > 1:
+            h = world // 2
+            tasks[r].append((r, r + h, 0) if r < h else (r - h, r, 1))
+    return tasks
+
+
+def _all_gather_var(t, group, nccl):
+    """All-gather tensors whose first dimension differs between ranks (padded to the largest)."""
+    world = dist.get_world_size(group)
+    dev = t.device
+    n = torch.tensor([len(t)], dtype=torch.int64, device=dev if nccl else "cpu")
+    sizes = [torch.zeros_like(n) for _ in range(world)]
+    dist.all_gather(sizes, n, group=group)
+    sizes = [int(s) for s in sizes]
+    pad = torch.zeros((max(sizes),) + tuple(t.shape[1:]), dtype=t.dtype, device=dev if nccl else "cpu")
+    pad[: len(t)] = t
+    parts = [torch.empty_like(pad) for _ in range(world)]
+    dist.all_gather(parts, pad, group=group)
+    return [p[:s].to(dev) for p, s in zip(parts, sizes)]
+
+
+def kernel_quadform_sharded(kernel, X_local, a_local, group=None) -> float:
+    """a^T kernel(X, X) a (ops.kernel_quadform) for X, a sharded by rows over the ranks, one process per GPU:
+    the shards are all-gathered, rank r adds its own Q(X_r, a_r) and the cross terms 2 B(X_i, a_i; X_j, a_j)
+    that quadform_pair_assignment gives it, and one all-reduce of a scalar sums the ranks.  Every rank
+    returns the total.  With a gloo group the collectives are staged through the host."""
+    from . import ops
+
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return ops.kernel_quadform(kernel, X_local, a_local)
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    nccl = dist.get_backend(group) == "nccl"
+    a_local = a_local.to(device=X_local.device, dtype=torch.float64)
+    Xs = _all_gather_var(X_local.contiguous(), group, nccl)
+    As = _all_gather_var(a_local.contiguous(), group, nccl)
+    total = ops.kernel_quadform(kernel, X_local, a_local) if len(X_local) else 0.0
+    for i, j, half in quadform_pair_assignment(world)[rank]:
+        lo, hi = 0, len(Xs[i])
+        if half is not None:
+            lo, hi = (0, hi // 2) if half == 0 else (hi // 2, hi)
+        if hi > lo and len(Xs[j]):
+            total += 2.0 * ops.kernel_bilinear(kernel, Xs[i][lo:hi], As[i][lo:hi], Xs[j], As[j])
+    s = torch.tensor([total], dtype=torch.float64, device=X_local.device if nccl else "cpu")
+    dist.all_reduce(s, group=group)
+    return float(s.item())

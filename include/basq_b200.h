@@ -139,6 +139,23 @@ int basq_gram(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_
 int basq_gp_predict(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N,
                     int space, double offset, double* mean_out, double* var_out);
 
+/* ---- weighted double sums: SOBER's full_quadrature variance (SOBER/BASQ/_basq.py:48-81) ------ */
+/* *out_host = a^T basq_gram(desc, X, X) a for weights a[N] (fp64, any sign, zeros allowed), without forming the
+   N x N matrix: the kernel of desc->mode exactly as basq_gram evaluates it, including the diagonal terms
+   (noise_diag, diag_add) of the square matrix.  The sum is accumulated in fp64 in a fixed order: the same
+   inputs give the same bits on every call.  1 <= N < 2^31 - 1024; non-finite weights: BASQ_ERR_NUMERIC.
+   Every mode.  fp32 inputs evaluate the kernel in fp32 (basq_ctx_allow_f32_eval applies to fp64 inputs as for
+   sessions); in WSABI-M and MMLT the conditioning guard (basq_ctx_conditioning) computes kappa over every row
+   of X and promotes fp32 inputs to the fp64 path beyond kappa_max.  The record buffer takes 64 B per point at
+   d = 10 (fp32; 96 B fp64), so device memory limits N well below the index limit.  Synchronises. */
+int basq_kernel_quadform(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N,
+                         const double* a, double* out_host);
+/* *out_host = sum_ij a_i b_j kernel(X[i], Y[j]) for X[N], Y[Mb] with weights a[N], b[Mb]: the kernel function
+   alone.  X and Y are different arrays, so basq_gram's diagonal terms (noise_diag, diag_add) do not enter,
+   even when Y is X.  Same conventions as basq_kernel_quadform. */
+int basq_kernel_bilinear(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N, const double* a,
+                         const void* Y, int64_t Mb, const double* b, double* out_host);
+
 /* ---- Nystrom eigenbasis: ker_svd_sparsify, BASQ/_rchq.py:28-31 ------------------------------ */
 /* Randomised range finder (Halko alg. 4.4, niter subspace iterations, as torch.svd_lowrank) on
    K(Z,Z) with the Gaussian test matrix Omega[M,q] (fp64): the caller's, or - Omega NULL, what
