@@ -1156,6 +1156,10 @@ int basq_gp_predict(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, 
   BASQ_CHECK(ctx && desc && X && mean_out, BASQ_ERR_INVALID, "basq_gp_predict: NULL argument");
   BASQ_CHECK(desc->n_obs > 0 && desc->Xobs && desc->W && desc->alpha, BASQ_ERR_INVALID,
              "basq_gp_predict needs the GP caches (n_obs, Xobs, W, alpha)");
+  const bool need_var = var_out != nullptr || (space == 1 && (desc->mode == BASQ_WSABI_M || desc->mode == BASQ_MMLT_G));
+  // the limit of the fp32 variance route, checked again in gp_variance_tc: here before anything is allocated
+  BASQ_CHECK(!(need_var && N > 0 && gpvar_route(ctx, desc)) || desc->n_obs <= GPV_MAX_OBS, BASQ_ERR_UNSUPPORTED,
+             "basq_gp_predict: %d observations; the fp32 posterior variance takes at most %d", desc->n_obs, GPV_MAX_OBS);
   BASQ_CUDA(cudaSetDevice(ctx->device));
   KParams kp;
   basq_kernel_desc d2 = *desc;
@@ -1165,7 +1169,6 @@ int basq_gp_predict(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, 
   Landmarks lmobs;
   BASQ_TRY(prep_landmarks(ctx, kp, d2.dtype, d2.Xobs, d2.n_obs, nullptr, 0, &lmobs));
   const bool warped = (desc->mode == BASQ_WSABI_L || desc->mode == BASQ_WSABI_M || desc->mode == BASQ_MMLT_G);
-  const bool need_var = var_out != nullptr || (space == 1 && (desc->mode == BASQ_WSABI_M || desc->mode == BASQ_MMLT_G));
   DevBuf vtmp;
   double* var = var_out;
   if (need_var && !var) {

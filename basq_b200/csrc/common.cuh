@@ -452,6 +452,9 @@ int landmark_dot(basq_ctx* ctx, const KParams& kp, const LmView& lm, const doubl
                  const void* P, int64_t N, double* out);
 // out[p] = c0 + sum_{j < cols} G[p, j]   (p < n; fixed order)
 int rowsum_cols(basq_ctx* ctx, const double* G, int64_t n, int cols, double c0, double* out);
+// whether gp_predict_impl computes the variance on the tensor cores (gp_variance_tc): fp32 inputs, unless
+// BASQ_GPVAR=0 selects the chunked fp64-GEMM route
+bool gpvar_route(basq_ctx* ctx, const basq_kernel_desc* desc);
 int gp_predict_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const LmView& lmobs,
                     const void* X, int64_t N, double* mean_out, double* var_out);
 // per-point / per-landmark factor of the warped kernels (m(x) or mu_g(x)); out == nullptr allowed
@@ -511,17 +514,23 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
 
 // gpvar.cu: fused posterior variance on the tensor cores (fp32 inputs)
 // mean_out != NULL: the fused kernel also writes the posterior mean (*mean_done tells whether it did)
+// At most GPV_MAX_OBS observations: KP^2 (the L^-1 operand tiles) stays inside int32 element indexing and the
+// fp64 factor (8 n_obs^2 B) inside a few GB.  The variance kernels themselves do not depend on it.
+constexpr int GPV_MAX_OBS = 32768;
 int gp_variance_tc(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const LmView& lmobs, const void* X,
                    int64_t N, double* var_out, double* mean_out = nullptr, bool* mean_done = nullptr);
 
 // dgemm.cu
 int dgemm(basq_ctx* ctx, bool ta, bool tb, int m, int n, int k, double alpha, const double* A, int64_t lda,
           const double* B, int64_t ldb, double beta, double* C, int64_t ldc, bool b_lower_tri = false,
-          bool a_lower_tri = false, bool c_symmetric = false);
+          bool a_lower_tri = false, bool c_symmetric = false, bool c_lower_only = false);
 // b_lower_tri (with tb): B is lower triangular, C = A B^T only visits k <= column
 // a_lower_tri (without ta): A is lower triangular, C = A B only visits k <= row
 // c_symmetric (m == n, beta == 0; e.g. A^T A): only the tiles that touch the lower triangle are computed, the
 //   K range is split so that they still fill the SMs, and the upper triangle is the mirror image
+// c_lower_only (m == n, any beta; e.g. the trailing update of a Cholesky factorisation): only the tiles that
+//   touch the lower triangle are computed and written, nothing is mirrored; entries above the diagonal inside
+//   those tiles are written too, the others keep their values
 
 // car.cu
 int caratheodory(basq_ctx* ctx, double* A, int n, int S, int lda, double* omega_out);

@@ -106,7 +106,7 @@ __global__ void __launch_bounds__(WM* WN * 32) dgemm_pipe_kernel(int M, int N, i
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int wm = warp / WN, wn = warp % WN;
   const int m0 = blockIdx.y * BM, n0 = blockIdx.x * BNN;
-  if (sym && n0 >= m0 + BM) return;     // tile strictly above the diagonal: mirrored afterwards
+  if (sym && n0 >= m0 + BM) return;     // tile strictly above the diagonal: mirrored afterwards (sym 1) or left alone (2)
   if (tri_k & 1) K = min(K, n0 + BNN);  // op(B)[k][n] = 0 for k > n
   if (tri_k & 2) K = min(K, m0 + BM);   // op(A)[m][k] = 0 for k > m
   // split-K (small outputs, long K): slice blockIdx.z covers k in [kb, K) with K clipped to the slice
@@ -220,12 +220,12 @@ int launch_pipe(basq_ctx* ctx, int m, int n, int k, double alpha, const double* 
     for (unsigned by = 0; by < grid.y; ++by) tiles += std::min<int64_t>(grid.x, ceil_div64((int64_t)(by + 1) * BM, BNN));
   }
   int splits = 1;
-  if (tri_k == 0 && tiles * 2 <= ctx->num_sms && k >= 16 * PK)
+  if (sym != 2 && tri_k == 0 && tiles * 2 <= ctx->num_sms && k >= 16 * PK)
     splits = (int)std::min<int64_t>(ctx->num_sms / tiles, k / (8 * PK));
   if (splits <= 1) {
     kern<<<grid, WM * WN * 32, SMEM, ctx->stream>>>(m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, a16, b16, 0,
                                                     nullptr, sym);
-    if (sym) {
+    if (sym == 1) {
       mirror_lower_kernel<<<(unsigned)ceil_div64((int64_t)n * n, 256), 256, 0, ctx->stream>>>(C, n, ldc);
       ctx->launches++;
     }
@@ -264,12 +264,15 @@ int launch_best(basq_ctx* ctx, int m, int n, int k, double alpha, const double* 
 
 int dgemm(basq_ctx* ctx, bool ta, bool tb, int m, int n, int k, double alpha, const double* A, int64_t lda,
           const double* B, int64_t ldb, double beta, double* C, int64_t ldc, bool b_lower_tri, bool a_lower_tri,
-          bool c_symmetric) {
+          bool c_symmetric, bool c_lower_only) {
   BASQ_CHECK(!c_symmetric || (m == n && beta == 0.0 && !b_lower_tri && !a_lower_tri), BASQ_ERR_INVALID,
              "dgemm: c_symmetric needs a square output, beta = 0 and dense operands");
+  BASQ_CHECK(!c_lower_only || (m == n && !c_symmetric && !b_lower_tri && !a_lower_tri), BASQ_ERR_INVALID,
+             "dgemm: c_lower_only needs a square output and dense operands");
   // A^T A and A A^T are recognised without the flag
   const bool gram = (ta != tb) && A == B && lda == ldb && m == n && beta == 0.0 && !b_lower_tri && !a_lower_tri;
-  const int sym = (c_symmetric || gram) ? 1 : 0;
+  // sym 1: lower tiles, then mirrored; 2: lower tiles only
+  const int sym = c_lower_only ? 2 : ((c_symmetric || gram) ? 1 : 0);
   const int tri_k = ((b_lower_tri && tb) ? 1 : 0) | ((a_lower_tri && !ta) ? 2 : 0);
   if (m <= 0 || n <= 0) return BASQ_OK;
   BASQ_CHECK(k >= 0, BASQ_ERR_INVALID, "dgemm: negative k");

@@ -52,10 +52,9 @@ struct GpvDev {
 
 struct GpvCfg {
   static constexpr int NSTAGE = 4;
-  static constexpr int MAX_KP = 4096;                          // observations (padded) the tinv table holds
   static constexpr int OFF_STAGE = 0;
-  static constexpr int OFF_TINV = NSTAGE * GPV_STAGE_BYTES;
-  static constexpr int OFF_COMB = OFF_TINV + MAX_KP * 4;
+  static constexpr int OFF_TINV = NSTAGE * GPV_STAGE_BYTES;    // [8 epilogue warps][128] scale factors
+  static constexpr int OFF_COMB = OFF_TINV + NLS_EPI_WARPS * (GPV_NT / 2) * 4;
   static constexpr int OFF_BAR = OFF_COMB + 128 * 8;
   static constexpr int SMEM_BYTES = OFF_BAR + 256;
   static_assert(SMEM_BYTES <= 227 * 1024, "gpvar: shared memory budget");
@@ -88,7 +87,6 @@ __global__ void __launch_bounds__(NLS_THREADS, 1) gpvar_kernel(const GpvDev a) {
     }
     mma::fence_barrier_init();
   }
-  for (int o = tid; o < a.KP; o += NLS_THREADS) sTinv[o] = a.tinv[o];
   if (warp == NLS_EPI_WARPS + 1) mma::tmem_alloc(tmem_slot, 512);
   mma::tc_fence_before();
   __syncthreads();
@@ -108,10 +106,15 @@ __global__ void __launch_bounds__(NLS_THREADS, 1) gpvar_kernel(const GpvDev a) {
       double acc = 0.0;
       for (int c = 0; c < n_ctiles; ++c, ++tc) {
         const uint32_t buf = tc & 1u, ph = (tc >> 1) & 1u;
+        // the 128 scale factors of this warp's column half, staged per column tile in the warp's own slot
+        // (a table of all KP of them would bound the observation count); the __syncwarp before the
+        // previous t_empty arrival ordered the previous tile's reads
+        float* ti = sTinv + warp * (NT / 2);
+        reinterpret_cast<float4*>(ti)[lane] = reinterpret_cast<const float4*>(a.tinv + c * NT + half * (NT / 2))[lane];
+        __syncwarp();
         mma::mbar_wait(&t_full[buf], ph);
         mma::tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + buf * NT + half * (NT / 2);
-        const float* ti = sTinv + c * NT + half * (NT / 2);
 #pragma unroll 1
         for (int cb = 0; cb < NT / 2; cb += 32) {
           uint32_t v[32];
@@ -250,8 +253,8 @@ struct GpfCfg {
   static constexpr int OFF_OBS = OFF_B + NB * GPF_B_STAGE;           // [2][32][OBF] floats
   static constexpr int OBS_BYTES = ((2 * NLS_KB * OBF * 4) + 15) / 16 * 16;
   static constexpr int OFF_ALPHA = OFF_OBS + OBS_BYTES;               // [2][32] doubles (mean cache of a K block)
-  static constexpr int OFF_TINV = OFF_ALPHA + 2 * NLS_KB * 8;
-  static constexpr int OFF_COMB = OFF_TINV + GpvCfg::MAX_KP * 4;
+  static constexpr int OFF_TINV = OFF_ALPHA + 2 * NLS_KB * 8;         // [8 epilogue warps][128] scale factors
+  static constexpr int OFF_COMB = OFF_TINV + GPF_EPI_WARPS * (GPV_NT / 2) * 4;
   static constexpr int OFF_MEAN = OFF_COMB + 128 * 8;                 // [128] doubles: second generator thread's part
   static constexpr int OFF_BAR = OFF_MEAN + 128 * 8;
   static constexpr int SMEM_BYTES = OFF_BAR + 256;
@@ -294,7 +297,6 @@ __global__ void __launch_bounds__(GPF_THREADS, 1) gpvar_fused_kernel(KParams kp,
     }
     mma::fence_barrier_init();
   }
-  for (int o = tid; o < a.KP; o += GPF_THREADS) sTinv[o] = a.tinv[o];
   if (warp == GPF_GEN_WARPS + GPF_EPI_WARPS + 1) mma::tmem_alloc(tmem_slot, 512);
   mma::tc_fence_before();
   __syncthreads();
@@ -426,10 +428,15 @@ __global__ void __launch_bounds__(GPF_THREADS, 1) gpvar_fused_kernel(KParams kp,
         for (int i = 0; i < 2; ++i) {
           const int c = 2 * sw + i;
           if (c >= n_ct) break;
+          // the 128 scale factors of this warp's column half, staged per column tile in the warp's own slot
+          // (a table of all KP of them would bound the observation count); the __syncwarp before the
+          // previous t_empty arrival ordered the previous tile's reads
+          float* ti = sTinv + ew * (NT / 2);
+          reinterpret_cast<float4*>(ti)[lane] = reinterpret_cast<const float4*>(a.tinv + c * NT + half * (NT / 2))[lane];
+          __syncwarp();
           mma::mbar_wait(&t_full[i], use[i] & 1u);
           mma::tc_fence_after();
           const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + i * NT + half * (NT / 2);
-          const float* ti = sTinv + c * NT + half * (NT / 2);
 #pragma unroll 1
           for (int cb = 0; cb < NT / 2; cb += 32) {
             uint32_t v[32];

@@ -306,12 +306,16 @@ int landmark_dot_tc(basq_ctx* ctx, const KParams& kp, const void* Xobs, int n_ob
   return BASQ_OK;
 }
 
+bool gpvar_route(basq_ctx* ctx, const basq_kernel_desc* desc) {
+  { const char* t = getenv("BASQ_GPVAR"); ctx->no_gpvar = t && t[0] == '0'; }
+  return desc->dtype == BASQ_F32 && !ctx->no_gpvar;
+}
+
 // Exact GP posterior mean / variance (likelihood noise included), BASQ/_gp.py:213-230.
 int gp_predict_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& kp, const LmView& lmobs,
                     const void* X, int64_t N, double* mean_out, double* var_out) {
   PhaseTimer timer(ctx, PH_GP);
-  { const char* t = getenv("BASQ_GPVAR"); ctx->no_gpvar = t && t[0] == '0'; }
-  if (var_out && N > 0 && desc->dtype == BASQ_F32 && !ctx->no_gpvar) {
+  if (var_out && N > 0 && gpvar_route(ctx, desc)) {
     // fused tensor-core kernel: variance, and the mean from the same kernel values
     bool mean_done = false;
     BASQ_TRY(gp_variance_tc(ctx, desc, kp, lmobs, X, N, var_out, mean_out, &mean_done));

@@ -484,16 +484,25 @@ __global__ void __launch_bounds__(NLS_NT) kxgen_kernel(const KxDev a) {
 // ---------------------------------------------------------------------------------------------
 // fp64 matrix -> row-scaled fp16 hi / lo operand tiles (Az here, T = tril(W + W^T) in gpvar.cuh)
 // ---------------------------------------------------------------------------------------------
+// REV (square A, rows == cols == n): the operand is the lower triangle of J G^T J, J the reversal
+// permutation - element [m, o] is G[n-1-o, n-1-m] for o <= m and 0 above the diagonal; G's upper
+// triangle is never read.  L^-1 of a GP comes out of the Cholesky factor G of J W J in this form (gpvar.cu).
+template <bool REV>
+__device__ __forceinline__ double op16_at(const double* __restrict__ A, int rows, int64_t lda, int m, int o) {
+  if (!REV) return A[(int64_t)m * lda + o];
+  return o <= m ? A[(int64_t)(rows - 1 - o) * lda + (rows - 1 - m)] : 0.0;
+}
+
 // one block per row: r = 2^(13 - floor(log2 max_o |A[m, o]|)), so that the scaled row lies in [2^13, 2^14);
 // inv[m] = 1 / (r * kx_scale) (a power of two, exact).  Rows beyond `rows` get 0.
-template <int THREADS>
+template <int THREADS, bool REV = false>
 __global__ void rowscale16_kernel(const double* __restrict__ A, int rows, int cols, int64_t lda, float kx_scale,
                                   float* __restrict__ rscale, float* __restrict__ inv) {
   __shared__ double sh[THREADS];
   const int m = blockIdx.x;
   double mx = 0.0;
   if (m < rows)
-    for (int o = threadIdx.x; o < cols; o += THREADS) mx = fmax(mx, fabs(A[(int64_t)m * lda + o]));
+    for (int o = threadIdx.x; o < (REV ? m + 1 : cols); o += THREADS) mx = fmax(mx, fabs(op16_at<REV>(A, rows, lda, m, o)));
   sh[threadIdx.x] = mx;
   __syncthreads();
   for (int w = THREADS / 2; w > 0; w >>= 1) {
@@ -516,7 +525,7 @@ __global__ void rowscale16_kernel(const double* __restrict__ A, int rows, int co
 
 // one thread per (row tile, K chunk of 8, row): 8 scaled values -> fp16 hi / lo, 16-byte stores into
 // [tile][KP / 8][TILE_ROWS][8 halves]
-template <int TILE_ROWS>
+template <int TILE_ROWS, bool REV = false>
 __global__ void split16_kernel(const double* __restrict__ A, int rows, int cols, int64_t lda, int KP, int n_tiles,
                                const float* __restrict__ rscale, __half* __restrict__ hi, __half* __restrict__ lo) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -531,7 +540,7 @@ __global__ void split16_kernel(const double* __restrict__ A, int rows, int cols,
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
     const int o = kc * 8 + e;
-    const double x = (m < rows && o < cols) ? A[(int64_t)m * lda + o] * rs : 0.0;
+    const double x = (m < rows && o < cols) ? op16_at<REV>(A, rows, lda, m, o) * rs : 0.0;
     h[e] = __double2half(x);
     l[e] = __double2half(x - (double)__half2float(h[e]));   // residual against the fp64 value: ~22 bits in hi + lo
   }

@@ -13,6 +13,8 @@
 // elimination of [G | I], one grid barrier per column).
 #include <math.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 #include "gridsync.cuh"
 #include "tgemm.cuh"
@@ -503,6 +505,64 @@ int spd_inverse_factor(basq_ctx* ctx, const double* A, int n, double* Linv_out) 
   BASQ_CUDA(cudaMemcpyAsync(&status, ws.flags.as<int>() + 64, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
   BASQ_CHECK(status == 0, BASQ_ERR_NUMERIC, "spd_inverse_factor: grid barrier watchdog fired in the Cholesky kernel");
+  return BASQ_OK;
+}
+
+namespace {
+// The diagonal block A [b, b] (ld lda) made symmetric from its lower triangle, in place, and copied to dst (ld b)
+__global__ void sym_block_kernel(double* __restrict__ A, int64_t lda, int b, double* __restrict__ dst) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= b * b) return;
+  const int i = t / b, j = t % b;
+  const double v = i >= j ? A[(int64_t)i * lda + j] : A[(int64_t)j * lda + i];
+  if (i < j) A[(int64_t)i * lda + j] = v;
+  dst[t] = v;
+}
+}  // namespace
+
+// In place: the lower triangle of the symmetric positive definite A [n, n] (row-major, ld n; only the lower
+// triangle is read) becomes its Cholesky factor G, A = G G^T.  The upper triangle is left with scratch values.
+// Blocked right-looking, panels of 256 columns:
+//   - the diagonal block goes through the cooperative Cholesky + inverse kernel above (G_kk^-1);
+//   - the column panel, diagonal block included, is A[k:, k:k+b] G_kk^-T (A_kk G_kk^-T = G_kk): one DMMA GEMM
+//     against a lower-triangular operand;
+//   - the trailing matrix loses P P^T of the panel rows below the diagonal block, lower tiles only.
+// n^3 / 3 flop, nearly all of it in the trailing updates; no triangular inverse of the whole matrix.
+int spd_chol_blocked(basq_ctx* ctx, double* A, int n) {
+  constexpr int CHB = 256;
+  BASQ_CHECK(A && n >= 1, BASQ_ERR_INVALID, "spd_chol_blocked: bad argument");
+  const int nb = n < CHB ? n : CHB;
+  OrthWs ws;
+  DevBuf panel;
+  BASQ_TRY(ws.gram.alloc(ctx, sizeof(double) * (size_t)nb * nb));
+  BASQ_TRY(ws.linv.alloc(ctx, sizeof(double) * (size_t)nb * nb));
+  BASQ_TRY(ws.prow.alloc(ctx, sizeof(double) * 4 * nb));
+  BASQ_TRY(ws.prow2.alloc(ctx, sizeof(double) * 2 * (size_t)nb * nb));
+  BASQ_TRY(ws.flags.alloc(ctx, 512));
+  BASQ_TRY(panel.alloc(ctx, sizeof(double) * (size_t)n * CHB));
+  BASQ_CUDA(cudaMemsetAsync(ws.flags.p, 0, 512, ctx->stream));   // the watchdog status (byte 256) stays set once fired
+  for (int k = 0; k < n; k += CHB) {
+    const int b = std::min(CHB, n - k);
+    double* Akk = A + (int64_t)k * n + k;
+    sym_block_kernel<<<ceil_div(b * b, 256), 256, 0, ctx->stream>>>(Akk, n, b, ws.gram.as<double>());
+    ctx->launches++;
+    BASQ_TRY(chol_inverse(ctx, ws, b, 1e-300));
+    // P [n - k, b] (ld CHB) = A[k:, k:k+b] G_kk^-T, written back over the panel's columns
+    BASQ_TRY(dgemm(ctx, false, true, n - k, b, b, 1.0, Akk, n, ws.linv.as<double>(), b, 0.0, panel.as<double>(), CHB,
+                   /*b_lower_tri=*/true));
+    BASQ_CUDA(cudaMemcpy2DAsync(Akk, sizeof(double) * n, panel.p, sizeof(double) * CHB, sizeof(double) * b, n - k,
+                                cudaMemcpyDeviceToDevice, ctx->stream));
+    const int t = n - k - b;
+    if (t > 0) {
+      const double* Pb = panel.as<double>() + (int64_t)b * CHB;
+      BASQ_TRY(dgemm(ctx, false, true, t, t, b, -1.0, Pb, CHB, Pb, CHB, 1.0, Akk + (int64_t)b * n + b, n, false, false,
+                     false, /*c_lower_only=*/true));
+    }
+  }
+  int status = 0;
+  BASQ_CUDA(cudaMemcpyAsync(&status, ws.flags.as<int>() + 64, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  BASQ_CHECK(status == 0, BASQ_ERR_NUMERIC, "spd_chol_blocked: grid barrier watchdog fired in the Cholesky kernel");
   return BASQ_OK;
 }
 

@@ -38,7 +38,9 @@ def gram(kernel, X, Y, device=None) -> torch.Tensor:
 
 def gp_predict(kernel, X, space=0, want_var=True, device=None):
     """GP posterior mean / variance over candidates (BASQ/_gp.py:213-230, exact variance).
-    space=1 returns the model-space moments of the kernel's mode (wsabi*_predict / gspace_predict)."""
+    space=1 returns the model-space moments of the kernel's mode (wsabi*_predict / gspace_predict).
+    For float32 inputs the variance (also needed by the WSABI-M / MMLT model space) takes GPs of at most 32768
+    observations; more raises BasqError with ERR_UNSUPPORTED."""
     spec, ctx, device, dtype = _common(kernel, X, device)
     Xd = _prep(X, device, dtype)
     desc, keep = spec.to_desc(Xd.shape[1], device, dtype)

@@ -135,7 +135,10 @@ int basq_gram(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_
 /* GP posterior over candidates, predict() of BASQ/_gp.py:213-230 with exact variance.
    space 0: the warped GP itself (mean, var incl. likelihood noise);
    space 1: the model space of desc->mode (wsabil_predict / wsabim_predict / gspace_predict),
-            `offset` is the WSABI alpha added to the mean.  var_out may be NULL. */
+            `offset` is the WSABI alpha added to the mean.  var_out may be NULL.
+   fp32 inputs: the variance (and the model-space moments of WSABI-M / MMLT, which need it) takes at most 32768
+   observations (desc->n_obs); more returns BASQ_ERR_UNSUPPORTED before anything is allocated.  The limit does
+   not apply with BASQ_GPVAR=0 or to fp64 inputs, which take the fp64-GEMM route. */
 int basq_gp_predict(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N,
                     int space, double offset, double* mean_out, double* var_out);
 
