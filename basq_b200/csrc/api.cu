@@ -953,8 +953,6 @@ int basq_ctx_create(int device, void* stream, basq_ctx** out) {
   if (const char* t = getenv("BASQ_POOL_KEEP_MB")) c->pool_keep = (uint64_t)strtoull(t, nullptr, 10) << 20;
   { const char* t = getenv("BASQ_TRACE"); c->trace = t && t[0] == '1'; }
   { const char* t = getenv("BASQ_CAR_GENERAL"); c->force_general_car = t && t[0] == '1'; }
-  { const char* t = getenv("BASQ_NYSTROM_FP64"); c->no_tensor_nystrom = t && t[0] == '1'; }
-  { const char* t = getenv("BASQ_SETSUM_SCALAR"); c->scalar_setsum = t && t[0] == '1'; }
   { const char* t = getenv("BASQ_F32_KAPPA_MAX"); if (t) c->kappa_max = atof(t); }
   { const char* t = getenv("BASQ_F64_EVAL_F32"); c->eval_f32 = t && t[0] == '1'; }
   *out = c;

@@ -129,8 +129,6 @@ struct basq_ctx {
   bool profile = false;
   int timer_depth = 0;
   bool force_general_car = false;  // BASQ_CAR_GENERAL=1: always use the global-memory kernel (tests)
-  bool scalar_setsum = false;      // BASQ_SETSUM_SCALAR=1: CUDA-core set-sum kernel for fp32 too (A/B timing)
-  bool no_tensor_nystrom = false;  // BASQ_NYSTROM_FP64=1: fp64 GEMMs in the Nystrom iteration for fp32 kernels too (A/B)
   bool no_gpvar = false;           // BASQ_GPVAR=0: chunked fp64-GEMM posterior variance for fp32 inputs too (A/B)
   // per-context driver objects that are expensive to create per call (api.cu): pinned staging ring of the level
   // calls, side stream + events of basq_recombine_host

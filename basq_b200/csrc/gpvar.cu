@@ -88,79 +88,27 @@ int gp_variance_tc(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& k
   }
   ctx->launches += 2;
   BASQ_CUDA(cudaGetLastError());
-  // Fused kernel (default): kernel values are generated on the SM, nothing is staged in HBM.
-  // BASQ_GPVAR_FUSED=0: the two-kernel version below (k(Xobs, X) staged as an fp16 operand), kept for A/B.
-  const bool fused = !([] { const char* e = getenv("BASQ_GPVAR_FUSED"); return e && e[0] == '0'; }());
-  if (fused) {
-    GpfDev f;
-    f.X = reinterpret_cast<const float*>(X);
-    f.n_points = N;
-    f.n_ptiles = (int)ceil_div64(N, GPV_MT);
-    f.ozz = reinterpret_cast<const float*>(lmobs.zz);
-    f.obz = lmobs.b;
-    f.n_obs = n_obs;
-    f.KP = KP;
-    f.kx_scale = kx_scale;
-    f.th = th.as<__half>(); f.tl = tl.as<__half>();
-    f.tinv = tinv.as<float>();
-    f.base = desc->outputscale + desc->noise;
-    f.var_out = var_out;
-    f.alpha = desc->alpha;          // the posterior mean rides along: its kernel values are the same ones
-    f.mean_c0 = desc->mean_const;
-    f.mean_out = mean_out;
-    if (mean_done) *mean_done = mean_out != nullptr;
-    switch (kp.family) {
-      case BASQ_RBF: BASQ_TRY(launch_gpvar_fused_rbf(ctx, kp, f)); break;
-      case BASQ_MATERN15: BASQ_TRY(launch_gpvar_fused_m15(ctx, kp, f)); break;
-      default: BASQ_TRY(launch_gpvar_fused_m25(ctx, kp, f)); break;
-    }
-    BASQ_CUDA(cudaStreamSynchronize(ctx->stream));  // scratch goes out of scope
-    return BASQ_OK;
-  }
-  // chunk of candidates: the kx operand (4 B x KP per candidate) takes at most ~2 GB
-  static const int64_t budget = [] {
-    const char* e = getenv("BASQ_GPV_CHUNK_MB");
-    return (int64_t)(e ? atoll(e) : 2048) << 20;
-  }();
-  int64_t P = std::max<int64_t>(GPV_MT, budget / (4ll * KP) / GPV_MT * GPV_MT);
-  P = std::min<int64_t>(P, ceil_div64(N, GPV_MT) * GPV_MT);
-  DevBuf kxh, kxl;
-  BASQ_TRY(kxh.alloc(ctx, (size_t)P * KP * 2));
-  BASQ_TRY(kxl.alloc(ctx, (size_t)P * KP * 2));
-  BASQ_CHECK((size_t)GpvCfg::SMEM_BYTES <= ctx->smem_optin, BASQ_ERR_UNSUPPORTED,
-             "gpvar: kernel needs %d B shared memory (limit %zu)", GpvCfg::SMEM_BYTES, ctx->smem_optin);
-  BASQ_CUDA(cudaFuncSetAttribute(gpvar_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GpvCfg::SMEM_BYTES));
-  for (int64_t p0 = 0; p0 < N; p0 += P) {
-    const int64_t cnt = std::min<int64_t>(P, N - p0);
-    const int n_ptiles = (int)ceil_div64(cnt, GPV_MT);
-    KxpDev kx;
-    kx.X = reinterpret_cast<const float*>(X) + p0 * desc->d;
-    kx.n_points = cnt;
-    kx.ozz = reinterpret_cast<const float*>(lmobs.zz);
-    kx.obz = lmobs.b;
-    kx.n_obs = n_obs;
-    kx.KP = KP;
-    kx.kx_scale = kx_scale;
-    kx.kxh = kxh.as<__half>();
-    kx.kxl = kxl.as<__half>();
-    switch (kp.family) {
-      case BASQ_RBF: BASQ_TRY(launch_kxgen_points_rbf(ctx, kp, kx, n_ptiles)); break;
-      case BASQ_MATERN15: BASQ_TRY(launch_kxgen_points_m15(ctx, kp, kx, n_ptiles)); break;
-      default: BASQ_TRY(launch_kxgen_points_m25(ctx, kp, kx, n_ptiles)); break;
-    }
-    GpvDev d;
-    d.kxh = kx.kxh; d.kxl = kx.kxl;
-    d.th = th.as<__half>(); d.tl = tl.as<__half>();
-    d.tinv = tinv.as<float>();
-    d.KP = KP;
-    d.n_ptiles = n_ptiles;
-    d.n_points = cnt;
-    d.os_f = kp.os_f;
-    d.base = desc->outputscale + desc->noise;
-    d.var_out = var_out + p0;
-    gpvar_kernel<0><<<std::min(ctx->num_sms, n_ptiles), NLS_THREADS, GpvCfg::SMEM_BYTES, ctx->stream>>>(d);
-    ctx->launches++;
-    BASQ_CUDA(cudaGetLastError());
+  GpfDev f;
+  f.X = reinterpret_cast<const float*>(X);
+  f.n_points = N;
+  f.n_ptiles = (int)ceil_div64(N, GPV_MT);
+  f.ozz = reinterpret_cast<const float*>(lmobs.zz);
+  f.obz = lmobs.b;
+  f.n_obs = n_obs;
+  f.KP = KP;
+  f.kx_scale = kx_scale;
+  f.th = th.as<__half>(); f.tl = tl.as<__half>();
+  f.tinv = tinv.as<float>();
+  f.base = desc->outputscale + desc->noise;
+  f.var_out = var_out;
+  f.alpha = desc->alpha;          // the posterior mean rides along: its kernel values are the same ones
+  f.mean_c0 = desc->mean_const;
+  f.mean_out = mean_out;
+  if (mean_done) *mean_done = mean_out != nullptr;
+  switch (kp.family) {
+    case BASQ_RBF: BASQ_TRY(launch_gpvar_fused_rbf(ctx, kp, f)); break;
+    case BASQ_MATERN15: BASQ_TRY(launch_gpvar_fused_m15(ctx, kp, f)); break;
+    default: BASQ_TRY(launch_gpvar_fused_m25(ctx, kp, f)); break;
   }
   BASQ_CUDA(cudaStreamSynchronize(ctx->stream));  // scratch goes out of scope
   return BASQ_OK;

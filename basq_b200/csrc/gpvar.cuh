@@ -17,12 +17,18 @@
 // Why L^-1 and not W: the rounding of a reduced-precision contraction scales with |M| |k|, and
 // |k|^T |W| |k| reaches 1e4 on the benchmark GP (1002 observations in 10-D, cond 1.5e4) where
 // 2 |v|^T |L^-1| |k| stays below 1e2: the T = tril(W + W^T) form measured 3e-3 absolute error, this one 1e-5.
-// Nothing of size n_obs x P is written to HBM in fp64 (round 1: V, Y = 4 x 8 B x n_obs per candidate);
-// the only staged operand is kx itself as fp16 hi / lo (4 B x n_obs per candidate, written once by
-// kxgen_points_kernel, read back through L2 by cp.async.bulk).
 //
-// CTA = 11 warps as nlsum_kernel: warp 8 streams operand stages, warp 9 issues the MMAs, warps 0-7 are
-// the epilogue (two column halves per lane quarter); warp 10 idles.
+// The kernel values k(Xobs, x) never leave the SM.  Eight generator warps (two threads per candidate of
+// the tile) evaluate the kernel values of one 32-observation K block, split them into fp16 hi / lo and
+// store them straight into the A stage in the tcgen05 K-major layout; the MMA warp contracts the stage
+// against the L^-1 tiles of TWO observation column tiles at once (two 256-column accumulators = all of
+// TMEM), so a K block is generated once per pair of column tiles (1.5x the unique evaluations at four
+// column tiles; they cost a third of the MMA time and hide under it).  DRAM traffic: the candidates in
+// (4 d B each), the variances out (8 B each).  The posterior mean rides along on the same kernel values.
+//   warps 0-7   generators (measured: four warps generate as slowly as the MMAs run; eight hide under them)
+//   warps 8-15  epilogue (TMEM lane quarter = warp % 4, two column halves)
+//   warp 16     L^-1 tile producer (cp.async.bulk, 32 KB units: hi / lo of one column tile's K block)
+//   warp 17     TMEM allocation + tcgen05.mma issue
 #pragma once
 #include <cuda_fp16.h>
 
@@ -36,191 +42,7 @@ constexpr int GPV_MT = 128;   // candidates per tile (MMA M)
 constexpr int GPV_NT = 256;   // observations per column tile (MMA N)
 constexpr int GPV_A_PIECE = (NLS_KB / 8) * GPV_MT * 16;   // 8 KB
 constexpr int GPV_B_PIECE = (NLS_KB / 8) * GPV_NT * 16;   // 16 KB
-constexpr int GPV_STAGE_BYTES = 2 * GPV_A_PIECE + 2 * GPV_B_PIECE;
 
-struct GpvDev {
-  const __half* kxh; const __half* kxl;   // [n_ptiles][KP / 8][128][8]
-  const __half* th; const __half* tl;     // [KP / 256][KP / 8][256][8]  L^-1 rows scaled per row
-  const float* tinv;                      // [KP] 1 / (row scale * kx scale)
-  int KP;                                 // n_obs padded to a multiple of 256
-  int n_ptiles;
-  int64_t n_points;                       // candidates in this chunk
-  float os_f;
-  double base;                            // sigma_f^2 + sigma_n^2
-  double* var_out;                        // [n_points]
-};
-
-struct GpvCfg {
-  static constexpr int NSTAGE = 4;
-  static constexpr int OFF_STAGE = 0;
-  static constexpr int OFF_TINV = NSTAGE * GPV_STAGE_BYTES;    // [8 epilogue warps][128] scale factors
-  static constexpr int OFF_COMB = OFF_TINV + NLS_EPI_WARPS * (GPV_NT / 2) * 4;
-  static constexpr int OFF_BAR = OFF_COMB + 128 * 8;
-  static constexpr int SMEM_BYTES = OFF_BAR + 256;
-  static_assert(SMEM_BYTES <= 227 * 1024, "gpvar: shared memory budget");
-};
-
-template <int VARIANT>   // a template only so that the header can be included from several translation units
-__global__ void __launch_bounds__(NLS_THREADS, 1) gpvar_kernel(const GpvDev a) {
-  using Cfg = GpvCfg;
-  constexpr int NSTAGE = Cfg::NSTAGE, NT = GPV_NT;
-  extern __shared__ __align__(1024) unsigned char smem_gpv[];
-  unsigned char* const smem = smem_gpv;
-  float* sTinv = reinterpret_cast<float*>(smem + Cfg::OFF_TINV);
-  double* sComb = reinterpret_cast<double*>(smem + Cfg::OFF_COMB);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::OFF_BAR);
-  uint64_t* s_full = bars;
-  uint64_t* s_empty = bars + NSTAGE;
-  uint64_t* t_full = bars + 2 * NSTAGE;
-  uint64_t* t_empty = t_full + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + 2);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (tid == 0) {
-    for (int s = 0; s < NSTAGE; ++s) {
-      mma::mbar_init(&s_full[s], 1);
-      mma::mbar_init(&s_empty[s], 1);
-    }
-    for (int b = 0; b < 2; ++b) {
-      mma::mbar_init(&t_full[b], 1);
-      mma::mbar_init(&t_empty[b], NLS_EPI_WARPS);
-    }
-    mma::fence_barrier_init();
-  }
-  if (warp == NLS_EPI_WARPS + 1) mma::tmem_alloc(tmem_slot, 512);
-  mma::tc_fence_before();
-  __syncthreads();
-  mma::tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const int n_ctiles = a.KP / NT;
-  auto nkb_of = [&](int c) { return min(a.KP, NT * (c + 1)) / NLS_KB; };   // K blocks up to the diagonal block
-
-  if (warp < NLS_EPI_WARPS) {
-    // ======================================================================== epilogue
-    const int quarter = warp & 3, half = warp >> 2;
-    const int row = quarter * 32 + lane;
-    uint32_t tc = 0;
-    for (int item = blockIdx.x; item < a.n_ptiles; item += gridDim.x) {
-      const int64_t p = (int64_t)item * GPV_MT + row;
-      double acc = 0.0;
-      for (int c = 0; c < n_ctiles; ++c, ++tc) {
-        const uint32_t buf = tc & 1u, ph = (tc >> 1) & 1u;
-        // the 128 scale factors of this warp's column half, staged per column tile in the warp's own slot
-        // (a table of all KP of them would bound the observation count); the __syncwarp before the
-        // previous t_empty arrival ordered the previous tile's reads
-        float* ti = sTinv + warp * (NT / 2);
-        reinterpret_cast<float4*>(ti)[lane] = reinterpret_cast<const float4*>(a.tinv + c * NT + half * (NT / 2))[lane];
-        __syncwarp();
-        mma::mbar_wait(&t_full[buf], ph);
-        mma::tc_fence_after();
-        const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + buf * NT + half * (NT / 2);
-#pragma unroll 1
-        for (int cb = 0; cb < NT / 2; cb += 32) {
-          uint32_t v[32];
-          mma::tmem_ld32(taddr + cb, v);
-          mma::tmem_ld_wait();
-          float part = 0.f;   // 32 squares in fp32, widened once per block
-#pragma unroll
-          for (int cc = 0; cc < 32; ++cc) {
-            const float vo = __fmul_rn(__uint_as_float(v[cc]), ti[cb + cc]);
-            part = __fmaf_rn(vo, vo, part);
-          }
-          acc += (double)part;
-        }
-        mma::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mma::mbar_arrive(&t_empty[buf]);
-      }
-      // combine the two column halves
-      if (half == 1) sComb[row] = acc;
-      mma::named_bar_sync(1, NLS_EPI_WARPS * 32);
-      if (half == 0 && p < a.n_points) a.var_out[p] = a.base - (acc + sComb[row]);
-      mma::named_bar_sync(2, NLS_EPI_WARPS * 32);   // sComb is reused by the next item
-    }
-  } else if (warp == NLS_EPI_WARPS) {
-    // ======================================================================== operand producer
-    if (lane == 0) {
-      uint32_t it = 0;
-      const size_t a_tile = (size_t)(a.KP / 8) * GPV_MT * 8;
-      const size_t b_tile = (size_t)(a.KP / 8) * NT * 8;
-      for (int item = blockIdx.x; item < a.n_ptiles; item += gridDim.x) {
-        for (int c = 0; c < n_ctiles; ++c) {
-          const int nkb = nkb_of(c);
-          for (int kb = 0; kb < nkb; ++kb, ++it) {
-            const int s = it % NSTAGE;
-            mma::mbar_wait(&s_empty[s], ((it / NSTAGE) & 1u) ^ 1u);
-            unsigned char* st = smem + Cfg::OFF_STAGE + (size_t)s * GPV_STAGE_BYTES;
-            mma::mbar_expect_tx(&s_full[s], GPV_STAGE_BYTES);
-            const size_t ka = (size_t)kb * (GPV_A_PIECE / 2), kbo = (size_t)kb * (GPV_B_PIECE / 2);
-            mma::bulk_g2s(st, a.kxh + item * a_tile + ka, GPV_A_PIECE, &s_full[s]);
-            mma::bulk_g2s(st + GPV_A_PIECE, a.kxl + item * a_tile + ka, GPV_A_PIECE, &s_full[s]);
-            mma::bulk_g2s(st + 2 * GPV_A_PIECE, a.th + c * b_tile + kbo, GPV_B_PIECE, &s_full[s]);
-            mma::bulk_g2s(st + 2 * GPV_A_PIECE + GPV_B_PIECE, a.tl + c * b_tile + kbo, GPV_B_PIECE, &s_full[s]);
-          }
-        }
-      }
-    }
-  } else if (warp == NLS_EPI_WARPS + 1) {
-    // ======================================================================== MMA issuer
-    constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(NT >> 3) << 17) | ((128u >> 4) << 24);
-    uint32_t it = 0, tc = 0;
-    for (int item = blockIdx.x; item < a.n_ptiles; item += gridDim.x) {
-      for (int c = 0; c < n_ctiles; ++c, ++tc) {
-        const uint32_t buf = tc & 1u;
-        const int nkb = nkb_of(c);
-        mma::mbar_wait(&t_empty[buf], ((tc >> 1) & 1u) ^ 1u);
-        mma::tc_fence_after();
-        for (int kb = 0; kb < nkb; ++kb, ++it) {
-          const int s = it % NSTAGE;
-          mma::mbar_wait(&s_full[s], (it / NSTAGE) & 1u);
-          mma::tc_fence_after();
-          if (lane == 0) {
-            const uint32_t st = mma::smem_u32(smem + Cfg::OFF_STAGE + (size_t)s * GPV_STAGE_BYTES);
-            const uint32_t ahi = st, alo = st + GPV_A_PIECE;
-            const uint32_t bhi = st + 2 * GPV_A_PIECE, blo = bhi + GPV_B_PIECE;
-            const uint32_t d = tmem_base + buf * NT;
-#pragma unroll
-            for (int p = 0; p < 3; ++p) {
-              const uint32_t aa = (p == 0) ? alo : ahi;
-              const uint32_t bb = (p == 1) ? blo : bhi;
-#pragma unroll
-              for (int ks = 0; ks < NLS_KB / 16; ++ks) {
-                const uint64_t ad = mma::smem_desc(aa + ks * 2 * (GPV_MT * 16), GPV_MT * 16, 128);
-                const uint64_t bd = mma::smem_desc(bb + ks * 2 * (NT * 16), NT * 16, 128);
-                umma_f16(d, ad, bd, IDESC, (kb > 0 || p > 0 || ks > 0) ? 1u : 0u);
-              }
-            }
-            mma::umma_commit(&s_empty[s]);
-            if (kb == nkb - 1) mma::umma_commit(&t_full[buf]);
-          }
-          __syncwarp();
-        }
-      }
-    }
-  }
-
-  mma::tc_fence_before();
-  __syncthreads();
-  if (warp == NLS_EPI_WARPS + 1) {
-    mma::tc_fence_after();
-    mma::tmem_dealloc(tmem_base, 512);
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Fully fused version: k(Xobs, x) never leaves the SM.  Eight generator warps (two threads per candidate of
-// the tile) evaluate the kernel values of one 32-observation K block, split them into fp16 hi / lo and
-// store them straight into the A stage in the tcgen05 K-major layout; the MMA warp contracts the stage
-// against the L^-1 tiles of TWO observation column tiles at once (two 256-column accumulators = all of
-// TMEM), so a K block is generated once per pair of column tiles (1.5x the unique evaluations at four
-// column tiles; they cost a third of the MMA time and hide under it).  DRAM traffic: the candidates in
-// (4 d B each), the variances out (8 B each).
-//   warps 0-7   generators (measured: four warps generate as slowly as the MMAs run; eight hide under them)
-//   warps 8-15  epilogue (TMEM lane quarter = warp % 4, two column halves)
-//   warp 16     L^-1 tile producer (cp.async.bulk, 32 KB units: hi / lo of one column tile's K block)
-//   warp 17     TMEM allocation + tcgen05.mma issue
-// ---------------------------------------------------------------------------------------------
 constexpr int GPF_GEN_WARPS = 8, GPF_EPI_WARPS = 8;   // two generator threads per candidate row (16 of a K block's 32 observations each)
 constexpr int GPF_THREADS = (GPF_GEN_WARPS + GPF_EPI_WARPS + 2) * 32;
 constexpr int GPF_A_STAGE = 2 * GPV_A_PIECE;          // hi + lo of one generated K block: 16 KB
@@ -586,102 +408,5 @@ int launch_gpvar_fused_family(basq_ctx* ctx, const KParams& kp, const GpfDev& de
 int launch_gpvar_fused_rbf(basq_ctx*, const KParams&, const GpfDev&);
 int launch_gpvar_fused_m15(basq_ctx*, const KParams&, const GpfDev&);
 int launch_gpvar_fused_m25(basq_ctx*, const KParams&, const GpfDev&);
-
-// k(Xobs, x) of a chunk of raw candidates as the A operand ([tile of 128][KP / 8][128][8] fp16 hi / lo);
-// one CTA per tile, one thread per candidate.
-struct KxpDev {
-  const float* X;          // [n_points, d] raw candidates of the chunk
-  int64_t n_points;
-  const float* ozz; const float* obz;
-  int n_obs, KP;
-  float kx_scale;
-  __half* kxh; __half* kxl;
-};
-
-template <int FAM, int DP>
-__global__ void __launch_bounds__(GPV_MT) kxgen_points_kernel(KParams kp, const KxpDev a) {
-  constexpr int OB = 64;
-  __shared__ __align__(16) float s_oz[OB * DP];
-  __shared__ float s_ob[OB];
-  const int tile = blockIdx.x, r = threadIdx.x;
-  const int64_t p = (int64_t)tile * GPV_MT + r;
-  const bool ok = p < a.n_points;
-  float x[DP];
-  float pa = 0.f;
-#pragma unroll
-  for (int i = 0; i < DP; ++i) x[i] = 0.f;
-  if (ok) {
-    float xl[BASQ_MAX_DIM];
-    float nrm;
-    prep_point_f32(kp, a.X + p * kp.d, xl, &nrm);
-#pragma unroll
-    for (int i = 0; i < DP; ++i) x[i] = xl[i];
-    pa = point_a_term(kp, nrm);
-  }
-  const size_t a_tile = (size_t)(a.KP / 8) * GPV_MT * 8;
-  uint4* oh = reinterpret_cast<uint4*>(a.kxh + (size_t)tile * a_tile) + r;
-  uint4* ol = reinterpret_cast<uint4*>(a.kxl + (size_t)tile * a_tile) + r;
-  for (int o0 = 0; o0 < a.KP; o0 += OB) {
-    __syncthreads();
-    for (int i = threadIdx.x; i < OB * DP; i += GPV_MT) {
-      const int o = o0 + i / DP;
-      s_oz[i] = o < a.n_obs ? a.ozz[(size_t)o * DP + i % DP] : 0.f;
-    }
-    if (threadIdx.x < OB) s_ob[threadIdx.x] = (o0 + (int)threadIdx.x < a.n_obs) ? a.obz[o0 + threadIdx.x] : 0.f;
-    __syncthreads();
-    for (int kc = 0; kc < OB / 8; ++kc) {
-      __half2 h2[4], l2[4];
-#pragma unroll
-      for (int u = 0; u < 8; u += 2) {
-        float vv[2];
-#pragma unroll
-        for (int w = 0; w < 2; ++w) {
-          const int ol_ = kc * 8 + u + w;
-          float kv = 0.f;
-          if (ok && o0 + ol_ < a.n_obs) kv = pair_eval_f32<FAM, DP>(x, pa, &s_oz[ol_ * DP], s_ob[ol_], kp.os_f);
-          vv[w] = __fmul_rn(kv, a.kx_scale);
-        }
-        const __half h0 = __float2half_rn(vv[0]), h1 = __float2half_rn(vv[1]);
-        h2[u / 2] = __halves2half2(h0, h1);
-        l2[u / 2] = __halves2half2(__float2half_rn(__fsub_rn(vv[0], __half2float(h0))),
-                                   __float2half_rn(__fsub_rn(vv[1], __half2float(h1))));
-      }
-      const size_t chunk = (size_t)(o0 / 8 + kc) * GPV_MT;
-      oh[chunk] = *reinterpret_cast<const uint4*>(h2);
-      ol[chunk] = *reinterpret_cast<const uint4*>(l2);
-    }
-  }
-}
-
-template <int FAM, int DP>
-int launch_kxgen_points_dp(basq_ctx* ctx, const KParams& kp, const KxpDev& kx, int n_ptiles) {
-  if (n_ptiles <= 0) return BASQ_OK;
-  kxgen_points_kernel<FAM, DP><<<n_ptiles, GPV_MT, 0, ctx->stream>>>(kp, kx);
-  ctx->launches++;
-  BASQ_CUDA(cudaGetLastError());
-  return BASQ_OK;
-}
-
-template <int FAM>
-int launch_kxgen_points_family(basq_ctx* ctx, const KParams& kp, const KxpDev& kx, int n_ptiles) {
-  switch (kp.dp) {
-    case 2: return launch_kxgen_points_dp<FAM, 2>(ctx, kp, kx, n_ptiles);
-    case 4: return launch_kxgen_points_dp<FAM, 4>(ctx, kp, kx, n_ptiles);
-    case 6: return launch_kxgen_points_dp<FAM, 6>(ctx, kp, kx, n_ptiles);
-    case 8: return launch_kxgen_points_dp<FAM, 8>(ctx, kp, kx, n_ptiles);
-    case 10: return launch_kxgen_points_dp<FAM, 10>(ctx, kp, kx, n_ptiles);
-    case 12: return launch_kxgen_points_dp<FAM, 12>(ctx, kp, kx, n_ptiles);
-    case 16: return launch_kxgen_points_dp<FAM, 16>(ctx, kp, kx, n_ptiles);
-    case 20: return launch_kxgen_points_dp<FAM, 20>(ctx, kp, kx, n_ptiles);
-    case 24: return launch_kxgen_points_dp<FAM, 24>(ctx, kp, kx, n_ptiles);
-    case 32: return launch_kxgen_points_dp<FAM, 32>(ctx, kp, kx, n_ptiles);
-  }
-  set_error("gpvar: no kernel compiled for padded dimension %d", kp.dp);
-  return BASQ_ERR_UNSUPPORTED;
-}
-
-int launch_kxgen_points_rbf(basq_ctx*, const KParams&, const KxpDev&, int);
-int launch_kxgen_points_m15(basq_ctx*, const KParams&, const KxpDev&, int);
-int launch_kxgen_points_m25(basq_ctx*, const KParams&, const KxpDev&, int);
 
 }  // namespace basq

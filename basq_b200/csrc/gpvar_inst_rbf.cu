@@ -1,9 +1,6 @@
-// gpvar_fused_kernel / kxgen_points_kernel instantiations: rbf (see gpvar.cuh)
+// gpvar_fused_kernel instantiations: rbf (see gpvar.cuh)
 #include "gpvar.cuh"
 namespace basq {
-int launch_kxgen_points_rbf(basq_ctx* ctx, const KParams& kp, const KxpDev& kx, int n_ptiles) {
-  return launch_kxgen_points_family<BASQ_RBF>(ctx, kp, kx, n_ptiles);
-}
 int launch_gpvar_fused_rbf(basq_ctx* ctx, const KParams& kp, const GpfDev& dev) {
   return launch_gpvar_fused_family<BASQ_RBF>(ctx, kp, dev);
 }

@@ -323,10 +323,9 @@ int gp_predict_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& 
     return BASQ_OK;
   }
   if (mean_out) {
-    static const bool mean_tc = [] { const char* e = getenv("BASQ_GPMEAN_TC"); return !(e && e[0] == '0'); }();
     // the choice depends on the GP only, never on N: the per-point factors of the warped kernels must come out
     // bit-identical for the 1e7 candidates of a session and for the handful of points of a feature / Gram call
-    if (mean_tc && desc->dtype == BASQ_F32 && N > 0 && desc->n_obs >= 64 && !ctx->scalar_setsum)
+    if (desc->dtype == BASQ_F32 && N > 0 && desc->n_obs >= 64)
       BASQ_TRY(landmark_dot_tc(ctx, kp, desc->Xobs, desc->n_obs, desc->alpha, desc->mean_const, X, N, mean_out));
     else
       BASQ_TRY(landmark_dot(ctx, kp, lmobs, desc->alpha, desc->mean_const, X, N, mean_out));

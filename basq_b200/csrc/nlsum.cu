@@ -5,7 +5,7 @@
 
 #include <algorithm>
 
-#include "nlsum2.cuh"
+#include "nlsum.cuh"
 
 namespace basq {
 
@@ -27,15 +27,6 @@ int launch_nlsum(basq_ctx* ctx, int fam, int nl, int dp, const NlsDev& dev, int 
   }
 }
 
-int launch_nlsum2(basq_ctx* ctx, int fam, int nl, int dp, const NlsDev& dev) {
-  const bool wm = (nl == NL_WSABIM);
-  switch (fam) {
-    case BASQ_RBF: return wm ? launch_nlsum2_rbf_wm(ctx, dp, dev) : launch_nlsum2_rbf_ml(ctx, dp, dev);
-    case BASQ_MATERN15: return wm ? launch_nlsum2_m15_wm(ctx, dp, dev) : launch_nlsum2_m15_ml(ctx, dp, dev);
-    default: return wm ? launch_nlsum2_m25_wm(ctx, dp, dev) : launch_nlsum2_m25_ml(ctx, dp, dev);
-  }
-}
-
 int launch_kxgen(basq_ctx* ctx, int fam, int dp, const KxDev& dev) {
   switch (fam) {
     case BASQ_RBF: return launch_kxgen_rbf(ctx, dp, dev);
@@ -49,7 +40,7 @@ int nls_prepare(basq_ctx* ctx, const KParams& kp, const double* Az, int M, int n
   op->M = M;
   op->n_obs = n_obs;
   op->KP = ceil_div(n_obs, NLS_KB) * NLS_KB;
-  op->n_mtiles = (ceil_div(M, 128) + 1) / 2 * 2;   // even: CTA pairs take two landmark tiles (nlsum2.cuh)
+  op->n_mtiles = ceil_div(M, 128);
   op->kx_scale = ldexpf(1.f, NLS_KX_SHIFT - (int)ceil(log2(kp.outputscale)));
   const size_t halves = (size_t)op->n_mtiles * (op->KP / 8) * 128 * 8;
   BASQ_TRY(op->azh.alloc(ctx, halves * 2));
@@ -85,10 +76,6 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
   // every cell has at most one member of the range: one column per cell (GRAM); else 8 sets x 32 members
   const bool gram = (p_hi - p_lo) <= (int64_t)S;
   const int JT = gram ? NLS_NT : NLS_JT, EC = NLS_NT / JT;
-  // BASQ_NLS_2CTA=1: set sums on CTA pairs (tcgen05 cta_group::2, nlsum2.cuh).  Measured slower than the
-  // one-CTA kernel (684 vs 625 ms for the config-5 sweep: tensor pipe 52 % vs 66 % active - the cross-CTA
-  // full / empty hand-shake costs more than the halved B stream saves), so it stays opt-in.
-  const bool pairs = !gram && ctx->num_sms >= 2 && ([] { const char* e = getenv("BASQ_NLS_2CTA"); return e && e[0] == '1'; }());
   const int n_jg_total = ceil_div(S, JT);
   // tile stride: an upper bound of any group's tile count.  The kernels start group g at
   // e_lo = ceil((p_lo + off - (g JT + JT - 1)) / S); the last group's column n_jg_total JT - 1 may exceed
@@ -126,7 +113,6 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
     kx.ozz = reinterpret_cast<const float*>(lmobs.zz); kx.obz = lmobs.b;
     kx.n_obs = op->n_obs; kx.KP = op->KP;
     kx.os_f = kp.os_f; kx.kx_scale = op->kx_scale;
-    kx.split_half = pairs ? 1 : 0;
     kx.kxh = op->kxh.as<__half>(); kx.kxl = op->kxl.as<__half>(); kx.trec = op->trec.as<unsigned char>();
     BASQ_TRY(launch_kxgen(ctx, kp.family, kp.dp, kx));
     NlsDev d;
@@ -137,8 +123,7 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
     d.zz = reinterpret_cast<const float*>(lmz.zz); d.bz = lmz.b; d.szf = op->szf.as<float>();
     d.M = op->M; d.n_mtiles = op->n_mtiles; d.os_f = kp.os_f;
     d.G = G; d.ldg = ldg;
-    if (pairs) BASQ_TRY(launch_nlsum2(ctx, kp.family, nl, kp.dp, d));
-    else BASQ_TRY(launch_nlsum(ctx, kp.family, nl, kp.dp, d, gram ? 1 : 0));
+    BASQ_TRY(launch_nlsum(ctx, kp.family, nl, kp.dp, d, gram ? 1 : 0));
   }
   return BASQ_OK;
 }

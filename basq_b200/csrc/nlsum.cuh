@@ -387,7 +387,6 @@ struct KxDev {
   int n_obs, KP;
   float os_f;
   float kx_scale;                       // 2^(14 - ceil(log2 os))
-  int split_half;                       // 0: [tile][K / 8][256][8] ; 1: [tile][half][K / 8][128][8] (CTA pairs, nlsum2.cuh)
   __half* kxh; __half* kxl;
   unsigned char* trec;
 };
@@ -443,11 +442,8 @@ __global__ void __launch_bounds__(NLS_NT) kxgen_kernel(const KxDev a) {
     for (int i = 0; i < DP; ++i) x[i] = f[2 + i];
   }
   const size_t b_tile = (size_t)(a.KP / 8) * NLS_NT * 8;
-  // chunk kc lies kc * rows uint4 further (rows = 256, or 128 within the slot's half)
-  const int rows = a.split_half ? NLS_NT / 2 : NLS_NT;
-  const size_t slot0 = a.split_half ? (size_t)(c >> 7) * (b_tile / 8 / 2) + (c & 127) : (size_t)c;
-  uint4* oh = reinterpret_cast<uint4*>(a.kxh + (size_t)tile * b_tile) + slot0;
-  uint4* ol = reinterpret_cast<uint4*>(a.kxl + (size_t)tile * b_tile) + slot0;
+  uint4* oh = reinterpret_cast<uint4*>(a.kxh + (size_t)tile * b_tile) + c;
+  uint4* ol = reinterpret_cast<uint4*>(a.kxl + (size_t)tile * b_tile) + c;
   for (int o0 = 0; o0 < a.KP; o0 += OB) {
     __syncthreads();
     for (int i = threadIdx.x; i < OB * DP; i += NLS_NT) {
@@ -474,7 +470,7 @@ __global__ void __launch_bounds__(NLS_NT) kxgen_kernel(const KxDev a) {
         l2[u / 2] = __halves2half2(__float2half_rn(__fsub_rn(vv[0], __half2float(h0))),
                                    __float2half_rn(__fsub_rn(vv[1], __half2float(h1))));
       }
-      const size_t chunk = (size_t)(o0 / 8 + kc) * rows;
+      const size_t chunk = (size_t)(o0 / 8 + kc) * NLS_NT;
       oh[chunk] = *reinterpret_cast<const uint4*>(h2);
       ol[chunk] = *reinterpret_cast<const uint4*>(l2);
     }

@@ -597,7 +597,7 @@ int nystrom_basis(basq_ctx* ctx, const basq_kernel_desc* desc, const void* Z, in
   // Y_out [M, q] = K Y_in.  fp32 kernels: on the tensor cores (fp16 hi/lo split products, tgemm.cu) - the Gram matrix itself
   // is only fp32-accurate, and the subspace iteration re-orthonormalises in fp64 after every product;
   // fp64 kernels: fp64 GEMM.  K is symmetric, so K^T Y = K Y.
-  const bool tensor = (desc->dtype == BASQ_F32) && !ctx->no_tensor_nystrom;
+  const bool tensor = desc->dtype == BASQ_F32;
   BASQ_TRY(gram_matrix(ctx, desc, Z, M, Z, M, K.as<double>(), tensor));
   BlkOperand Kb, Yb;
   if (tensor) {
@@ -704,7 +704,7 @@ int nystrom_basis_sharded(basq_ctx* ctx, const basq_kernel_desc* desc, const voi
   BASQ_TRY(ws.flags.alloc(ctx, 512));
   BASQ_CUDA(cudaMemsetAsync(ws.flags.p, 0, 512, ctx->stream));
   BASQ_TRY(ws.scal.alloc(ctx, 64));
-  const bool tensor = (desc->dtype == BASQ_F32) && !ctx->no_tensor_nystrom;
+  const bool tensor = desc->dtype == BASQ_F32;
   BlkOperand Kb, Yb;
   if (nr > 0) {
     const unsigned char* Zr = static_cast<const unsigned char*>(Z) + (size_t)row0 * desc->d * esz;

@@ -32,7 +32,7 @@ int set_sums(basq_ctx* ctx, const KParams& kp, const SetSumArgs& a) {
   dev.G = a.G;
   dev.ldg = a.ldg;
   dev.accumulate = a.accumulate ? 1 : 0;
-  if (pool.dtype == BASQ_F32 && a.nl == NL_LIN && lm.lmA != nullptr && !ctx->scalar_setsum) {
+  if (pool.dtype == BASQ_F32 && a.nl == NL_LIN && lm.lmA != nullptr) {
     // fp32 linear modes: argument tiles on the tensor cores (setsum_mma.cuh)
     SetSumMmaDev md;
     md.recs = dev.recs;

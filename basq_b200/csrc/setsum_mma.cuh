@@ -5,10 +5,12 @@
 // The exponent argument of every kernel family is bilinear in prepared operands,
 //   arg(m, p) = a_p + b_m + sum_i x'_{p,i} zz_{m,i}        (see common.cuh: KParams),
 // so a 128-landmark x NT-point tile of arguments is ONE small GEMM with K = 3 DP + 6 (padded to the MMA's K step):
-//   * x' and zz are split into "hi + lo" parts with 11 significant bits each - fp16 by default
-//     (BASQ_SETSUM_F16, kind::f16: K = 48 at d = 10, three MMAs per tile), tf32 in round 1 (kind::tf32, K = 40,
-//     five MMAs) - and the three significant cross products (hi hi, lo hi, hi lo) occupy three K columns per
-//     dimension (~2^-21 relative);
+//   * x' and zz are split into fp16 "hi + lo" parts with 11 significant bits each (kind::f16: K = 48 at
+//     d = 10, three MMAs per tile), and the three significant cross products (hi hi, lo hi, hi lo) occupy
+//     three K columns per dimension (~2^-21 relative).  fp16's range is enough for centred,
+//     lengthscale-scaled coordinates (values beyond +-6e4 are clamped: such pairs have k = 0 either way);
+//     pieces below 6e-5 lose bits to the subnormal spacing 6e-8, an absolute 3e-8 |zz| per term of the
+//     argument - below its fp32 rounding;
 //   * a_p and b_m ride along as three pieces each against constant-one columns.
 // tcgen05.mma (M = 128, N = NT, operands K-major in shared memory, no swizzle) writes the
 // argument tile into TMEM; the epilogue warps read it back with tcgen05.ld, apply exp2 / the Matern
@@ -40,7 +42,7 @@ struct SetSumMmaDev {
   int64_t off;
   int S;
   int64_t p_lo, p_hi;
-  const float* lmA;  // [n_mtiles_alloc][KA/4][128][4] landmark operand, tile-blocked
+  const float* lmA;  // [n_mtiles_alloc][KA/8][128][8 halves] landmark operand, tile-blocked
   int Mtot;
   int n_mgroups;     // ceil(Mtot / (MT * 128))
   int n_jgroups;     // ceil(S / JT)
@@ -50,37 +52,17 @@ struct SetSumMmaDev {
   int accumulate;
 };
 
-// BASQ_SETSUM_F16 = 1 (default): the split operands are fp16 (kind::f16, K = 16 per MMA) instead of tf32
-// (kind::tf32, K = 8): the same 11 significant bits per piece, half the bytes, 3 instead of 5 MMAs per
-// 128 x 256 tile at d = 10.  fp16's range is enough for centred, lengthscale-scaled coordinates (values
-// beyond +-6e4 are clamped: such pairs have k = 0 either way); pieces below 6e-5 lose bits to the
-// subnormal spacing 6e-8, an absolute 3e-8 |zz| per term of the argument - below its fp32 rounding.
-#ifndef BASQ_SETSUM_F16
-#define BASQ_SETSUM_F16 1
-#endif
-
-// BASQ_SETSUM_POLY_ROWS = r (0..4): of the four landmark rows a thread owns, r evaluate exp2 with a
-// degree-6 polynomial on the FMA pipe (Cody-Waite split, 1.1e-7 relative, like ex2.approx) instead of the
-// MUFU: the choice depends on the landmark only, so k(z, x) stays bit-identical across passes.
-#ifndef BASQ_SETSUM_POLY_ROWS
-#define BASQ_SETSUM_POLY_ROWS 0
-#endif
-
 template <int DP>
 struct MmaCfg {
-  static constexpr bool F16 = BASQ_SETSUM_F16 != 0;
-  static constexpr int KSTEP = F16 ? 16 : 8;           // K of one MMA
-  static constexpr int ESZ = F16 ? 2 : 4;              // bytes per operand element
-  static constexpr int CH = 16 / ESZ;                  // elements per 16-byte K chunk
-  static constexpr int KA = (3 * DP + 6 + KSTEP - 1) / KSTEP * KSTEP;  // K columns (multiple of the MMA K)
-  static constexpr int NT = KA * ESZ <= 160 ? 256 : 128;  // points per tile (MMA N)
-  static constexpr int MT = KA * ESZ > 320 ? 1 : 2;       // landmark tiles (of 128) per work item
+  static constexpr int KA = (3 * DP + 6 + 15) / 16 * 16;  // K columns (multiple of the MMA K, 16)
+  static constexpr int NT = KA <= 80 ? 256 : 128;      // points per tile (MMA N)
+  static constexpr int MT = KA > 160 ? 1 : 2;          // landmark tiles (of 128) per work item
   static constexpr int JT = 8;                         // sets per work item
   static constexpr int EC = NT / JT;                   // set members per tile
   static constexpr int NSTAGE = 3;
   static constexpr int RB = ((24 + 4 * DP) + 15) / 16 * 16;  // record bytes (rec_bytes_f32)
-  static constexpr int A_TILE_BYTES = KA * 128 * ESZ;
-  static constexpr int B_STAGE_BYTES = KA * NT * ESZ;
+  static constexpr int A_TILE_BYTES = KA * 128 * 2;   // fp16 operands
+  static constexpr int B_STAGE_BYTES = KA * NT * 2;
   static constexpr int W_STAGE_BYTES = NT * 8;
 #ifndef BASQ_EPI_WARPS
 #define BASQ_EPI_WARPS 16
@@ -155,18 +137,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
 }
-// D[tmem] (+)= A[smem] * B[smem]^T, tf32 inputs, fp32 accumulate
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-      "}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // D[tmem] (+)= A[smem] * B[smem]^T, fp16 inputs, fp32 accumulate
 __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
                                          uint32_t accumulate) {
@@ -179,7 +149,7 @@ __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// K-major operand without swizzle, stored as [K / 4][rows][4 floats]: 8-row core matrices are
+// K-major operand without swizzle, stored as [K / 8][rows][8 halves]: 8-row core matrices are
 // contiguous (SBO = 128 B), the next 16-byte K chunk lies one plane further (LBO = rows * 16 B).
 __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
@@ -188,11 +158,6 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes
   d |= (uint64_t)(sbo_bytes >> 4) << 32;
   d |= (uint64_t)1 << 46;  // descriptor version (Blackwell)
   return d;
-}
-__device__ __forceinline__ float tf32_rna(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return __uint_as_float(r);
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
@@ -225,14 +190,6 @@ __device__ __forceinline__ void named_bar_arrive(int id, int nthreads) {
   asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-// the three tf32 pieces of an fp32 value (sum reproduces it to ~2^-33 relative)
-__device__ __forceinline__ void split3(float v, float& p1, float& p2, float& p3) {
-  p1 = tf32_rna(v);
-  const float r = __fsub_rn(v, p1);
-  p2 = tf32_rna(r);
-  p3 = tf32_rna(__fsub_rn(r, p2));
-}
-
 // fp16 pieces of an fp32 value: hi = the value cut to 11 significant bits (exact in fp16 within its normal
 // range), lo = the remainder rounded to fp16 (sum reproduces the value to ~2^-22); values are clamped to
 // fp16's range first
@@ -251,35 +208,10 @@ __device__ __forceinline__ void split3h(float v, __half& p1, __half& p2, __half&
   p3 = __float2half_rn(__fsub_rn(r, __half2float(p2)));
 }
 
-// 2^x on the FMA / ALU pipes: x = n + f, n = round(x), |f| <= 1/2; degree-6 minimax of 2^f (1.1e-7 relative
-// including the fp32 Horner rounding); the exponent is added to the bit pattern (n sits in the low mantissa
-// bits of x + 1.5 * 2^23).  12 instructions; no MUFU.
-__device__ __forceinline__ float exp2_poly(float x) {
-  x = fmaxf(x, -125.f);
-  const float r = __fadd_rn(x, 12582912.f);
-  const float f = __fsub_rn(x, __fsub_rn(r, 12582912.f));
-  float p = 0.000154697319723078f;
-  p = __fmaf_rn(p, f, 0.0013400432165225804f);
-  p = __fmaf_rn(p, f, 0.009618025602985998f);
-  p = __fmaf_rn(p, f, 0.05550327214209406f);
-  p = __fmaf_rn(p, f, 0.2402265121359483f);
-  p = __fmaf_rn(p, f, 0.6931472067106204f);
-  p = __fmaf_rn(p, f, 0.9999999999595486f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(r) << 23));
-}
-
 }  // namespace mma
 
-// kernel value from the exponent argument: MUFU path (finish_f32) or, for RBF rows selected at compile
-// time, the FMA-pipe polynomial
-template <int FAM, bool POLY>
-__device__ __forceinline__ float finish_sel(float acc, float os_f) {
-  if (FAM == BASQ_RBF && POLY) return mma::exp2_poly(acc);
-  return finish_f32(FAM, acc, os_f);
-}
-
 // ---------------------------------------------------------------------------------------------
-// landmark operand: lmA[tile][kc][row][4] from the prepared zz [Mtot, DP] / b [Mtot]
+// landmark operand: lmA[tile][kc][row][8 halves] from the prepared zz [Mtot, DP] / b [Mtot]
 //   K column 3i   : zz_hi_i   (x hi)      3i+1 : zz_hi_i  (x lo)      3i+2 : zz_lo_i  (x hi)
 //   3DP .. 3DP+2  : 1 (a pieces)          3DP+3 .. 3DP+5 : b pieces (x 1)      rest : 0
 // ---------------------------------------------------------------------------------------------
@@ -291,47 +223,24 @@ __global__ void build_lmA_kernel(const float* __restrict__ zz, const float* __re
   const int m = blockIdx.x * blockDim.x + threadIdx.x;
   if (m >= n_tiles * 128) return;
   const int tile = m >> 7, row = m & 127;
-  if constexpr (Cfg::F16) {
-    __half vals[KA];
+  __half vals[KA];
 #pragma unroll
-    for (int k = 0; k < KA; ++k) vals[k] = __float2half_rn(0.f);
-    if (m < Mtot) {
+  for (int k = 0; k < KA; ++k) vals[k] = __float2half_rn(0.f);
+  if (m < Mtot) {
 #pragma unroll
-      for (int i = 0; i < DP; ++i) {
-        __half zh, zl;
-        mma::split2h(zz[(int64_t)m * DP + i], zh, zl);
-        vals[3 * i] = zh;
-        vals[3 * i + 1] = zh;
-        vals[3 * i + 2] = zl;
-      }
-      vals[3 * DP] = vals[3 * DP + 1] = vals[3 * DP + 2] = __float2half_rn(1.f);
-      mma::split3h(bz[m], vals[3 * DP + 3], vals[3 * DP + 4], vals[3 * DP + 5]);
+    for (int i = 0; i < DP; ++i) {
+      __half zh, zl;
+      mma::split2h(zz[(int64_t)m * DP + i], zh, zl);
+      vals[3 * i] = zh;
+      vals[3 * i + 1] = zh;
+      vals[3 * i + 2] = zl;
     }
-    uint4* dst = reinterpret_cast<uint4*>(lmA) + (int64_t)tile * (KA / 8) * 128 + row;
-#pragma unroll
-    for (int kc = 0; kc < KA / 8; ++kc) dst[kc * 128] = *reinterpret_cast<const uint4*>(&vals[8 * kc]);
-  } else {
-    float vals[KA];
-#pragma unroll
-    for (int k = 0; k < KA; ++k) vals[k] = 0.f;
-    if (m < Mtot) {
-#pragma unroll
-      for (int i = 0; i < DP; ++i) {
-        const float z = zz[(int64_t)m * DP + i];
-        const float zh = mma::tf32_rna(z);
-        const float zl = mma::tf32_rna(__fsub_rn(z, zh));
-        vals[3 * i] = zh;
-        vals[3 * i + 1] = zh;
-        vals[3 * i + 2] = zl;
-      }
-      vals[3 * DP] = vals[3 * DP + 1] = vals[3 * DP + 2] = 1.f;
-      mma::split3(bz[m], vals[3 * DP + 3], vals[3 * DP + 4], vals[3 * DP + 5]);
-    }
-    float4* dst = reinterpret_cast<float4*>(lmA) + (int64_t)tile * (KA / 4) * 128 + row;
-#pragma unroll
-    for (int kc = 0; kc < KA / 4; ++kc)
-      dst[kc * 128] = make_float4(vals[4 * kc], vals[4 * kc + 1], vals[4 * kc + 2], vals[4 * kc + 3]);
+    vals[3 * DP] = vals[3 * DP + 1] = vals[3 * DP + 2] = __float2half_rn(1.f);
+    mma::split3h(bz[m], vals[3 * DP + 3], vals[3 * DP + 4], vals[3 * DP + 5]);
   }
+  uint4* dst = reinterpret_cast<uint4*>(lmA) + (int64_t)tile * (KA / 8) * 128 + row;
+#pragma unroll
+  for (int kc = 0; kc < KA / 8; ++kc) dst[kc * 128] = *reinterpret_cast<const uint4*>(&vals[8 * kc]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -437,20 +346,13 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
               const double2 w2 = *reinterpret_cast<const double2*>(wst + cb + 8 * k);
 #pragma unroll
               for (int h = 0; h < 2; ++h) {
-                // row slots 2 h and 2 h + 1; the last BASQ_SETSUM_POLY_ROWS slots take the FMA-pipe exp2
-                constexpr int PR = BASQ_SETSUM_POLY_ROWS;
+                // row slots 2 h and 2 h + 1
                 const float u00 = __uint_as_float(h ? vb[4 * k + 0] : va[4 * k + 0]);
                 const float u01 = __uint_as_float(h ? vb[4 * k + 1] : va[4 * k + 1]);
                 const float u10 = __uint_as_float(h ? vb[4 * k + 2] : va[4 * k + 2]);
                 const float u11 = __uint_as_float(h ? vb[4 * k + 3] : va[4 * k + 3]);
-                float k00, k01, k10, k11;
-                if (h == 0) {
-                  k00 = finish_sel<FAM, (PR >= 4)>(u00, a.os_f); k01 = finish_sel<FAM, (PR >= 4)>(u01, a.os_f);
-                  k10 = finish_sel<FAM, (PR >= 3)>(u10, a.os_f); k11 = finish_sel<FAM, (PR >= 3)>(u11, a.os_f);
-                } else {
-                  k00 = finish_sel<FAM, (PR >= 2)>(u00, a.os_f); k01 = finish_sel<FAM, (PR >= 2)>(u01, a.os_f);
-                  k10 = finish_sel<FAM, (PR >= 1)>(u10, a.os_f); k11 = finish_sel<FAM, (PR >= 1)>(u11, a.os_f);
-                }
+                const float k00 = finish_f32(FAM, u00, a.os_f), k01 = finish_f32(FAM, u01, a.os_f);
+                const float k10 = finish_f32(FAM, u10, a.os_f), k11 = finish_f32(FAM, u11, a.os_f);
                 acc[mt][2 * h][0] = fma(f2d_pos(k00), w2.x, acc[mt][2 * h][0]);
                 acc[mt][2 * h][1] = fma(f2d_pos(k01), w2.y, acc[mt][2 * h][1]);
                 acc[mt][2 * h + 1][0] = fma(f2d_pos(k10), w2.x, acc[mt][2 * h + 1][0]);
@@ -544,7 +446,7 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
       for (int64_t t = 0; t < n_tiles; ++t, ++it) {
         const int stage = it % NSTAGE;
         mma::mbar_wait(&b_empty[stage], ((it / NSTAGE) & 1u) ^ 1u);
-        float4* bst = reinterpret_cast<float4*>(sB + (size_t)stage * Cfg::B_STAGE_BYTES);
+        uint4* bst = reinterpret_cast<uint4*>(sB + (size_t)stage * Cfg::B_STAGE_BYTES);
         double* wst = sW + stage * NT;
 #pragma unroll
         for (int c = ptid; c < NT; c += NPROD) {
@@ -571,59 +473,36 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
             f[(v - 1) * 4 + 2] = __uint_as_float(q[v].z);
             f[(v - 1) * 4 + 3] = __uint_as_float(q[v].w);
           }
-          if constexpr (Cfg::F16) {
-            // pieces as floats first (hi = the value cut to 11 significant bits by a mask, lo = the exact fp32
-            // remainder), then packed pair conversions only: scalar float <-> half conversions run on the
-            // 16-lane pipe of the epilogue's ex2 - the pipe that bounds this kernel
-            float fv[KA];
+          // pieces as floats first (hi = the value cut to 11 significant bits by a mask, lo = the exact fp32
+          // remainder), then packed pair conversions only: scalar float <-> half conversions run on the
+          // 16-lane pipe of the epilogue's ex2 - the pipe that bounds this kernel
+          float fv[KA];
 #pragma unroll
-            for (int k = 0; k < KA; ++k) fv[k] = 0.f;
-            if (ok) {
+          for (int k = 0; k < KA; ++k) fv[k] = 0.f;
+          if (ok) {
 #pragma unroll
-              for (int i = 0; i < DP; ++i) {
-                const float x = mma::clamp_h(f[2 + i]);
-                const float xh = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-                fv[3 * i] = xh;
-                fv[3 * i + 1] = __fsub_rn(x, xh);
-                fv[3 * i + 2] = xh;
-              }
-              const float av = mma::clamp_h(f[1]);
-              const float a1 = __uint_as_float(__float_as_uint(av) & 0xFFFFE000u);
-              const float r1 = __fsub_rn(av, a1);
-              const float a2 = __uint_as_float(__float_as_uint(r1) & 0xFFFFE000u);
-              fv[3 * DP] = a1;
-              fv[3 * DP + 1] = a2;
-              fv[3 * DP + 2] = __fsub_rn(r1, a2);
-              fv[3 * DP + 3] = fv[3 * DP + 4] = fv[3 * DP + 5] = 1.f;
+            for (int i = 0; i < DP; ++i) {
+              const float x = mma::clamp_h(f[2 + i]);
+              const float xh = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
+              fv[3 * i] = xh;
+              fv[3 * i + 1] = __fsub_rn(x, xh);
+              fv[3 * i + 2] = xh;
             }
-            uint4* bst16 = reinterpret_cast<uint4*>(bst);
+            const float av = mma::clamp_h(f[1]);
+            const float a1 = __uint_as_float(__float_as_uint(av) & 0xFFFFE000u);
+            const float r1 = __fsub_rn(av, a1);
+            const float a2 = __uint_as_float(__float_as_uint(r1) & 0xFFFFE000u);
+            fv[3 * DP] = a1;
+            fv[3 * DP + 1] = a2;
+            fv[3 * DP + 2] = __fsub_rn(r1, a2);
+            fv[3 * DP + 3] = fv[3 * DP + 4] = fv[3 * DP + 5] = 1.f;
+          }
 #pragma unroll
-            for (int kc = 0; kc < KA / 8; ++kc) {
-              __half2 h2[4];
+          for (int kc = 0; kc < KA / 8; ++kc) {
+            __half2 h2[4];
 #pragma unroll
-              for (int u = 0; u < 4; ++u) h2[u] = __floats2half2_rn(fv[8 * kc + 2 * u], fv[8 * kc + 2 * u + 1]);
-              bst16[kc * NT + c] = *reinterpret_cast<const uint4*>(h2);
-            }
-          } else {
-            float vals[KA];
-#pragma unroll
-            for (int k = 0; k < KA; ++k) vals[k] = 0.f;
-            if (ok) {
-#pragma unroll
-              for (int i = 0; i < DP; ++i) {
-                const float x = f[2 + i];
-                const float xh = mma::tf32_rna(x);
-                const float xl = mma::tf32_rna(__fsub_rn(x, xh));
-                vals[3 * i] = xh;
-                vals[3 * i + 1] = xl;
-                vals[3 * i + 2] = xh;
-              }
-              mma::split3(f[1], vals[3 * DP], vals[3 * DP + 1], vals[3 * DP + 2]);
-              vals[3 * DP + 3] = vals[3 * DP + 4] = vals[3 * DP + 5] = 1.f;
-            }
-#pragma unroll
-            for (int kc = 0; kc < KA / 4; ++kc)
-              bst[kc * NT + c] = make_float4(vals[4 * kc], vals[4 * kc + 1], vals[4 * kc + 2], vals[4 * kc + 3]);
+            for (int u = 0; u < 4; ++u) h2[u] = __floats2half2_rn(fv[8 * kc + 2 * u], fv[8 * kc + 2 * u + 1]);
+            bst[kc * NT + c] = *reinterpret_cast<const uint4*>(h2);
           }
           wst[c] = w;
         }
@@ -633,9 +512,8 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
     }
   } else {
     // ======================================================================== MMA issuer
-    // instruction descriptor: D fp32; A / B tf32 (format 2) or fp16 (format 0), K-major; N, M
-    constexpr uint32_t FMT = Cfg::F16 ? 0u : 2u;
-    constexpr uint32_t IDESC = (1u << 4) | (FMT << 7) | (FMT << 10) | ((uint32_t)(NT >> 3) << 17) | ((128u >> 4) << 24);
+    // instruction descriptor: D fp32 (bit 4), A / B fp16 (formats 0), K-major both; N, M
+    constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(NT >> 3) << 17) | ((128u >> 4) << 24);
     constexpr int NABUF = Cfg::NABUF;
     uint32_t it = 0, tc = 0, ac = 0;  // ac counts the work items with tiles (= landmark tile loads)
     auto next_item = [&](int item) {  // first item >= `item` of this CTA that has tiles; n_items if none
@@ -681,11 +559,10 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
             const uint32_t a_base = mma::smem_u32(sAcur + mt * Cfg::A_TILE_BYTES);
             const uint32_t b_base = mma::smem_u32(sB + (size_t)stage * Cfg::B_STAGE_BYTES);
 #pragma unroll
-            for (int ks = 0; ks < KA / Cfg::KSTEP; ++ks) {   // one MMA = two 16-byte K chunks of either type
+            for (int ks = 0; ks < KA / 16; ++ks) {   // one MMA (K = 16) = two 16-byte K chunks
               const uint64_t ad = mma::smem_desc(a_base + ks * 2 * (128 * 16), 128 * 16, 128);
               const uint64_t bd = mma::smem_desc(b_base + ks * 2 * (NT * 16), NT * 16, 128);
-              if (Cfg::F16) mma::umma_f16(tmem_base + buf * NT, ad, bd, IDESC, ks > 0 ? 1u : 0u);
-              else mma::umma_tf32(tmem_base + buf * NT, ad, bd, IDESC, ks > 0 ? 1u : 0u);
+              mma::umma_f16(tmem_base + buf * NT, ad, bd, IDESC, ks > 0 ? 1u : 0u);
             }
             mma::umma_commit(&t_full[buf]);
           }

@@ -381,10 +381,9 @@ int tgemm(basq_ctx* ctx, const BlkOperand& A, const BlkOperand& B, double alpha,
   // rounds split).  Two addends per element: the sum does not depend on their order.  (Cutting the (tile, K block)
   // sequence into equal contiguous ranges - "stream-K" - balances perfectly but lets neighbouring CTAs drift
   // apart in K: measured L2 hit rate 20 % instead of 76 %, 3.8 GB instead of 0.54 GB from HBM, and slower.)
-  static const bool allow_split = [] { const char* e = getenv("BASQ_TGEMM_KSPLIT"); return !(e && e[0] == '0'); }();
   const int nkb = A.KC / TG_KCH;
   d.ksplit = 1;
-  if (allow_split && nkb >= 8 && 2 * ceil_div(n_items, grid) > ceil_div(2 * n_items, grid)) d.ksplit = 2;
+  if (nkb >= 8 && 2 * ceil_div(n_items, grid) > ceil_div(2 * n_items, grid)) d.ksplit = 2;
   if (d.ksplit > 1 && !accumulate) {   // both parts are added onto zeros
     const size_t width = sizeof(double) * (size_t)(transposed ? d.I : d.J);
     BASQ_CUDA(cudaMemset2DAsync(out, sizeof(double) * (size_t)ldo, 0, width, (size_t)(transposed ? d.J : d.I), ctx->stream));

@@ -78,13 +78,6 @@ def test_gp_predict_large_matern(family, nu):
     _check_predict(model, twin, _cands(4096, 2))
 
 
-def test_gp_predict_large_two_kernel_variant(monkeypatch):
-    """BASQ_GPVAR_FUSED=0: k(Xobs, x) staged as an operand, then the A/B variance kernel."""
-    monkeypatch.setenv("BASQ_GPVAR_FUSED", "0")
-    model, twin = _build(_obs(9000, 9000))
-    _check_predict(model, twin, _cands(4096, 3))
-
-
 def test_route_continuity_4096_4097():
     """The 4097th observation lies far from every candidate, so the posterior variance there is the same
     for both GPs: the two L^-1 preparations (two inversions / reversed Cholesky) agree across the switch."""
