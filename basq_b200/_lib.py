@@ -94,6 +94,7 @@ def _load():
         "basq_sir_resample": (I, [P, P, L, L, C.c_uint64, P, C.POINTER(L)]),
         "basq_dgemm": (I, [P, I, I, I, I, I, D, P, I, P, I, D, P, I]),
         "basq_tgemm": (I, [P, I, I, I, P, I, P, I, P, I]),
+        "basq_igemm": (I, [P, I, I, I, P, I, I, I, P, I, P, I, I]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

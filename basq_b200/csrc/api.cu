@@ -9,6 +9,7 @@
 #include <new>
 
 #include "common.cuh"
+#include "igemm.cuh"
 #include "tgemm.cuh"
 
 namespace basq {
@@ -153,6 +154,12 @@ struct Piece {   // a typed view of a slice of the context's host-call buffer (b
   template <typename T> T* as() const { return static_cast<T*>(p); }
 };
 
+// Sessions with at least this many basis rows q and landmark rows Mtot project their level columns on the int8
+// tensor cores (scripts/time_projection.py, B200 at 1000 W: GEMM kernel 2.7-3.3x faster than the fp64 GEMM at
+// q = 999, Mtot = 10000-11002); below, slicing the level columns eats the gain (q = 499, Mtot = 5000: 0.15 ms
+// kernel + 0.05 ms slicing against 0.24 ms) and the fp64 GEMM stays.
+constexpr int INT8_PROJ_MIN_Q = 512, INT8_PROJ_MIN_MTOT = 8192;
+
 struct basq_session {
   basq_ctx* ctx = nullptr;
   basq_kernel_desc desc;
@@ -162,6 +169,10 @@ struct basq_session {
   Landmarks lm;     // Z (+ Xobs appended for the linear posterior-covariance modes)
   Landmarks lmobs;  // Xobs alone
   DevBuf Uprime;    // [q, Mtot]
+  // Large sessions project on the int8 tensor cores (igemm.cu): U' as digits once, the level columns per level.
+  // Decided once per session: hi = parent - lo mixes the projections of two levels, which must share one arithmetic.
+  bool int8_proj = false;
+  DigOperand Udig, Gdig;
   DevBuf sz;        // [M] per-landmark factor
   DevBuf Az;        // [M, n_obs] = K(Z, Xobs) W          (non-linear modes)
   RecPool pool;
@@ -430,6 +441,8 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
     BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
     s->Az.release();
   }
+  s->int8_proj = q >= INT8_PROJ_MIN_Q && s->Mtot >= INT8_PROJ_MIN_MTOT;
+  if (s->int8_proj) BASQ_TRY(dig_from_f64(ctx, s->Uprime.as<double>(), s->Mtot, false, q, s->Mtot, 0, 128, &s->Udig));
 
   // candidate records
   const double uniform_w = 1.0 / (double)(N_glob > 0 ? N_glob : 1);
@@ -601,7 +614,10 @@ int session_level_project(basq_session* s, int lvl, int K, const int* node_host,
                                                                             raw + (int64_t)n * S, S);
     ctx->launches++;
   }
-  if (nrows > 0) {
+  if (nrows > 0 && s->int8_proj) {
+    BASQ_TRY(dig_from_f64(ctx, Gf_rows, ld_gf, true, K, nrows, row0, 64, &s->Gdig));
+    BASQ_TRY(igemm(ctx, s->Udig, s->Gdig, 1.0, raw + S, S, false));
+  } else if (nrows > 0) {
     BASQ_TRY(dgemm(ctx, false, false, s->q, K, nrows, 1.0, s->Uprime.as<double>() + row0, s->Mtot, Gf_rows, ld_gf, 0.0,
                    raw + S, S));
   } else {
@@ -1066,6 +1082,21 @@ int basq_tgemm(basq_ctx* ctx, int m, int n, int k, const double* A, int lda, con
   BASQ_TRY(blk_from_f64(ctx, A, lda, false, &a));
   BASQ_TRY(blk_from_f64(ctx, B, ldb, false, &b));
   BASQ_TRY(tgemm(ctx, a, b, 1.0, C, ldc, false));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  return BASQ_OK;
+}
+
+int basq_igemm(basq_ctx* ctx, int m, int n, int k, const double* A, int lda, int row0, int nrows, const double* B,
+               int ldb, double* C, int ldc, int accumulate) {
+  BASQ_CHECK(ctx && A && B && C, BASQ_ERR_INVALID, "basq_igemm: NULL argument");
+  BASQ_CHECK(m >= 1 && n >= 1 && k >= 1 && lda >= k && row0 >= 0 && nrows >= 1 && row0 + nrows <= k && ldb >= n &&
+                 ldc >= n,
+             BASQ_ERR_INVALID, "basq_igemm: bad shape");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  DigOperand a, b;
+  BASQ_TRY(dig_from_f64(ctx, A, lda, false, m, k, 0, 128, &a));
+  BASQ_TRY(dig_from_f64(ctx, B, ldb, true, n, nrows, row0, 64, &b));
+  BASQ_TRY(igemm(ctx, a, b, 1.0, C, ldc, accumulate != 0));
   BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
   return BASQ_OK;
 }

@@ -149,6 +149,18 @@ __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem]^T, signed int8 inputs, exact s32 accumulate
+__device__ __forceinline__ void umma_i8(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                        uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n"
+      "}" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // K-major operand without swizzle, stored as [K / 8][rows][8 halves]: 8-row core matrices are
 // contiguous (SBO = 128 B), the next 16-byte K chunk lies one plane further (LBO = rows * 16 B).
 __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {

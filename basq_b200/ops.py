@@ -164,6 +164,24 @@ def tgemm(A, B):
     return Cm
 
 
+def igemm(A, B, row0=0, out=None):
+    """A[:, row0:row0 + len(B)] @ B with fp64 accuracy on the int8 tensor cores (Ozaki slicing, the projection's
+    GEMM); fp64 tensors in and out.  With ``out`` the product is added to it."""
+    ctx = _lib.context_for(A.device)
+    A = A.to(torch.float64).contiguous(); B = B.to(torch.float64).contiguous()
+    m, k = A.shape
+    nrows, n = B.shape
+    if row0 < 0 or row0 + nrows > k:
+        raise ValueError(f"rows [{row0}, {row0 + nrows}) of B lie outside A's {k} columns")
+    accumulate = out is not None
+    if out is None:
+        out = torch.empty(m, n, dtype=torch.float64, device=A.device)
+    assert out.shape == (m, n) and out.dtype == torch.float64 and out.is_contiguous()
+    _lib.check(_lib.lib.basq_igemm(ctx.handle, m, n, k, A.data_ptr(), k, row0, nrows, B.data_ptr(), n,
+                                   out.data_ptr(), n, int(accumulate)))
+    return out
+
+
 def recombine(kernel, pts_rec, pts_nys, U, mu=None, device=None, obj=None):
     """Tchernychova-Lyons recombination with a given basis U [q, M]: (idx int64, w fp64) on device.
     obj [N]: the reference's ``-calc_obj(samp)`` for the objective-aware variant (SOBER/_rchq.py:67-69)."""

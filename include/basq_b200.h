@@ -340,6 +340,14 @@ int basq_dgemm(basq_ctx* ctx, int transA, int transB, int m, int n, int k, doubl
 int basq_tgemm(basq_ctx* ctx, int m, int n, int k, const double* A, int lda, const double* B, int ldb,
                double* C, int ldc);
 
+/* C[m,n] (+)= A[:, row0 .. row0 + nrows) B[nrows, n] with fp64 accuracy on the int8 tensor cores (Ozaki
+   slicing: every row of A and column of B scaled by a power of two and cut into 8 signed int8 digits, 36 digit
+   products accumulated exactly in s32; error <= 2^-50.8 nrows max|A_i.| max|B_.j| + 7 ulp(C)).  A is [m, k],
+   fp64 row-major in and out; accumulate != 0 adds to C.  This is the GEMM behind the projection of the level
+   columns of large sessions, U'[:, row0 ..) Gf_rows. */
+int basq_igemm(basq_ctx* ctx, int m, int n, int k, const double* A, int lda, int row0, int nrows, const double* B,
+               int ldb, double* C, int ldc, int accumulate);
+
 #ifdef __cplusplus
 }
 #endif
