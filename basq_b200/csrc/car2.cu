@@ -8,10 +8,11 @@
 //   * The tableau never touches shared or global memory between pivots: CTA k keeps a block of B
 //     consecutive rows (stage 1) / non-basic columns (stage 2) in REGISTERS, thread t holding the
 //     entries of columns (rows) t, t+NT, t+2NT, ... of each of them.
-//   * The owner CTA performs its B pivots back to back on its own registers: pivot search = block
-//     arg-reduce with one __syncthreads (the signed pivot travels with the reduction), multipliers
-//     of the B-1 sibling rows broadcast through a double-buffered shared array (second
-//     __syncthreads), sibling updates are register FMAs.
+//   * The owner CTA performs its B pivots back to back on its own registers with ONE __syncthreads
+//     per pivot: the block arg-reduce carries, next to the winner's key, the B multipliers of its
+//     column (stage 1) / row (stage 2) and the correctly rounded reciprocal of its pivot, which
+//     every lane computes for its own candidate ahead of the reduction; sibling updates are
+//     register FMAs.
 //   * Publication is "the data is the flag": the pivot row (column) and a per-thread copy of the
 //     pivot index are streamed to L2 buffers that the host pre-filled with a NaN / -1 sentinel; a
 //     consumer thread simply polls the few words IT needs until they are no longer the sentinel.
@@ -65,23 +66,24 @@ __device__ __forceinline__ void stamp(unsigned long long* stamps, int i) {
 // (is_sentinel / poll_f64 / poll_i32: gridsync.cuh)
 
 // ---------------------------------------------------------------------------------------------
-// Block-wide arg-max / arg-min with ONE barrier and two shuffles per butterfly round.
+// Block-wide arg-max / arg-min with ONE barrier.
 // The key is a non-negative double, so its bit pattern orders like an unsigned integer; the low 12
 // mantissa bits are replaced by the candidate's index (complemented for the maximum), which makes
 // every candidate unique and breaks ties (keys equal to 2^-40 relative) towards the smaller index.
-// The winner's exact payload (signed pivot / exact ratio) travels through the scratch row: the lane
-// that recognises its own packed key as the warp's best writes it, and after the barrier every warp
-// reduces the NT/32 warp results itself.  (Two calls never touch the same scratch row while a thread
-// still reads it: a thread passes the barrier of call N+1 only after all threads finished reading
-// the row of call N.)
+// The winner's exact payload (W words: signed pivot / exact ratio, reciprocal, multipliers) travels
+// through the scratch slots: the lane that recognises its own packed key as the warp's best writes
+// its key and calls fill(payload row), and after the barrier every warp reduces the NT/32 warp keys
+// itself and reads the global winner's payload row.
+// The slots are double-buffered by the CTA-uniform parity spar, and every read of the slots of call
+// N (keys, and the payload words the caller reads before its next call) happens before the reading
+// thread arrives at the barrier of call N+1.  A thread writes the same parity again only in call
+// N+2, after passing that barrier, i.e. after every thread has finished reading call N.
 // ---------------------------------------------------------------------------------------------
-struct Slot {
-  unsigned long long key;
-  double val;
-};
-struct Best {
-  int idx;     // -1: no candidate
-  double val;  // exact payload of the winner
+template <int NT, int W>
+struct Scratch {
+  static_assert(W % 2 == 0, "payload rows stay 16-byte aligned");
+  unsigned long long key[2][NT / 32];
+  alignas(16) double pay[2][NT / 32][W];
 };
 
 __device__ __forceinline__ unsigned long long pack_max(double key, int idx) {
@@ -106,38 +108,41 @@ __device__ __forceinline__ unsigned long long warp_best_u64(unsigned long long x
   }
 }
 
-// MAX: `none` = 0 ; MIN: `none` = ~0
-template <bool MAX, int NT>
-__device__ __forceinline__ Best block_best(unsigned long long mine, double payload, Slot (*scratch)[NT / 32], int& spar) {
+template <bool MAX>
+__device__ __forceinline__ int key_index(unsigned long long key) {
+  return MAX ? (0xFFF - (int)(key & 0xFFFull)) : (int)(key & 0xFFFull);
+}
+
+// Returns the winner's index (-1: no candidate; MAX: `none` = 0, MIN: `none` = ~0) and points `pay`
+// at its payload row (valid only for a winner).
+template <bool MAX, int NT, int W, class Fill>
+__device__ __forceinline__ int block_best(unsigned long long mine, Scratch<NT, W>& s, int& spar, const double*& pay,
+                                          Fill fill) {
   constexpr unsigned long long NONE = MAX ? 0ull : ~0ull;
   const unsigned long long x = warp_best_u64<MAX>(mine);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if (x == NONE) {
-    if (lane == 0) scratch[spar][warp] = Slot{NONE, 0.0};
+    if (lane == 0) s.key[spar][warp] = NONE;
   } else if (mine == x) {
-    scratch[spar][warp] = Slot{x, payload};
+    s.key[spar][warp] = x;
+    fill(s.pay[spar][warp]);
   }
   __syncthreads();
-  const Slot* row = scratch[spar];
+  const int p = spar;
   spar ^= 1;
-  const unsigned long long w = row[lane & (NT / 32 - 1)].key;
+  const unsigned long long w = s.key[p][lane & (NT / 32 - 1)];
   const unsigned long long y = warp_best_u64<MAX>(w);
-  Best r;
-  if (y == NONE) {
-    r.idx = -1;
-    r.val = 0.0;
-    return r;
-  }
   const unsigned hit = __ballot_sync(FULLMASK, w == y);
-  r.val = row[(__ffs(hit) - 1) & (NT / 32 - 1)].val;
-  r.idx = MAX ? (0xFFF - (int)(y & 0xFFFull)) : (int)(y & 0xFFFull);
-  return r;
+  pay = s.pay[p][(__ffs(hit) - 1) & (NT / 32 - 1)];
+  return y == NONE ? -1 : key_index<MAX>(y);
 }
 
 template <int B, int NT, int CPT, int RPT>
 __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
-  __shared__ Slot scratch[2][NT / 32];
-  __shared__ double fbuf[2][8];
+  // payload row: stage 1 {B multipliers, reciprocal of the pivot}, stage 2 {B multipliers, ratio}
+  constexpr int W = (B + 2) & ~1;
+  __shared__ Scratch<NT, W> scratch;
+  __shared__ double fbuf[2][B];
   __shared__ int abort_sh;
   extern __shared__ int nbcol[];  // [S] non-basic column list (stage 2)
 
@@ -155,7 +160,9 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
   const int r0 = b * B;
   const int rows_mine = max(0, min(B, n - r0));
   double reg[B][CPT];
-  double rscale[B];
+  // largest |entry| of each own row (CTA-uniform; in shared memory, which keeps B = 8 free of spills at
+  // 128 registers).  Thread 0 writes it; the barrier of the next block_best publishes it.
+  __shared__ double rscale[B];
   unsigned elig = 0;
 #pragma unroll
   for (int j = 0; j < CPT; ++j)
@@ -179,46 +186,42 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
         if ((elig >> j & 1u) && pk > mk) { mk = pk; mv = reg[i][j]; }
       }
     }
-    rscale[i] = fabs(block_best<true, NT>(mk, mv, scratch, spar).val);  // (CTA-uniform loop: every thread calls it B times)
+    const double* w;
+    const int idx = block_best<true>(mk, scratch, spar, w, [&](double* p) { p[0] = mv; });
+    if (tid == 0) rscale[i] = idx < 0 ? 0.0 : fabs(w[0]);  // (CTA-uniform loop: every thread calls it B times)
   }
 
-  // rank-1 update of the own rows with pivot-row entries `pr` (pivot column cs); skip_row: the
-  // pivot row itself when it lives in this CTA
-  static_assert(CPT <= 4 && RPT <= 4, "the column / row selectors below enumerate up to four slots");
-  auto eliminate = [&](const double (&pr)[CPT], int cs, int skip_row) {
+  // Rows and columns past the own block (rows_mine < B, cols_mine < B: a ragged last block or an
+  // idle CTA) start at zero, receive the same updates as the others and are never read: no
+  // predicates for them in the updates below.
+  // Consumer replay: rank-1 update of the own rows with pivot-row entries `pr` (pivot column cs);
+  // the thread holding column cs broadcasts its B multipliers through fbuf.
+  auto eliminate = [&](const double (&pr)[CPT], int cs) {
+    const bool holder = (cs & (NT - 1)) == tid;
     const int js = cs / NT;
-    if ((cs % NT) == tid) {
-      // this thread holds column cs: publish the multipliers of the B rows.  js is uniform, so a
-      // switch with static register indices replaces B*CPT select chains.
+    if (holder) {
       elig &= ~(1u << js);
-#define BASQ_CAR_COL(J)                                                   \
-  if (J < CPT) {                                                          \
-    _Pragma("unroll") for (int i2 = 0; i2 < B; ++i2) fbuf[par][i2] = reg[i2][J < CPT ? J : 0]; \
-  }
-      switch (js) {
-        case 0: BASQ_CAR_COL(0) break;
-        case 1: BASQ_CAR_COL(1) break;
-        case 2: BASQ_CAR_COL(2) break;
-        default: BASQ_CAR_COL(3) break;
-      }
-#undef BASQ_CAR_COL
+#pragma unroll
+      for (int j = 0; j < CPT; ++j)
+        if (j == js) {
+#pragma unroll
+          for (int i2 = 0; i2 < B; ++i2) fbuf[par][i2] = reg[i2][j];
+        }
     }
     __syncthreads();
 #pragma unroll
     for (int i2 = 0; i2 < B; ++i2) {
-      if (i2 != skip_row && i2 < rows_mine) {
-        const double f = fbuf[par][i2];
+      const double f = fbuf[par][i2];
 #pragma unroll
-        for (int j = 0; j < CPT; ++j) reg[i2][j] = fma(-f, pr[j], reg[i2][j]);
-      }
+      for (int j = 0; j < CPT; ++j) reg[i2][j] = fma(-f, pr[j], reg[i2][j]);
     }
-    if ((cs % NT) == tid) {  // the eliminated column is exactly zero in every other row
-      switch (js) {
-        case 0: _Pragma("unroll") for (int i2 = 0; i2 < B; ++i2) if (i2 != skip_row) reg[i2][0] = 0.0; break;
-        case 1: _Pragma("unroll") for (int i2 = 0; i2 < B; ++i2) if (i2 != skip_row && CPT > 1) reg[i2][CPT > 1 ? 1 : 0] = 0.0; break;
-        case 2: _Pragma("unroll") for (int i2 = 0; i2 < B; ++i2) if (i2 != skip_row && CPT > 2) reg[i2][CPT > 2 ? 2 : 0] = 0.0; break;
-        default: _Pragma("unroll") for (int i2 = 0; i2 < B; ++i2) if (i2 != skip_row && CPT > 3) reg[i2][CPT > 3 ? 3 : 0] = 0.0; break;
-      }
+    if (holder) {  // the eliminated column is exactly zero in every other row
+#pragma unroll
+      for (int j = 0; j < CPT; ++j)
+        if (j == js) {
+#pragma unroll
+          for (int i2 = 0; i2 < B; ++i2) reg[i2][j] = 0.0;
+        }
     }
     par ^= 1;
   };
@@ -239,26 +242,57 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
             const unsigned long long pk = pack_max(fabs(reg[i][j]), tid + j * NT);
             if ((elig >> j & 1u) && pk > mk) { mk = pk; mv = reg[i][j]; }
           }
-          const Best m = block_best<true, NT>(mk, mv, scratch, spar);
-          const bool skip = (m.idx < 0) || !(fabs(m.val) > a.tol * rscale[i]) || !(rscale[i] > 0.0);
+          // every lane inverts its own candidate while the reduction runs (1 avoids the slow path
+          // for lanes without one; a zero pivot is skipped below and its reciprocal never used)
+          const double rinv = __drcp_rn(mv != 0.0 ? mv : 1.0);
+          const double* w;
+          // payload: the PRE-scaling entries of the candidate column in all B rows (the sibling
+          // multipliers; entry i is the pivot itself) and the reciprocal of the pivot
+          const int cs = block_best<true>(mk, scratch, spar, w, [&](double* p) {
+            const int jm = key_index<true>(mk) / NT;
+#pragma unroll
+            for (int j = 0; j < CPT; ++j)
+              if (j == jm) {
+#pragma unroll
+                for (int i2 = 0; i2 < B; ++i2) p[i2] = reg[i2][j];
+              }
+            p[B] = rinv;
+          });
+          const bool skip = (cs < 0) || !(fabs(w[i]) > a.tol * rscale[i]) || !(rscale[i] > 0.0);
           const int row = kr0 + i;
           if (skip) {
             __stcg(&a.prep[(int64_t)row * NT + tid], 1);
             if (tid == 0) a.pinfo[row] = -1;
           } else {
-            const int cs = m.idx;
-            const double inv = 1.0 / m.val;
-            // the multipliers of the sibling rows are the PRE-scaling entries of column cs: grab them
-            // (eliminate reads reg[i2][js] for i2 != i) after the pivot row has been scaled
+            const double inv = w[B];
+#pragma unroll
+            for (int j = 0; j < CPT; ++j) reg[i][j] = (tid + j * NT == cs) ? 1.0 : reg[i][j] * inv;
+            // the next pivot's row first, then the other siblings, then the publication stores
+#pragma unroll
+            for (int s = 1; s < B; ++s) {
+              const int i2 = (i + s) % B;
+              const double f = w[i2];
+#pragma unroll
+              for (int j = 0; j < CPT; ++j) reg[i2][j] = fma(-f, reg[i][j], reg[i2][j]);
+            }
+            if ((cs & (NT - 1)) == tid) {  // the eliminated column is exactly zero in every other row
+              const int js = cs / NT;
+              elig &= ~(1u << js);
+#pragma unroll
+              for (int j = 0; j < CPT; ++j)
+                if (j == js) {
+#pragma unroll
+                  for (int i2 = 0; i2 < B; ++i2)
+                    if (i2 != i) reg[i2][j] = 0.0;
+                }
+            }
 #pragma unroll
             for (int j = 0; j < CPT; ++j) {
               const int c = tid + j * NT;
-              reg[i][j] = (c == cs) ? 1.0 : reg[i][j] * inv;
               if (c < S) __stcg(&a.prow[(int64_t)row * S + c], reg[i][j]);
             }
             __stcg(&a.prep[(int64_t)row * NT + tid], cs + 2);
             if (tid == 0) a.pinfo[row] = cs;
-            eliminate(reg[i], cs, i);
           }
         }
       }
@@ -318,7 +352,7 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
             const int c = tid + j * NT;
             if (i + PF < B) win[i % PF][j] = (i + PF < krows && c < S) ? __ldcg(&a.prow[(int64_t)(kr0 + i + PF) * S + c]) : 0.0;
           }
-          if (cd >= 2) eliminate(cur, cd - 2, -1);
+          if (cd >= 2) eliminate(cur, cd - 2);
         }
       }
     }
@@ -395,39 +429,34 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
     }
   }
 
-  // pivot the own columns [first, cols_mine) on basic row istar of the published column pv
-  auto col_update = [&](const double (&pv)[RPT], int istar, int first) {
+  // consumer replay: pivot the own columns on basic row istar of the published column pv; the
+  // thread holding row istar broadcasts the B multipliers through fbuf
+  auto col_update = [&](const double (&pv)[RPT], int istar) {
+    const bool holder = (istar & (NT - 1)) == tid;
     const int js = istar / NT;
-    if ((istar % NT) == tid) {
-      double p = 0.0;
+    if (holder) {
 #pragma unroll
       for (int jj = 0; jj < RPT; ++jj)
-        if (jj == js) p = pv[jj];
-      const double invp = 1.0 / p;
+        if (jj == js) {
+          const double invp = __drcp_rn(pv[jj]);
 #pragma unroll
-      for (int l2 = 0; l2 < B; ++l2) {
-        double t = 0.0;
-#pragma unroll
-        for (int jj = 0; jj < RPT; ++jj)
-          if (jj == js) t = tc[l2][jj];
-        fbuf[par][l2] = t * invp;
-      }
+          for (int l2 = 0; l2 < B; ++l2) fbuf[par][l2] = tc[l2][jj] * invp;
+        }
     }
     __syncthreads();
 #pragma unroll
     for (int l2 = 0; l2 < B; ++l2) {
-      if (l2 >= first && l2 < cols_mine) {
-        const double t = fbuf[par][l2];
+      const double t = fbuf[par][l2];
 #pragma unroll
-        for (int jj = 0; jj < RPT; ++jj) tc[l2][jj] = fma(-pv[jj], t, tc[l2][jj]);
-      }
+      for (int jj = 0; jj < RPT; ++jj) tc[l2][jj] = fma(-pv[jj], t, tc[l2][jj]);
     }
-    if ((istar % NT) == tid) {  // the leaving row holds the multiplier itself
+    if (holder) {  // the leaving row holds the multiplier itself
 #pragma unroll
-      for (int l2 = 0; l2 < B; ++l2)
+      for (int jj = 0; jj < RPT; ++jj)
+        if (jj == js) {
 #pragma unroll
-        for (int jj = 0; jj < RPT; ++jj)
-          if (jj == js && l2 >= first && l2 < cols_mine) tc[l2][jj] = fbuf[par][l2];
+          for (int l2 = 0; l2 < B; ++l2) tc[l2][jj] = fbuf[par][l2];
+        }
     }
     par ^= 1;
   };
@@ -477,7 +506,7 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
               }
             }
           }
-          if (code[l] >= 2) col_update(pvs[l], code[l] - 2, 0);
+          if (code[l] >= 2) col_update(pvs[l], code[l] - 2);
         }
       }
     } else {
@@ -496,28 +525,40 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
       for (int l = 0; l < B; ++l) {
         if (l < kcols) {
           unsigned long long bk = ~0ull;
-          double bv = 0.0;
+          double bv = 0.0, bt = -1.0;  // (-1: no candidate; keeps the reciprocal off its slow path)
 #pragma unroll
           for (int jj = 0; jj < RPT; ++jj) {
             const double t = tc[l][jj];
             if (rowpt[jj] >= 0 && t < 0.0) {
               const double ratio = muB[jj] / (-t);
               const unsigned long long pk = pack_min(ratio, tid + jj * NT);
-              if (pk < bk) { bk = pk; bv = ratio; }
+              if (pk < bk) { bk = pk; bv = ratio; bt = t; }
             }
           }
-          const Best best = block_best<false, NT>(bk, bv, scratch, spar);
+          const double rinvp = __drcp_rn(bt);  // computed by every lane while the reduction runs
+          const double* w;
+          // payload: the multipliers of the later own columns (entries of the candidate row scaled
+          // by the reciprocal of the pivot) and the ratio
+          const int best = block_best<false>(bk, scratch, spar, w, [&](double* p) {
+            const int jm = key_index<false>(bk) / NT;
+#pragma unroll
+            for (int jj = 0; jj < RPT; ++jj)
+              if (jj == jm) {
+#pragma unroll
+                for (int l2 = l + 1; l2 < B; ++l2) p[l2] = tc[l2][jj] * rinvp;
+              }
+            p[B] = bv;
+          });
           // the non-basic set itself has +1 in its null vector and weight 1: ratio 1
-          const bool self = (best.idx < 0) || !(best.val < 1.0);
-          const double alpha = self ? 1.0 : best.val;
-          const int istar = self ? -1 : best.idx;
+          const bool self = (best < 0) || !(w[B] < 1.0);
+          const double alpha = self ? 1.0 : w[B];
+          const int istar = self ? -1 : best;
           const int jn = kc0 + l;
           double pv[RPT];
 #pragma unroll
           for (int jj = 0; jj < RPT; ++jj) {
             const int i = tid + jj * NT;
             pv[jj] = tc[l][jj];
-            if (i < n && istar >= 0) __stcg(&a.pcol[(int64_t)jn * n + i], pv[jj]);
             if (rowpt[jj] >= 0) {
               const double v = fma(alpha, pv[jj], muB[jj]);
               muB[jj] = v > 0.0 ? v : 0.0;
@@ -527,8 +568,27 @@ __global__ void __launch_bounds__(NT, 1) car2_kernel(const Car2Dev a) {
               rowpt[jj] = nbcol[jn];
             }
           }
+          if (istar >= 0) {  // pivot the later own columns on row istar
+#pragma unroll
+            for (int l2 = l + 1; l2 < B; ++l2) {
+              const double t = w[l2];
+#pragma unroll
+              for (int jj = 0; jj < RPT; ++jj) tc[l2][jj] = fma(-pv[jj], t, tc[l2][jj]);
+            }
+            if ((istar & (NT - 1)) == tid) {  // the leaving row holds the multiplier itself
+              const int js = istar / NT;
+#pragma unroll
+              for (int jj = 0; jj < RPT; ++jj)
+                if (jj == js) {
+#pragma unroll
+                  for (int l2 = l + 1; l2 < B; ++l2) tc[l2][jj] = w[l2];
+                }
+            }
+#pragma unroll
+            for (int jj = 0; jj < RPT; ++jj)
+              if (tid + jj * NT < n) __stcg(&a.pcol[(int64_t)jn * n + tid + jj * NT], pv[jj]);
+          }
           __stcg(&a.srep[(int64_t)jn * NT + tid], istar >= 0 ? istar + 2 : 1);
-          if (istar >= 0) col_update(pv, istar, l + 1);
         }
       }
       if (k == G2 - 1) {
@@ -559,10 +619,9 @@ int launch_car2(basq_ctx* ctx, const Car2Dev& d, int grid, size_t smem) {
   return BASQ_OK;
 }
 
-#ifndef BASQ_CAR2_NT
-#define BASQ_CAR2_NT 512
-#endif
-constexpr int C2_NT = BASQ_CAR2_NT, C2_CPT = 2048 / C2_NT, C2_RPT = 1024 / C2_NT;
+// 512 threads: at 256 (CPT = 8, RPT = 4) the owner pivots issue fewer warp instructions, yet stage 2
+// took 1.44 instead of 1.12 ms at n = 1000, S = 2000 (B200, 1000 W)
+constexpr int C2_NT = 512, C2_CPT = 2048 / C2_NT, C2_RPT = 1024 / C2_NT;
 
 }  // namespace
 
