@@ -1220,7 +1220,7 @@ int basq_nystrom_basis(basq_ctx* ctx, const basq_kernel_desc* desc, const void* 
                        const double* Omega, int niter, double* U_out, double* S_out) {
   BASQ_CHECK(ctx && desc && Z && U_out, BASQ_ERR_INVALID, "basq_nystrom_basis: NULL argument");
   BASQ_CUDA(cudaSetDevice(ctx->device));
-  const int rc = nystrom_basis(ctx, desc, Z, M, q, Omega, niter, U_out, S_out);
+  const int rc = nystrom_basis(ctx, desc, Z, M, q, Omega, niter, U_out, S_out, nullptr);
   basq_ctx_trim(ctx, -1);
   return rc;
 }
@@ -1231,8 +1231,8 @@ int basq_nystrom_basis_sharded(basq_ctx* ctx, const basq_kernel_desc* desc, cons
   BASQ_CHECK(ctx && desc && Z && U_out && gram_buf && rows_buf && exchange, BASQ_ERR_INVALID,
              "basq_nystrom_basis_sharded: NULL argument");
   BASQ_CUDA(cudaSetDevice(ctx->device));
-  const int rc = nystrom_basis_sharded(ctx, desc, Z, M, q, Omega, niter, rank, world, gram_buf, rows_buf, exchange, user,
-                                       U_out);
+  const NysShard shard{rank, world, exchange, user, gram_buf, rows_buf};
+  const int rc = nystrom_basis(ctx, desc, Z, M, q, Omega, niter, U_out, nullptr, &shard);
   basq_ctx_trim(ctx, -1);
   return rc;
 }
@@ -1403,7 +1403,8 @@ static int recombine_host_impl(basq_ctx* ctx, const basq_kernel_desc* desc, cons
   }
   if (!U_host) {
     trace_point(ctx, "host: Z / Omega copies issued");
-    rc = nystrom_basis(ctx, desc, dZ.p, M, q, Omega_host ? dOm.as<double>() : nullptr, niter, dU.as<double>(), nullptr);
+    rc = nystrom_basis(ctx, desc, dZ.p, M, q, Omega_host ? dOm.as<double>() : nullptr, niter, dU.as<double>(), nullptr,
+                       nullptr);
   }
   if (rc == BASQ_OK && cudaStreamWaitEvent(ctx->stream, x_ready, 0) != cudaSuccess) rc = BASQ_ERR_CUDA;
   if (rc != BASQ_OK) {

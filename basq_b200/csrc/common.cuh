@@ -565,10 +565,16 @@ int nl_sweep_sums(basq_ctx* ctx, const KParams& kp, int nl, NlSweep* w, const Re
 // nystrom.cu
 // out[rows, cols] fp64 N(0, 1) draws of the Philox stream `seed` (candidates.cu)
 int standard_normals(basq_ctx* ctx, uint64_t seed, int64_t offset, int64_t rows, int cols, double* out);
-int nystrom_basis_sharded(basq_ctx* ctx, const basq_kernel_desc* desc, const void* Z, int64_t M, int q,
-                          const double* Omega, int niter, int rank, int world, double* gram_buf, double* rows_buf,
-                          basq_exchange_fn fn, void* user, double* U_out);
+// The ranks of a row-sharded Nystrom basis and the caller's exchange (basq_nystrom_basis_sharded)
+struct NysShard {
+  int rank = 0, world = 1;
+  basq_exchange_fn fn = nullptr;
+  void* user = nullptr;
+  double* gram_buf = nullptr;   // [q, q], the buffer the exchange function all-reduces
+  double* rows_buf = nullptr;   // [world * chunk, q], the buffer it all-gathers
+};
+// U_out [q, M]; shard == nullptr: this process holds all M rows.  S_out (Rayleigh quotients, may be NULL) only then.
 int nystrom_basis(basq_ctx* ctx, const basq_kernel_desc* desc, const void* Z, int64_t M, int q,
-                  const double* Omega, int niter, double* U_out, double* S_out);
+                  const double* Omega, int niter, double* U_out, double* S_out, const NysShard* shard);
 
 }  // namespace basq

@@ -14,6 +14,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <utility>
 
 #include "common.cuh"
 #include "gridsync.cuh"
@@ -369,6 +370,29 @@ __global__ void transpose_kernel(const double* __restrict__ in, int rows, int co
 
 struct OrthWs {
   DevBuf gram, linv, tmp, prow, prow2, flags, scal;
+  // the Cholesky + inverse workspace of q x q factors; tmp [tmp_rows, q] and scal (orthonormalise's product
+  // and scalars) only when tmp_rows > 0
+  int alloc(basq_ctx* ctx, int q, int64_t tmp_rows) {
+    BASQ_TRY(gram.alloc(ctx, sizeof(double) * (size_t)q * q));
+    BASQ_TRY(linv.alloc(ctx, sizeof(double) * (size_t)q * q));
+    BASQ_TRY(prow.alloc(ctx, sizeof(double) * 4 * q));
+    BASQ_TRY(prow2.alloc(ctx, sizeof(double) * 2 * (size_t)q * q));
+    BASQ_TRY(flags.alloc(ctx, 512));
+    BASQ_CUDA(cudaMemsetAsync(flags.p, 0, 512, ctx->stream));   // the watchdog status (byte 256) stays set once fired
+    if (tmp_rows > 0) {
+      BASQ_TRY(tmp.alloc(ctx, sizeof(double) * (size_t)tmp_rows * q));
+      BASQ_TRY(scal.alloc(ctx, 64));
+    }
+    return BASQ_OK;
+  }
+  // BASQ_ERR_NUMERIC if the grid barrier watchdog of a Cholesky kernel fired since alloc (synchronises)
+  int check_status(basq_ctx* ctx, const char* who) {
+    int status = 0;
+    BASQ_CUDA(cudaMemcpyAsync(&status, flags.as<int>() + 64, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+    BASQ_CHECK(status == 0, BASQ_ERR_NUMERIC, "%s: grid barrier watchdog fired in the Cholesky kernel", who);
+    return BASQ_OK;
+  }
 };
 
 int chol_inverse(basq_ctx* ctx, OrthWs& ws, int q, double floor_val) {
@@ -420,19 +444,12 @@ int chol_inverse(basq_ctx* ctx, OrthWs& ws, int q, double floor_val) {
 
 // Y [M, q] (ld = q) <- basis of span(Y) by shifted CholeskyQR: `passes` = 3 gives an orthonormal
 // basis to machine precision (sCholQR3); 2 is enough between subspace iterations, where only the
-// conditioning of the basis matters
-// `sh` (row-sharded basis): Y holds this rank's rows only; the Gram matrix is summed over the ranks through the
+// conditioning of the basis matters.  M_glob = rows of the whole matrix (the shift depends on it).
+// `sh` (row-sharded basis): Y holds this rank's M rows only; the Gram matrix is summed over the ranks through the
 // caller's exchange function, everything after it (trace, shift, Cholesky + inverse) is replicated and the
-// factor is applied to the local rows.  M_glob = rows of the whole matrix (the shift depends on it).
-struct ShardXchg {
-  basq_exchange_fn fn = nullptr;
-  void* user = nullptr;
-  double* gram_buf = nullptr;   // [q, q], the buffer the exchange function reduces
-};
-
-int orthonormalise(basq_ctx* ctx, OrthWs& ws, double* Y, int64_t M, int q, int passes, const ShardXchg* sh = nullptr,
-                   int64_t M_glob = 0) {
-  if (!sh) M_glob = M;
+// factor is applied to the local rows.
+int orthonormalise(basq_ctx* ctx, OrthWs& ws, double* Y, int64_t M, int q, int passes, int64_t M_glob,
+                   const NysShard* sh) {
   // passes < 0: "until orthonormal to fp64" - a pass whose input Gram matrix is within 0.1 of the
   // identity is the last one (CholeskyQR squares the distance to orthonormality); at most 4.
   const bool adaptive = passes < 0;
@@ -478,11 +495,7 @@ int orthonormalise(basq_ctx* ctx, OrthWs& ws, double* Y, int64_t M, int q, int p
       BASQ_CUDA(cudaMemcpyAsync(Y, ws.tmp.p, sizeof(double) * (size_t)M * q, cudaMemcpyDeviceToDevice, ctx->stream));
     }
   }
-  int status = 0;
-  BASQ_CUDA(cudaMemcpyAsync(&status, ws.flags.as<int>() + 64, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
-  BASQ_CHECK(status == 0, BASQ_ERR_NUMERIC, "nystrom: grid barrier watchdog fired in the Cholesky kernel");
-  return BASQ_OK;
+  return ws.check_status(ctx, "nystrom");
 }
 
 }  // namespace
@@ -492,20 +505,11 @@ int orthonormalise(basq_ctx* ctx, OrthWs& ws, double* Y, int64_t M, int q, int p
 int spd_inverse_factor(basq_ctx* ctx, const double* A, int n, double* Linv_out) {
   BASQ_CHECK(A && Linv_out && n >= 1, BASQ_ERR_INVALID, "spd_inverse_factor: bad argument");
   OrthWs ws;
-  BASQ_TRY(ws.gram.alloc(ctx, sizeof(double) * (size_t)n * n));
-  BASQ_TRY(ws.linv.alloc(ctx, sizeof(double) * (size_t)n * n));
-  BASQ_TRY(ws.prow.alloc(ctx, sizeof(double) * 4 * n));
-  BASQ_TRY(ws.prow2.alloc(ctx, sizeof(double) * 2 * (size_t)n * n));
-  BASQ_TRY(ws.flags.alloc(ctx, 512));
-  BASQ_CUDA(cudaMemsetAsync(ws.flags.p, 0, 512, ctx->stream));
+  BASQ_TRY(ws.alloc(ctx, n, 0));
   BASQ_CUDA(cudaMemcpyAsync(ws.gram.p, A, sizeof(double) * (size_t)n * n, cudaMemcpyDeviceToDevice, ctx->stream));
   BASQ_TRY(chol_inverse(ctx, ws, n, 1e-300));
   BASQ_CUDA(cudaMemcpyAsync(Linv_out, ws.linv.p, sizeof(double) * (size_t)n * n, cudaMemcpyDeviceToDevice, ctx->stream));
-  int status = 0;
-  BASQ_CUDA(cudaMemcpyAsync(&status, ws.flags.as<int>() + 64, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
-  BASQ_CHECK(status == 0, BASQ_ERR_NUMERIC, "spd_inverse_factor: grid barrier watchdog fired in the Cholesky kernel");
-  return BASQ_OK;
+  return ws.check_status(ctx, "spd_inverse_factor");
 }
 
 namespace {
@@ -534,13 +538,8 @@ int spd_chol_blocked(basq_ctx* ctx, double* A, int n) {
   const int nb = n < CHB ? n : CHB;
   OrthWs ws;
   DevBuf panel;
-  BASQ_TRY(ws.gram.alloc(ctx, sizeof(double) * (size_t)nb * nb));
-  BASQ_TRY(ws.linv.alloc(ctx, sizeof(double) * (size_t)nb * nb));
-  BASQ_TRY(ws.prow.alloc(ctx, sizeof(double) * 4 * nb));
-  BASQ_TRY(ws.prow2.alloc(ctx, sizeof(double) * 2 * (size_t)nb * nb));
-  BASQ_TRY(ws.flags.alloc(ctx, 512));
+  BASQ_TRY(ws.alloc(ctx, nb, 0));
   BASQ_TRY(panel.alloc(ctx, sizeof(double) * (size_t)n * CHB));
-  BASQ_CUDA(cudaMemsetAsync(ws.flags.p, 0, 512, ctx->stream));   // the watchdog status (byte 256) stays set once fired
   for (int k = 0; k < n; k += CHB) {
     const int b = std::min(CHB, n - k);
     double* Akk = A + (int64_t)k * n + k;
@@ -559,74 +558,101 @@ int spd_chol_blocked(basq_ctx* ctx, double* A, int n) {
                      false, /*c_lower_only=*/true));
     }
   }
-  int status = 0;
-  BASQ_CUDA(cudaMemcpyAsync(&status, ws.flags.as<int>() + 64, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
-  BASQ_CHECK(status == 0, BASQ_ERR_NUMERIC, "spd_chol_blocked: grid barrier watchdog fired in the Cholesky kernel");
-  return BASQ_OK;
+  return ws.check_status(ctx, "spd_chol_blocked");
 }
 
+// Rank r of `world` (shard == nullptr: one rank holding everything) owns rows [r chunk, min(M, (r + 1) chunk)),
+// chunk = ceil(M / world), of K(Z, Z) - it evaluates, converts and multiplies only those.  Sharded (multi-GPU), the
+// ranks meet twice per product: a sum of the q x q Gram matrices (CholeskyQR) and an all-gather of the
+// orthonormalised rows, both done by the caller's exchange function on buffers the caller owns (the library stays
+// free of any communication dependency; basq_b200/sharded.py passes torch.distributed collectives).  rows_buf
+// [world * chunk, q] is the full basis in global row order (rank r's rows at r * chunk).  The Cholesky
+// factorisations are replicated, so every rank takes the same decisions and issues the same exchanges.
 int nystrom_basis(basq_ctx* ctx, const basq_kernel_desc* desc, const void* Z, int64_t M, int q, const double* Omega,
-                  int niter, double* U_out, double* S_out) {
+                  int niter, double* U_out, double* S_out, const NysShard* shard) {
   PhaseTimer timer(ctx, PH_NYS);
   BASQ_CHECK(q >= 1 && q <= M, BASQ_ERR_INVALID, "nystrom: need 1 <= q <= M (q=%d M=%lld)", q, (long long)M);
-  BASQ_CHECK(M <= 46000, BASQ_ERR_UNSUPPORTED, "nystrom: M=%lld landmarks need a %.1f GB Gram matrix", (long long)M,
-             8.0 * M * M / 1e9);
+  const int rank = shard ? shard->rank : 0, world = shard ? shard->world : 1;
+  BASQ_CHECK(!shard || (world >= 1 && rank >= 0 && rank < world && shard->fn && shard->gram_buf && shard->rows_buf &&
+                        !S_out),
+             BASQ_ERR_INVALID, "nystrom (sharded): bad rank / world / buffers");
+  BASQ_CHECK(M <= 46000 * (int64_t)world, BASQ_ERR_UNSUPPORTED, "nystrom: M=%lld landmarks need a %.1f GB Gram matrix%s",
+             (long long)M, 8.0 * M * M / world / 1e9, shard ? " per rank" : "");
   BASQ_CHECK(niter >= 0 && niter <= 16, BASQ_ERR_INVALID, "nystrom: niter out of range");
+  const int64_t chunk = (M + world - 1) / world;
+  const int64_t row0 = std::min<int64_t>(M, (int64_t)rank * chunk);
+  const int nr = (int)(std::min<int64_t>(M, row0 + chunk) - row0);
+  const int Mi = (int)M;
+  const size_t esz = desc->dtype == BASQ_F64 ? 8 : 4;
   DevBuf K, Y, Y2, drawn;
   if (!Omega) {
     // torch.svd_lowrank draws its own Gaussian test matrix (BASQ/_rchq.py:28-31); so does the library when
-    // the caller passes none: Philox stream of key seed + number of earlier draws (basq_ctx_set_seed)
+    // the caller passes none: Philox stream of key seed + number of earlier draws (basq_ctx_set_seed), the
+    // same on every rank
     BASQ_TRY(drawn.alloc(ctx, sizeof(double) * (size_t)M * q));
     BASQ_TRY(standard_normals(ctx, ctx->seed + ctx->draws, 0, M, q, drawn.as<double>()));
     ctx->draws++;
     Omega = drawn.as<double>();
   }
-  BASQ_TRY(K.alloc(ctx, sizeof(double) * (size_t)M * M));
-  BASQ_TRY(Y.alloc(ctx, sizeof(double) * (size_t)M * q));
+  BASQ_TRY(K.alloc(ctx, sizeof(double) * (size_t)std::max(nr, 1) * M));
+  BASQ_TRY(Y.alloc(ctx, sizeof(double) * (size_t)std::max(nr, 1) * q));
+  if (!shard) BASQ_TRY(Y2.alloc(ctx, sizeof(double) * (size_t)M * q));
   OrthWs ws;
-  BASQ_TRY(ws.gram.alloc(ctx, sizeof(double) * (size_t)q * q));
-  BASQ_TRY(ws.linv.alloc(ctx, sizeof(double) * (size_t)q * q));
-  BASQ_TRY(ws.tmp.alloc(ctx, sizeof(double) * (size_t)M * q));
-  BASQ_TRY(ws.prow.alloc(ctx, sizeof(double) * 4 * q));
-  BASQ_TRY(ws.prow2.alloc(ctx, sizeof(double) * 2 * (size_t)q * q));
-  BASQ_TRY(ws.flags.alloc(ctx, 512));
-  BASQ_CUDA(cudaMemsetAsync(ws.flags.p, 0, 512, ctx->stream));
-  BASQ_TRY(ws.scal.alloc(ctx, 64));
-  const int Mi = (int)M;
-  // Y_out [M, q] = K Y_in.  fp32 kernels: on the tensor cores (fp16 hi/lo split products, tgemm.cu) - the Gram matrix itself
-  // is only fp32-accurate, and the subspace iteration re-orthonormalises in fp64 after every product;
-  // fp64 kernels: fp64 GEMM.  K is symmetric, so K^T Y = K Y.
+  BASQ_TRY(ws.alloc(ctx, q, std::max(nr, 1)));
+  // K [nr, M] = K(Z, Z)[rows, :].  fp32 kernels: products on the tensor cores (fp16 hi/lo split products, tgemm.cu) -
+  // the Gram matrix itself is only fp32-accurate, and the subspace iteration re-orthonormalises in fp64 after every
+  // product; fp64 kernels: fp64 GEMM.  K(Z, Z) is symmetric, so K^T Y = K Y.
   const bool tensor = desc->dtype == BASQ_F32;
-  BASQ_TRY(gram_matrix(ctx, desc, Z, M, Z, M, K.as<double>(), tensor));
   BlkOperand Kb, Yb;
-  if (tensor) {
-    BASQ_TRY(Kb.alloc(ctx, Mi, Mi));
-    BASQ_TRY(blk_from_f64(ctx, K.as<double>(), M, false, &Kb));
-    BASQ_TRY(Yb.alloc(ctx, q, Mi));
+  if (nr > 0) {
+    const unsigned char* Zr = static_cast<const unsigned char*>(Z) + (size_t)row0 * desc->d * esz;
+    BASQ_TRY(gram_matrix(ctx, desc, Zr, nr, Z, M, K.as<double>(), tensor, /*diag_col0=*/row0));
+    if (tensor) {
+      BASQ_TRY(Kb.alloc(ctx, nr, Mi));
+      BASQ_TRY(blk_from_f64(ctx, K.as<double>(), M, false, &Kb));
+      BASQ_TRY(Yb.alloc(ctx, q, Mi));
+    }
   }
-  auto multiply = [&](const double* Yin, double* Yout) -> int {
-    if (!tensor) return dgemm(ctx, false, false, Mi, q, Mi, 1.0, K.as<double>(), M, Yin, q, 0.0, Yout, q);
+  double* Yr = Y.as<double>();                                  // [nr, q] this rank's rows of the latest product
+  double* Yfull = shard ? shard->rows_buf : Y2.as<double>();    // [M, q] the input of the next product
+  // Yr <- K[rows, :] Yin  (Yin: a full [M, q] matrix)
+  auto multiply = [&](const double* Yin) -> int {
+    if (nr == 0) return BASQ_OK;
+    if (!tensor) return dgemm(ctx, false, false, nr, q, Mi, 1.0, K.as<double>(), M, Yin, q, 0.0, Yr, q);
     BASQ_TRY(blk_from_f64(ctx, Yin, q, true, &Yb));                 // Y^T as [q, M] operand
-    return tgemm(ctx, Yb, Kb, 1.0, Yout, q, true);                  // (Y^T K^T)^T = K Y
+    return tgemm(ctx, Yb, Kb, 1.0, Yr, q, true);                    // (Y^T K^T)^T = K Y
+  };
+  // Yfull <- every rank's Yr.  One rank: the two buffers trade roles (no copy), the next product writes the other.
+  auto publish = [&]() -> int {
+    if (!shard) {
+      std::swap(Yr, Yfull);
+      return BASQ_OK;
+    }
+    if (nr > 0)
+      BASQ_CUDA(cudaMemcpyAsync(Yfull + (size_t)row0 * q, Yr, sizeof(double) * (size_t)nr * q, cudaMemcpyDeviceToDevice,
+                                ctx->stream));
+    BASQ_CHECK(shard->fn(shard->user, BASQ_XCHG_ALLGATHER_ROWS, chunk * q) == 0, BASQ_ERR_INVALID,
+               "nystrom: the exchange function failed (all-gather of the basis rows)");
+    return BASQ_OK;
   };
   // Between products one shifted CholeskyQR pass is enough: it only has to keep the basis well
   // enough conditioned for the next product (directions it damps by more than the working precision
   // are lost to that product's rounding anyway); the last product is followed by passes until the
   // basis is orthonormal to fp64 (two at M = 1e4, q = 999, d = 10: |U U^T - I| = 9e-15; three for
   // numerically rank-deficient Gram matrices such as d = 2).
-  static const int final_passes = [] { const char* e = getenv("BASQ_NYS_FINAL_PASSES"); return e ? atoi(e) : -1; }();
-  BASQ_TRY(multiply(Omega, Y.as<double>()));
-  BASQ_TRY(orthonormalise(ctx, ws, Y.as<double>(), M, q, niter > 0 ? 1 : final_passes));
-  BASQ_TRY(Y2.alloc(ctx, sizeof(double) * (size_t)M * q));
+  constexpr int TO_FP64 = -1;   // orthonormalise's adaptive passes
+  BASQ_TRY(multiply(Omega));
+  BASQ_TRY(orthonormalise(ctx, ws, Yr, nr, q, niter > 0 ? 1 : TO_FP64, M, shard));
+  BASQ_TRY(publish());
   // Within a power iteration (K^T then K) the intermediate basis need not be re-orthonormalised when
   // the spectrum behind the basis is flat enough: two products damp the weakest captured direction by
   // (sigma_q / sigma_1)^2 relative to the strongest, which must stay well above the split product's rounding
   // (1e-7) of the second product.  sigma_q / sigma_1 is read off the diagonal of the Cholesky factor
-  // of the first CholeskyQR pass (L^-1 is at hand).  Measured at M = 1e4, q = 999, d = 10 (spread 0.38):
-  // the captured trace tr(U K U^T) agrees to 9 digits with the fully re-orthonormalised run
-  // (1530.730019 vs 1530.730022); at d = 2 (spread 1e-8) the skip would double the approximation
-  // error, and the criterion keeps every orthonormalisation.  BASQ_NYS_ORTH_MID=1 forces them all.
+  // of the first CholeskyQR pass (L^-1 is at hand, and replicated: every rank takes the same decision).
+  // Measured at M = 1e4, q = 999, d = 10 (spread 0.38): the captured trace tr(U K U^T) agrees to 9 digits
+  // with the fully re-orthonormalised run (1530.730019 vs 1530.730022); at d = 2 (spread 1e-8) the skip
+  // would double the approximation error, and the criterion keeps every orthonormalisation.
+  // BASQ_NYS_ORTH_MID=1 forces them all.
   const bool force_mid = [] { const char* e = getenv("BASQ_NYS_ORTH_MID"); return e && e[0] == '1'; }();  // read per call (tests toggle it)
   bool skip_mid = false;
   if (!force_mid && niter > 0) {
@@ -640,122 +666,24 @@ int nystrom_basis(basq_ctx* ctx, const basq_kernel_desc* desc, const void* Z, in
                             skip_mid ? "one orthonormalisation per power iteration" : "orthonormalise after every product");
   }
   for (int it = 0; it < niter; ++it) {
-    BASQ_TRY(multiply(Y.as<double>(), Y2.as<double>()));
-    if (!skip_mid) BASQ_TRY(orthonormalise(ctx, ws, Y2.as<double>(), M, q, 1));
-    BASQ_TRY(multiply(Y2.as<double>(), Y.as<double>()));
-    BASQ_TRY(orthonormalise(ctx, ws, Y.as<double>(), M, q, it + 1 == niter ? final_passes : 1));
+    BASQ_TRY(multiply(Yfull));
+    if (!skip_mid) BASQ_TRY(orthonormalise(ctx, ws, Yr, nr, q, 1, M, shard));
+    BASQ_TRY(publish());
+    BASQ_TRY(multiply(Yfull));
+    BASQ_TRY(orthonormalise(ctx, ws, Yr, nr, q, it + 1 == niter ? TO_FP64 : 1, M, shard));
+    BASQ_TRY(publish());
   }
   // U = Q^T  [q, M]
   {
     dim3 grid((unsigned)ceil_div(q, 32), (unsigned)ceil_div(Mi, 32));
-    transpose_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Y.as<double>(), Mi, q, U_out);
+    transpose_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Yfull, Mi, q, U_out);
     ctx->launches++;
   }
   if (S_out) {
-    // Rayleigh quotients q_i^T K q_i
-    BASQ_TRY(dgemm(ctx, false, false, Mi, q, Mi, 1.0, K.as<double>(), M, Y.as<double>(), q, 0.0, Y2.as<double>(), q));
-    BASQ_TRY(dgemm(ctx, true, false, q, q, Mi, 1.0, Y.as<double>(), q, Y2.as<double>(), q, 0.0, ws.gram.as<double>(), q));
+    // Rayleigh quotients q_i^T K q_i (one rank: K holds every row; Yr is free scratch)
+    BASQ_TRY(dgemm(ctx, false, false, Mi, q, Mi, 1.0, K.as<double>(), M, Yfull, q, 0.0, Yr, q));
+    BASQ_TRY(dgemm(ctx, true, false, q, q, Mi, 1.0, Yfull, q, Yr, q, 0.0, ws.gram.as<double>(), q));
     diag_kernel<<<ceil_div(q, 256), 256, 0, ctx->stream>>>(ws.gram.as<double>(), q, q, S_out);
-    ctx->launches++;
-  }
-  BASQ_CUDA(cudaGetLastError());
-  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
-  return BASQ_OK;
-}
-
-// Row-sharded variant (multi-GPU): rank r of `world` owns rows [r chunk, min(M, (r + 1) chunk)), chunk = ceil(M / world),
-// of K(Z, Z) - it evaluates, converts and multiplies only those - and the ranks meet twice per product: a sum
-// of the q x q Gram matrices (CholeskyQR) and an all-gather of the orthonormalised rows, both done by the
-// caller's exchange function on buffers the caller owns (the library stays free of any communication
-// dependency; basq_b200/sharded.py passes torch.distributed collectives).  rows_buf [world * chunk, q] is the
-// full basis in global row order (rank r's rows at r * chunk).  The Cholesky factorisations are replicated.
-int nystrom_basis_sharded(basq_ctx* ctx, const basq_kernel_desc* desc, const void* Z, int64_t M, int q,
-                          const double* Omega, int niter, int rank, int world, double* gram_buf, double* rows_buf,
-                          basq_exchange_fn fn, void* user, double* U_out) {
-  PhaseTimer timer(ctx, PH_NYS);
-  BASQ_CHECK(q >= 1 && q <= M, BASQ_ERR_INVALID, "nystrom: need 1 <= q <= M (q=%d M=%lld)", q, (long long)M);
-  BASQ_CHECK(world >= 1 && rank >= 0 && rank < world && fn && gram_buf && rows_buf, BASQ_ERR_INVALID,
-             "nystrom (sharded): bad rank / world / buffers");
-  BASQ_CHECK(M <= 46000 * (int64_t)world, BASQ_ERR_UNSUPPORTED, "nystrom: M=%lld landmarks too many", (long long)M);
-  BASQ_CHECK(niter >= 0 && niter <= 16, BASQ_ERR_INVALID, "nystrom: niter out of range");
-  const int64_t chunk = (M + world - 1) / world;
-  const int64_t row0 = std::min<int64_t>(M, (int64_t)rank * chunk);
-  const int nr = (int)(std::min<int64_t>(M, row0 + chunk) - row0);
-  const int Mi = (int)M;
-  const size_t esz = desc->dtype == BASQ_F64 ? 8 : 4;
-  ShardXchg sh;
-  sh.fn = fn; sh.user = user; sh.gram_buf = gram_buf;
-
-  DevBuf K, Yr, drawn;
-  if (!Omega) {
-    BASQ_TRY(drawn.alloc(ctx, sizeof(double) * (size_t)M * q));
-    BASQ_TRY(standard_normals(ctx, ctx->seed + ctx->draws, 0, M, q, drawn.as<double>()));   // the same on every rank
-    ctx->draws++;
-    Omega = drawn.as<double>();
-  }
-  BASQ_TRY(K.alloc(ctx, sizeof(double) * (size_t)std::max(nr, 1) * M));
-  BASQ_TRY(Yr.alloc(ctx, sizeof(double) * (size_t)std::max(nr, 1) * q));
-  OrthWs ws;
-  BASQ_TRY(ws.gram.alloc(ctx, sizeof(double) * (size_t)q * q));
-  BASQ_TRY(ws.linv.alloc(ctx, sizeof(double) * (size_t)q * q));
-  BASQ_TRY(ws.tmp.alloc(ctx, sizeof(double) * (size_t)std::max(nr, 1) * q));
-  BASQ_TRY(ws.prow.alloc(ctx, sizeof(double) * 4 * q));
-  BASQ_TRY(ws.prow2.alloc(ctx, sizeof(double) * 2 * (size_t)q * q));
-  BASQ_TRY(ws.flags.alloc(ctx, 512));
-  BASQ_CUDA(cudaMemsetAsync(ws.flags.p, 0, 512, ctx->stream));
-  BASQ_TRY(ws.scal.alloc(ctx, 64));
-  const bool tensor = desc->dtype == BASQ_F32;
-  BlkOperand Kb, Yb;
-  if (nr > 0) {
-    const unsigned char* Zr = static_cast<const unsigned char*>(Z) + (size_t)row0 * desc->d * esz;
-    BASQ_TRY(gram_matrix(ctx, desc, Zr, nr, Z, M, K.as<double>(), tensor, /*diag_col0=*/row0));
-    if (tensor) {
-      BASQ_TRY(Kb.alloc(ctx, nr, Mi));
-      BASQ_TRY(blk_from_f64(ctx, K.as<double>(), M, false, &Kb));
-      BASQ_TRY(Yb.alloc(ctx, q, Mi));
-    }
-  }
-  // Yr [nr, q] = K[rows, :] Yin  (Yin: the full [M, q] matrix)
-  auto multiply = [&](const double* Yin) -> int {
-    if (nr == 0) return BASQ_OK;
-    if (!tensor) return dgemm(ctx, false, false, nr, q, Mi, 1.0, K.as<double>(), M, Yin, q, 0.0, Yr.as<double>(), q);
-    BASQ_TRY(blk_from_f64(ctx, Yin, q, true, &Yb));
-    return tgemm(ctx, Yb, Kb, 1.0, Yr.as<double>(), q, true);
-  };
-  // this rank's rows into the shared layout, then every rank's
-  auto gather = [&]() -> int {
-    if (nr > 0)
-      BASQ_CUDA(cudaMemcpyAsync(rows_buf + (size_t)row0 * q, Yr.p, sizeof(double) * (size_t)nr * q, cudaMemcpyDeviceToDevice,
-                                ctx->stream));
-    BASQ_CHECK(fn(user, BASQ_XCHG_ALLGATHER_ROWS, chunk * q) == 0, BASQ_ERR_INVALID,
-               "nystrom: the exchange function failed (all-gather of the basis rows)");
-    return BASQ_OK;
-  };
-  static const int final_passes = [] { const char* e = getenv("BASQ_NYS_FINAL_PASSES"); return e ? atoi(e) : -1; }();
-  BASQ_TRY(multiply(Omega));
-  BASQ_TRY(orthonormalise(ctx, ws, Yr.as<double>(), nr, q, niter > 0 ? 1 : final_passes, &sh, M));
-  BASQ_TRY(gather());
-  const bool force_mid = [] { const char* e = getenv("BASQ_NYS_ORTH_MID"); return e && e[0] == '1'; }();
-  bool skip_mid = false;
-  if (!force_mid && niter > 0) {   // the factor is replicated: every rank takes the same decision
-    diag_spread_kernel<<<1, 256, 0, ctx->stream>>>(ws.linv.as<double>(), q, q, ws.scal.as<double>());
-    ctx->launches++;
-    double spread = 0.0;
-    BASQ_CUDA(cudaMemcpyAsync(&spread, ws.scal.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
-    skip_mid = spread > 1e-2;
-  }
-  for (int it = 0; it < niter; ++it) {
-    BASQ_TRY(multiply(rows_buf));
-    if (!skip_mid) BASQ_TRY(orthonormalise(ctx, ws, Yr.as<double>(), nr, q, 1, &sh, M));
-    BASQ_TRY(gather());
-    BASQ_TRY(multiply(rows_buf));
-    BASQ_TRY(orthonormalise(ctx, ws, Yr.as<double>(), nr, q, it + 1 == niter ? final_passes : 1, &sh, M));
-    BASQ_TRY(gather());
-  }
-  {
-    dim3 grid((unsigned)ceil_div(q, 32), (unsigned)ceil_div(Mi, 32));
-    transpose_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(rows_buf, Mi, q, U_out);
     ctx->launches++;
   }
   BASQ_CUDA(cudaGetLastError());

@@ -1,5 +1,5 @@
 """One-off probes: (1) cuBLAS fp64 GEMM rate on the projection shape vs basq_dgemm; (2) orthonormality
-of the Nystrom basis for BASQ_NYS_FINAL_PASSES (set in the environment before the run)."""
+and captured trace of the Nystrom basis."""
 import math, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -44,5 +44,5 @@ if "nys" in sys.argv:
     # captured energy of the posterior-covariance Gram in span(U), relative to the exact top-q eigenspace
     ev = torch.linalg.eigvalsh(Kp)
     cap = torch.trace(U @ Kp @ U.T)
-    print(f"nystrom final_passes={os.environ.get('BASQ_NYS_FINAL_PASSES', '3')}: {t:.2f} ms  |UU^T-I|_max={float(E.abs().max()):.2e}  "
+    print(f"nystrom: {t:.2f} ms  |UU^T-I|_max={float(E.abs().max()):.2e}  "
           f"captured trace {float(cap):.6f} vs top-q eigenvalues {float(ev[-q:].sum()):.6f} (total {float(ev.sum()):.6f})")

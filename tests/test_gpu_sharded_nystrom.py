@@ -29,12 +29,16 @@ def _case(kind):
     return Z, omega, q, kern
 
 
-@pytest.mark.parametrize("kind", ["plain", "pred_cov_noise_diag"])
-def test_one_shard_equals_the_plain_entry(kind):
+@pytest.mark.parametrize("kind,dtype,niter", [
+    pytest.param(kind, dtype, niter, id=kind + suffix)
+    for dtype, niter, suffix in [(torch.float32, 2, ""), (torch.float64, 2, "-fp64"), (torch.float32, 0, "-niter0")]
+    for kind in ("plain", "pred_cov_noise_diag")])
+def test_one_shard_equals_the_plain_entry(kind, dtype, niter):
     from basq_b200 import ops, sharded
     Z, omega, q, kern = _case(kind)
-    _, U0 = ops.nystrom_basis(kern, Z.to(DEV), q, omega=omega.to(DEV), want_S=False)
-    U1 = sharded.nystrom_basis_sharded(kern, Z.to(DEV), q, omega=omega.to(DEV))
+    Z = Z.to(DEV, dtype)
+    _, U0 = ops.nystrom_basis(kern, Z, q, omega=omega.to(DEV), niter=niter, want_S=False)
+    U1 = sharded.nystrom_basis_sharded(kern, Z, q, omega=omega.to(DEV), niter=niter)
     assert torch.equal(U0, U1)
 
 
