@@ -117,19 +117,77 @@ __global__ void row_l1_max_kernel(const double* __restrict__ A, int rows, int co
   if (threadIdx.x == 0) atomicMax(out, (unsigned long long)__double_as_longlong(sh[0]));
 }
 
-}  // namespace
-
-int narrow_f64(basq_ctx* ctx, const double* in, int64_t n, float* out) {
-  f64_to_f32_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(in, n, out);
+// dst = src [rows, d] in `dtype`, converted from the other precision; zero rows get a one-row allocation
+int convert_rows(basq_ctx* ctx, int dtype, const void* src, int64_t rows, int d, DevBuf* dst) {
+  const size_t esz = dtype == BASQ_F32 ? sizeof(float) : sizeof(double);
+  BASQ_TRY(dst->alloc(ctx, esz * (size_t)std::max<int64_t>(rows, 1) * d));
+  const int64_t n = rows * d;
+  if (n == 0) return BASQ_OK;
+  if (dtype == BASQ_F32)
+    f64_to_f32_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>((const double*)src, n, dst->as<float>());
+  else
+    f32_to_f64_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>((const float*)src, n, dst->as<double>());
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
   return BASQ_OK;
 }
 
-int widen_f32(basq_ctx* ctx, const float* in, int64_t n, double* out) {
-  f32_to_f64_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(in, n, out);
-  ctx->launches++;
-  BASQ_CUDA(cudaGetLastError());
+}  // namespace
+
+int EvalRoute::copy_points(basq_ctx* ctx, int dtype) {
+  for (int i = 0; i < 2; ++i) {
+    if (i == 1 && src_[1] == src_[0] && rows_[1] == rows_[0]) {
+      pts[1] = pts[0];
+      break;
+    }
+    BASQ_TRY(convert_rows(ctx, dtype, src_[i], rows_[i], caller_.d, &copies_[i]));
+    pts[i] = copies_[i].p;
+  }
+  return BASQ_OK;
+}
+
+int EvalRoute::begin(basq_ctx* ctx, const basq_kernel_desc* caller, const void* a, int64_t na, const void* b,
+                     int64_t nb) {
+  desc = caller_ = *caller;
+  pts[0] = src_[0] = a;
+  pts[1] = src_[1] = b;
+  rows_[0] = na;
+  rows_[1] = nb;
+  if (caller->dtype != BASQ_F64 || !ctx->eval_f32) return BASQ_OK;
+  // opt-in: evaluate the kernel in fp32 (tensor-core set sums) although the caller's arrays are fp64 - SOBER runs
+  // everything in torch.double (SOBER/_settings.py:4-11); accumulation, projection and Caratheodory stay fp64 as on
+  // the fp32 path, and the caller's conditioning guard may still send the call back to fp64
+  BASQ_TRY(copy_points(ctx, BASQ_F32));
+  if (caller->mode != BASQ_PLAIN) {
+    BASQ_TRY(convert_rows(ctx, BASQ_F32, caller->Xobs, caller->n_obs, caller->d, &copies_[2]));
+    desc.Xobs = copies_[2].p;
+    desc.Xobs_f64 = static_cast<const double*>(caller->Xobs);
+  }
+  desc.dtype = BASQ_F32;
+  demoted_ = true;
+  ctx->demotions++;
+  return BASQ_OK;
+}
+
+int EvalRoute::promote(basq_ctx* ctx) {
+  ctx->promotions++;
+  if (demoted_) {   // the caller's arrays were fp64 to begin with: go back to them
+    for (DevBuf& c : copies_) c.release();
+    desc = caller_;
+    pts[0] = src_[0];
+    pts[1] = src_[1];
+    return BASQ_OK;
+  }
+  BASQ_TRY(copy_points(ctx, BASQ_F64));
+  if (desc.mode != BASQ_PLAIN) {
+    if (desc.Xobs_f64) {
+      desc.Xobs = desc.Xobs_f64;   // W belongs to these coordinates, not to their fp32 roundings
+    } else {
+      BASQ_TRY(convert_rows(ctx, BASQ_F64, desc.Xobs, desc.n_obs, desc.d, &copies_[2]));
+      desc.Xobs = copies_[2].p;
+    }
+  }
+  desc.dtype = BASQ_F64;
   return BASQ_OK;
 }
 
@@ -191,20 +249,13 @@ struct basq_session {
   int raw_cur = 0;
   DevBuf lnode, lppos, lfpar;  // device copies of a level's node ids, parent positions, parent factors
   NlSweep nls;      // set sums of the non-linear modes (tensor-core operands or chunk buffers)
-  // fp32 inputs whose posterior correction would amplify the fp32 kernel noise beyond tolerance are
-  // promoted to the all-fp64 path (session_create_impl): fp64 copies of the inputs live here
-  DevBuf X64, Z64, Xobs64;
-  bool promoted = false;
+  // the precision the session evaluates in (session_create_impl); holds the narrowed or widened input copies
+  EvalRoute route;
   double kappa = 0.0;
   int64_t idx_base = 0;
   bool scale_wf = true;
   std::vector<double> omega_host;
   std::vector<int> rank_host;
-  // fp64 inputs evaluated in fp32 at the caller's request (basq_ctx_allow_f32_eval): narrowed copies, and the
-  // original fp64 arrays in case the conditioning guard sends the session back to the fp64 path
-  DevBuf X32, Z32, Xobs32;
-  bool demoted = false;
-  const void *origX = nullptr, *origZ = nullptr, *origXobs = nullptr;
 };
 
 namespace basq {
@@ -326,33 +377,6 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
   BASQ_CHECK(q >= 1 && M >= q, BASQ_ERR_INVALID, "session: need 1 <= q <= M (q=%d, M=%lld)", q, (long long)M);
   BASQ_CHECK(M <= 1000000, BASQ_ERR_UNSUPPORTED, "session: more than 1e6 landmarks");
   s->ctx = ctx;
-  if (desc->dtype == BASQ_F64 && ctx->eval_f32 && !s->promoted && !s->demoted) {
-    // opt-in: evaluate the kernel in fp32 (tensor-core set sums) although the caller's arrays are fp64 - SOBER
-    // runs everything in torch.double (SOBER/_settings.py:4-11); accumulation, projection and Caratheodory stay
-    // fp64 as on the fp32 path, and the conditioning guard below may still send the session back to fp64
-    const int d = desc->d;
-    auto narrow = [&](const void* src, int64_t rows, DevBuf* dst) -> int {
-      BASQ_TRY(dst->alloc(ctx, sizeof(float) * (size_t)std::max<int64_t>(rows, 1) * d));
-      if (rows > 0) BASQ_TRY(narrow_f64(ctx, (const double*)src, rows * d, dst->as<float>()));
-      return BASQ_OK;
-    };
-    BASQ_TRY(narrow(X, N_loc, &s->X32));
-    BASQ_TRY(narrow(Z, M, &s->Z32));
-    basq_kernel_desc d32 = *desc;
-    d32.dtype = BASQ_F32;
-    if (desc->mode != BASQ_PLAIN) {
-      BASQ_TRY(narrow(desc->Xobs, desc->n_obs, &s->Xobs32));
-      d32.Xobs = s->Xobs32.p;
-      d32.Xobs_f64 = static_cast<const double*>(desc->Xobs);
-    }
-    s->demoted = true;
-    s->origX = X; s->origZ = Z; s->origXobs = desc->Xobs;
-    ctx->demotions++;
-    return session_create_impl(ctx, &d32, s->X32.p, N_loc, N_glob, idx_base, s->Z32.p, M, U, q, mu, S_override, s);
-  }
-  s->desc = *desc;
-  BASQ_TRY(make_kparams(desc, &s->kp));
-  BASQ_TRY(compute_center(ctx, desc, Z, M, &s->kp));
   s->M = (int)M;
   s->q = q;
   s->n = q + 1;
@@ -364,55 +388,29 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
   const bool nonlin = (mode == BASQ_WSABI_M || mode == BASQ_MMLT_G);
   s->nl = mode == BASQ_WSABI_M ? NL_WSABIM : (mode == BASQ_MMLT_G ? NL_MMLT : NL_LIN);
   s->scale_wf = !nonlin;
-
-  if (mode != BASQ_PLAIN) BASQ_TRY(prep_landmarks(ctx, s->kp, desc->dtype, desc->Xobs, n_obs, nullptr, 0, &s->lmobs));
   const bool augment = (mode == BASQ_PRED_COV || mode == BASQ_WSABI_L);
-  BASQ_TRY(prep_landmarks(ctx, s->kp, desc->dtype, Z, M, augment ? desc->Xobs : nullptr, augment ? n_obs : 0, &s->lm));
-  s->Mtot = s->lm.count;
 
-  if (mode != BASQ_PLAIN) {
+  // From here on the session evaluates on the route's arrays.  At most two attempts: an fp32 one whose conditioning
+  // guard trips is dropped and redone in fp64.
+  BASQ_TRY(s->route.begin(ctx, desc, X, N_loc, Z, M));
+  for (;;) {
+    desc = &s->route.desc;
+    X = s->route.pts[0];
+    Z = s->route.pts[1];
+    s->desc = *desc;
+    BASQ_TRY(make_kparams(desc, &s->kp));
+    BASQ_TRY(compute_center(ctx, desc, Z, M, &s->kp));
+    if (mode != BASQ_PLAIN) BASQ_TRY(prep_landmarks(ctx, s->kp, desc->dtype, desc->Xobs, n_obs, nullptr, 0, &s->lmobs));
+    BASQ_TRY(prep_landmarks(ctx, s->kp, desc->dtype, Z, M, augment ? desc->Xobs : nullptr, augment ? n_obs : 0, &s->lm));
+    s->Mtot = s->lm.count;
+    if (mode == BASQ_PLAIN) break;
     BASQ_TRY(s->Az.alloc(ctx, sizeof(double) * (size_t)M * n_obs));
     BASQ_TRY(posterior_az(ctx, desc, s->kp, s->lm.view(0, (int)M), s->Az.as<double>(), &s->kappa));
-    if (desc->dtype == BASQ_F32 && ctx->kappa_max > 0.0 && s->kappa > ctx->kappa_max) {
-      // promote: fp64 copies of X, Z, Xobs, then the same construction with dtype = F64
-      const int d = desc->d;
-      auto widen = [&](const void* src, int64_t rows, DevBuf* dst) -> int {
-        BASQ_TRY(dst->alloc(ctx, sizeof(double) * (size_t)std::max<int64_t>(rows, 1) * d));
-        if (rows > 0) BASQ_TRY(widen_f32(ctx, (const float*)src, rows * d, dst->as<double>()));
-        return BASQ_OK;
-      };
-      if (s->demoted) {   // the caller's arrays were fp64 to begin with: go back to them
-        s->lm.zz.release(); s->lm.b.release(); s->lm.lmA.release();
-        s->lmobs.zz.release(); s->lmobs.b.release(); s->lmobs.lmA.release();
-        s->Az.release();
-        s->X32.release(); s->Z32.release(); s->Xobs32.release();
-        basq_kernel_desc d64 = *desc;
-        d64.dtype = BASQ_F64;
-        d64.Xobs = s->origXobs;
-        d64.Xobs_f64 = nullptr;
-        s->promoted = true;
-        ctx->promotions++;
-        return session_create_impl(ctx, &d64, s->origX, N_loc, N_glob, idx_base, s->origZ, M, U, q, mu, S_override, s);
-      }
-      BASQ_TRY(widen(X, N_loc, &s->X64));
-      BASQ_TRY(widen(Z, M, &s->Z64));
-      if (desc->Xobs_f64) {
-        BASQ_TRY(s->Xobs64.alloc(ctx, sizeof(double) * (size_t)n_obs * d));
-        BASQ_CUDA(cudaMemcpyAsync(s->Xobs64.p, desc->Xobs_f64, sizeof(double) * (size_t)n_obs * d, cudaMemcpyDeviceToDevice,
-                                  ctx->stream));
-      } else {
-        BASQ_TRY(widen(desc->Xobs, n_obs, &s->Xobs64));
-      }
-      s->lm.zz.release(); s->lm.b.release(); s->lm.lmA.release();
-      s->lmobs.zz.release(); s->lmobs.b.release(); s->lmobs.lmA.release();
-      s->Az.release();
-      basq_kernel_desc d64 = *desc;
-      d64.dtype = BASQ_F64;
-      d64.Xobs = s->Xobs64.p;
-      s->promoted = true;
-      ctx->promotions++;
-      return session_create_impl(ctx, &d64, s->X64.p, N_loc, N_glob, idx_base, s->Z64.p, M, U, q, mu, S_override, s);
-    }
+    if (!(s->route.can_promote(ctx) && s->kappa > ctx->kappa_max)) break;
+    s->lm.release();
+    s->lmobs.release();
+    s->Az.release();
+    BASQ_TRY(s->route.promote(ctx));
   }
 
   // per-landmark and per-point factors of the warped kernels

@@ -414,6 +414,11 @@ struct Landmarks {
   DevBuf zz;
   DevBuf b;
   DevBuf lmA;
+  void release() {
+    zz.release();
+    b.release();
+    lmA.release();
+  }
   LmView view(int first = 0, int cnt = -1) const {
     LmView v;
     if (cnt < 0) cnt = count - first;
@@ -538,9 +543,27 @@ int caratheodory(basq_ctx* ctx, double* A, int n, int S, int lda, double* omega_
 // (noise, jitter) then sit at (i, diag_col0 + i)
 int gram_matrix(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t a, const void* Y, int64_t b,
                 double* out, bool tensor_correction, int64_t diag_col0 = 0);
-// out[n] (fp32) = in[n] (fp64), rounded to nearest
-int narrow_f64(basq_ctx* ctx, const double* in, int64_t n, float* out);
-int widen_f32(basq_ctx* ctx, const float* in, int64_t n, double* out);
+// The arrays a call evaluates the kernel on, in the precision it evaluates it in (sessions, weighted double sums).
+// begin: fp64 inputs are narrowed to fp32 when the caller opted in (basq_ctx_allow_f32_eval; counts a demotion),
+// Xobs_f64 then keeps the caller's observations.  promote: after the caller's conditioning guard tripped on an fp32
+// evaluation, the call restarts in fp64 - on the caller's own arrays after a demotion, else on widened copies with
+// the observations from Xobs_f64 (widened when it is NULL); counts a promotion.  After it can_promote is false.
+struct EvalRoute {
+  basq_kernel_desc desc;                   // what evaluation sees: dtype, Xobs
+  const void* pts[2] = {nullptr, nullptr}; // the two point sets in desc.dtype (session: X, Z; double sums: X, Y)
+  // b == a with nb == na (the symmetric double sum) shares one copy; a set of zero rows gets no copy
+  int begin(basq_ctx* ctx, const basq_kernel_desc* caller, const void* a, int64_t na, const void* b, int64_t nb);
+  bool can_promote(const basq_ctx* ctx) const { return desc.dtype == BASQ_F32 && ctx->kappa_max > 0.0; }
+  int promote(basq_ctx* ctx);
+
+ private:
+  int copy_points(basq_ctx* ctx, int dtype);
+  basq_kernel_desc caller_;
+  const void* src_[2] = {nullptr, nullptr};
+  int64_t rows_[2] = {0, 0};
+  DevBuf copies_[3];   // the point sets and the observations in the other precision
+  bool demoted_ = false;
+};
 // Landmark side of the posterior modes, shared by sessions and the weighted double sums (quadform.cu):
 // Az[M, n_obs] = K(Z, Xobs) W for the prepared landmarks lmz (M = lmz.count) and the conditioning guard's
 // kappa = max_m |Az_m|_1 (also stored in ctx->last_kappa; synchronises)

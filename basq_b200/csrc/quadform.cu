@@ -249,20 +249,9 @@ int all_rows_kappa(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& k
   return BASQ_OK;
 }
 
-int copy_widened(basq_ctx* ctx, const void* src, int64_t count, DevBuf* dst) {
-  BASQ_TRY(dst->alloc(ctx, sizeof(double) * (size_t)count));
-  return widen_f32(ctx, (const float*)src, count, dst->as<double>());
-}
-
-int copy_narrowed(basq_ctx* ctx, const void* src, int64_t count, DevBuf* dst) {
-  BASQ_TRY(dst->alloc(ctx, sizeof(float) * (size_t)count));
-  return narrow_f64(ctx, (const double*)src, count, dst->as<float>());
-}
-
-// sym: Q(X, a) (Y, b ignored); else B(X, a; Y, b).  may_demote: basq_ctx_allow_f32_eval applies (not after a
-// promotion back to fp64).
+// sym: Q(X, a) (Y, b ignored); else B(X, a; Y, b)
 int form_impl(basq_ctx* ctx, const basq_kernel_desc* desc_in, const void* X, int64_t N, const double* a,
-              const void* Y, int64_t Mb, const double* b, bool sym, double* out_host, bool may_demote) {
+              const void* Y, int64_t Mb, const double* b, bool sym, double* out_host) {
   const char* who = sym ? "basq_kernel_quadform" : "basq_kernel_bilinear";
   BASQ_CHECK(ctx && desc_in && X && a && out_host && (sym || (Y && b)), BASQ_ERR_INVALID, "%s: NULL argument", who);
   BASQ_CHECK(N >= 1 && (sym || Mb >= 1), BASQ_ERR_INVALID, "%s: empty operand", who);
@@ -276,53 +265,25 @@ int form_impl(basq_ctx* ctx, const basq_kernel_desc* desc_in, const void* X, int
   if (sym) { Y = X; Mb = N; b = a; }
   const bool nonlin = mode == BASQ_WSABI_M || mode == BASQ_MMLT_G;
 
-  // fp64 arrays evaluated on the fp32 path at the caller's request (basq_ctx_allow_f32_eval)
-  basq_kernel_desc dsc = *desc_in;
-  DevBuf X32, Y32, Xobs32;
-  bool demoted = false;
-  if (dsc.dtype == BASQ_F64 && ctx->eval_f32 && may_demote) {
-    BASQ_TRY(copy_narrowed(ctx, X, N * dsc.d, &X32));
-    if (!sym) BASQ_TRY(copy_narrowed(ctx, Y, Mb * dsc.d, &Y32));
-    if (mode != BASQ_PLAIN) {
-      BASQ_TRY(copy_narrowed(ctx, dsc.Xobs, (int64_t)dsc.n_obs * dsc.d, &Xobs32));
-      dsc.Xobs_f64 = static_cast<const double*>(dsc.Xobs);
-      dsc.Xobs = Xobs32.p;
-    }
-    dsc.dtype = BASQ_F32;
-    demoted = true;
-    ctx->demotions++;
-  }
-  const basq_kernel_desc* desc = &dsc;
-  const void* Xe = demoted ? X32.p : X;
-  const void* Ye = sym ? Xe : (demoted ? Y32.p : Y);
-  const size_t esz = desc->dtype == BASQ_F32 ? 4 : 8;
-
+  EvalRoute route;
+  BASQ_TRY(route.begin(ctx, desc_in, X, N, Y, Mb));
+  const basq_kernel_desc* desc = &route.desc;
   KParams kp;
   BASQ_TRY(make_kparams(desc, &kp));
-  BASQ_TRY(compute_center(ctx, desc, Xe, N, &kp));
-
-  if (nonlin && desc->dtype == BASQ_F32 && ctx->kappa_max > 0.0) {
+  BASQ_TRY(compute_center(ctx, desc, route.pts[0], N, &kp));
+  if (nonlin && route.can_promote(ctx)) {
     // conditioning guard, over every landmark row before the sweep (as sessions do for Z)
     double kappa = 0.0;
-    BASQ_TRY(all_rows_kappa(ctx, desc, kp, Xe, N, &kappa));
+    BASQ_TRY(all_rows_kappa(ctx, desc, kp, route.pts[0], N, &kappa));
     if (kappa > ctx->kappa_max) {
-      ctx->promotions++;
-      if (demoted) return form_impl(ctx, desc_in, X, N, a, Y, Mb, b, sym, out_host, false);
-      DevBuf X64, Y64, Xobs64;
-      BASQ_TRY(copy_widened(ctx, X, N * desc->d, &X64));
-      if (!sym) BASQ_TRY(copy_widened(ctx, Y, Mb * desc->d, &Y64));
-      basq_kernel_desc d64 = *desc_in;
-      d64.dtype = BASQ_F64;
-      if (desc_in->Xobs_f64) {
-        d64.Xobs = desc_in->Xobs_f64;   // W belongs to these coordinates, not to their fp32 roundings
-      } else {
-        BASQ_TRY(copy_widened(ctx, desc_in->Xobs, (int64_t)desc_in->n_obs * desc_in->d, &Xobs64));
-        d64.Xobs = Xobs64.p;
-      }
-      d64.Xobs_f64 = nullptr;
-      return form_impl(ctx, &d64, X64.p, N, a, sym ? nullptr : Y64.p, Mb, b, sym, out_host, false);
+      BASQ_TRY(route.promote(ctx));
+      BASQ_TRY(make_kparams(desc, &kp));
+      BASQ_TRY(compute_center(ctx, desc, route.pts[0], N, &kp));
     }
   }
+  const void* Xe = route.pts[0];
+  const void* Ye = route.pts[1];
+  const size_t esz = desc->dtype == BASQ_F32 ? 4 : 8;
 
   Landmarks lmobs;
   if (mode != BASQ_PLAIN) BASQ_TRY(prep_landmarks(ctx, kp, desc->dtype, desc->Xobs, desc->n_obs, nullptr, 0, &lmobs));
@@ -436,14 +397,14 @@ extern "C" {
 
 int basq_kernel_quadform(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N, const double* a,
                          double* out_host) {
-  const int rc = basq::form_impl(ctx, desc, X, N, a, nullptr, 0, nullptr, true, out_host, true);
+  const int rc = basq::form_impl(ctx, desc, X, N, a, nullptr, 0, nullptr, true, out_host);
   if (ctx) basq_ctx_trim(ctx, -1);
   return rc;
 }
 
 int basq_kernel_bilinear(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, int64_t N, const double* a,
                          const void* Y, int64_t Mb, const double* b, double* out_host) {
-  const int rc = basq::form_impl(ctx, desc, X, N, a, Y, Mb, b, false, out_host, true);
+  const int rc = basq::form_impl(ctx, desc, X, N, a, Y, Mb, b, false, out_host);
   if (ctx) basq_ctx_trim(ctx, -1);
   return rc;
 }

@@ -82,11 +82,11 @@ class KernelSpec:
                 raise ValueError("inconsistent GP cache shapes")
             # fp64 observations beside the dtype copy: W belongs to these, and a call whose fp32 inputs are
             # promoted to the fp64 path (conditioning guard) must not evaluate k at their fp32 roundings
-            Xobs64 = Xobs if dtype == torch.float64 else self.Xobs.detach().to(device=device, dtype=torch.float64).contiguous()
-            keep += [Xobs, W, alpha, Xobs64]
+            Xobs_f64 = Xobs if dtype == torch.float64 else self.Xobs.detach().to(device=device, dtype=torch.float64).contiguous()
+            keep += [Xobs, W, alpha, Xobs_f64]
             desc.n_obs = len(Xobs)
             desc.Xobs, desc.W, desc.alpha = Xobs.data_ptr(), W.data_ptr(), alpha.data_ptr()
-            desc.Xobs_f64 = Xobs64.data_ptr()
+            desc.Xobs_f64 = Xobs_f64.data_ptr()
         return desc, keep
 
 
