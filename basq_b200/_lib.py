@@ -92,6 +92,13 @@ def _load():
         "basq_candidate_weights": (I, [P, I, D, I, P, P, L, I, P]),
         "basq_cleanse_weights": (I, [P, P, L, D]),
         "basq_sir_resample": (I, [P, P, L, L, C.c_uint64, P, C.POINTER(L)]),
+        "basq_weights_sum": (I, [P, P, L, C.POINTER(D)]),
+        "basq_weights_normalise": (I, [P, P, L, D, L]),
+        "basq_weights_cleanse": (I, [P, P, L, D]),
+        "basq_sir_keys": (I, [P, P, L, C.c_uint64, L, P]),
+        "basq_sir_histogram": (I, [P, P, L, C.c_uint64, C.c_uint64, I, P]),
+        "basq_sir_collect": (I, [P, P, L, C.c_uint64, L, L, P, P, C.POINTER(L)]),
+        "basq_sir_sort": (I, [P, P, P, L]),
         "basq_dgemm": (I, [P, I, I, I, I, I, D, P, I, P, I, D, P, I]),
         "basq_tgemm": (I, [P, I, I, I, P, I, P, I, P, I]),
         "basq_igemm": (I, [P, I, I, I, P, I, I, I, P, I, P, I, I]),

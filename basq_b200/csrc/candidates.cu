@@ -9,6 +9,8 @@
 //                          PI_BQ.lfi (SOBER/_pi.py:121-139)
 //   basq_cleanse_weights   WeightsStabiliser.cleansing_weights (SOBER/_weights.py:21-38)
 //   basq_sir_resample      UncertaintySampler.SIR = torch.multinomial(weights, n) (BASQ/_sampler.py:104-118)
+//   basq_weights_*,        the same stages on one shard of a row-sharded candidate set; the caller sums their
+//   basq_sir_*             host results over the ranks (basq_b200/sharded.py)
 //
 // Random numbers: Philox4x32-10 (Salmon et al., SC'11), counter = (sample index lo, hi, block of 4
 // dimensions, 0), key = 64-bit seed.  A sample depends only on (seed, global index), so shards drawn
@@ -191,6 +193,16 @@ __global__ void scale_or_fill_kernel(double* __restrict__ w, int64_t N, const do
 // like n successive draws proportional to the remaining weights.  u_i = Philox(seed; i): a 53-bit
 // uniform from two output words ((r0 >> 5) 2^26 + (r1 >> 6) + 0.5) 2^-53, so that the keys of 1e7+
 // candidates are distinct and their gaps resolved (a 24-bit uniform has 1.6e7 values in all).
+// The key of global row g with weight wi > 0; the counter depends on the row alone, so a shard that passes its
+// first global row draws the same keys as the whole set.
+__device__ __forceinline__ double sir_key(uint64_t g, uint64_t seed, double wi) {
+  uint32_t r[4];
+  philox4x32_10((uint32_t)g, (uint32_t)(g >> 32), 0u, 0x53495200u /* "SIR" stream */, (uint32_t)seed,
+                (uint32_t)(seed >> 32), r);
+  const double u = ((double)(r[0] >> 5) * 67108864.0 + (double)(r[1] >> 6) + 0.5) * 1.1102230246251565e-16;  // 2^-53
+  return -log(u) / wi;
+}
+
 // This kernel appends every (key, index) with key < cut to out (unordered; the host sorts the few
 // survivors) and counts them.
 __global__ void sir_keys_kernel(const double* __restrict__ w, int64_t N, uint64_t seed, double cut, int64_t cap,
@@ -200,11 +212,7 @@ __global__ void sir_keys_kernel(const double* __restrict__ w, int64_t N, uint64_
   if (i >= N) return;
   const double wi = w[i];
   if (!(wi > 0.0)) return;
-  uint32_t r[4];
-  philox4x32_10((uint32_t)i, (uint32_t)((uint64_t)i >> 32), 0u, 0x53495200u /* "SIR" stream */, (uint32_t)seed,
-                (uint32_t)(seed >> 32), r);
-  const double u = ((double)(r[0] >> 5) * 67108864.0 + (double)(r[1] >> 6) + 0.5) * 1.1102230246251565e-16;  // 2^-53
-  const double key = -log(u) / wi;
+  const double key = sir_key((uint64_t)i, seed, wi);
   if (key < cut) {
     const unsigned long long slot = atomicAdd(count, 1ull);
     if ((int64_t)slot < cap) {
@@ -212,6 +220,209 @@ __global__ void sir_keys_kernel(const double* __restrict__ w, int64_t N, uint64_
       idx_out[slot] = i;
     }
   }
+}
+
+// ---- the race over a sharded candidate set: device selection of the n smallest keys ------------------------
+// Keys are non-negative doubles, so they order like their bit patterns as uint64.  Rows without a key (weight
+// not > 0, or a key that overflowed to +inf, which basq_sir_resample never draws either) hold SIR_NO_KEY,
+// which sorts after every key and falls into histogram bin SIR_BINS - 1 of the first digit (a key's sign bit
+// is 0, so its first digit is below 1024).
+constexpr uint64_t SIR_NO_KEY = ~0ull;
+constexpr int SIR_BINS = 1 << BASQ_SIR_DIGIT_BITS;
+constexpr int TILE_THREADS = 256, TILE_ITEMS = 16, TILE = TILE_THREADS * TILE_ITEMS;
+constexpr unsigned FULL = 0xffffffffu;
+
+__global__ void sir_race_keys_kernel(const double* __restrict__ w, int64_t N, uint64_t seed, int64_t idx_base,
+                                     uint64_t* __restrict__ keys) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  const double wi = w[i];
+  uint64_t k = SIR_NO_KEY;
+  if (wi > 0.0) {
+    const double key = sir_key((uint64_t)(idx_base + i), seed, wi);
+    if (key < INFINITY) k = (uint64_t)__double_as_longlong(key);
+  }
+  keys[i] = k;
+}
+
+// hist[digit] += #{keys k : (k & mask) == bits}, digit = (k >> shift) mod SIR_BINS.  Warp-uniform loop so that
+// lanes with the same digit (the leading digit holds a key's exponent: few bins, many keys) add once.
+__global__ void __launch_bounds__(1024) sir_histogram_kernel(const uint64_t* __restrict__ keys, int64_t N,
+                                                             uint64_t mask, uint64_t bits, int shift,
+                                                             unsigned long long* __restrict__ hist) {
+  __shared__ unsigned int h[SIR_BINS];
+  for (int b = threadIdx.x; b < SIR_BINS; b += blockDim.x) h[b] = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t b0 = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); b0 < N; b0 += stride) {
+    const int64_t i = b0 + lane;
+    unsigned dig = SIR_BINS;   // none
+    if (i < N) {
+      const uint64_t k = keys[i];
+      if ((k & mask) == bits) dig = (unsigned)(k >> shift) & (SIR_BINS - 1);
+    }
+    const unsigned peers = __match_any_sync(FULL, dig);
+    if (dig < SIR_BINS && lane == __ffs(peers) - 1) atomicAdd(&h[dig], (unsigned)__popc(peers));
+  }
+  __syncthreads();
+  for (int b = threadIdx.x; b < SIR_BINS; b += blockDim.x)
+    if (h[b]) atomicAdd(&hist[b], (unsigned long long)h[b]);
+}
+
+// Exclusive prefix sum of a[n] in place (one block of 1024 threads, each folding a contiguous run), total out.
+__global__ void __launch_bounds__(1024) exclusive_scan_kernel(int64_t* __restrict__ a, int64_t n,
+                                                              int64_t* __restrict__ total) {
+  __shared__ int64_t part[1024];
+  const int t = threadIdx.x;
+  const int64_t per = (n + 1023) / 1024, lo = min(n, t * per), hi = min(n, lo + per);
+  int64_t s = 0;
+  for (int64_t i = lo; i < hi; ++i) s += a[i];
+  part[t] = s;
+  __syncthreads();
+  for (int o = 1; o < 1024; o <<= 1) {
+    const int64_t v = t >= o ? part[t - o] : 0;
+    __syncthreads();
+    part[t] += v;
+    __syncthreads();
+  }
+  s = part[t] - s;
+  for (int64_t i = lo; i < hi; ++i) {
+    const int64_t v = a[i];
+    a[i] = s;
+    s += v;
+  }
+  if (t == 1023 && total) *total = part[1023];
+}
+
+// Exclusive scan of one flag per thread across a block of TILE_THREADS; returns the block's total.
+__device__ __forceinline__ int block_scan_flag(bool f, int* rank, int* warp_tot /* smem [8] */) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned bal = __ballot_sync(FULL, f);
+  if (lane == 0) warp_tot[warp] = __popc(bal);
+  __syncthreads();
+  int before = 0, tot = 0;
+#pragma unroll
+  for (int w = 0; w < TILE_THREADS / 32; ++w) {
+    before += w < warp ? warp_tot[w] : 0;
+    tot += warp_tot[w];
+  }
+  __syncthreads();
+  *rank = before + __popc(bal & ((1u << lane) - 1u));
+  return tot;
+}
+
+// Collect: tile counts of keys <= T, then an order-preserving write of (key, global index) at the scanned offsets.
+__global__ void __launch_bounds__(TILE_THREADS) sir_tile_count_kernel(const uint64_t* __restrict__ keys, int64_t N,
+                                                                      uint64_t T, int64_t* __restrict__ counts) {
+  __shared__ int warp_tot[TILE_THREADS / 32];
+  const int64_t t0 = (int64_t)blockIdx.x * TILE;
+  int c = 0;
+#pragma unroll 4
+  for (int r = 0; r < TILE_ITEMS; ++r) {
+    const int64_t i = t0 + r * TILE_THREADS + threadIdx.x;
+    c += (i < N && keys[i] <= T) ? 1 : 0;
+  }
+  c = __reduce_add_sync(FULL, c);
+  if ((threadIdx.x & 31) == 0) warp_tot[threadIdx.x >> 5] = c;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int s = 0;
+    for (int w = 0; w < TILE_THREADS / 32; ++w) s += warp_tot[w];
+    counts[blockIdx.x] = s;
+  }
+}
+
+__global__ void __launch_bounds__(TILE_THREADS) sir_collect_kernel(const uint64_t* __restrict__ keys, int64_t N,
+                                                                   uint64_t T, int64_t idx_base,
+                                                                   const int64_t* __restrict__ offsets,
+                                                                   uint64_t* __restrict__ keys_out,
+                                                                   int64_t* __restrict__ idx_out) {
+  __shared__ int warp_tot[TILE_THREADS / 32];
+  const int64_t t0 = (int64_t)blockIdx.x * TILE;
+  int64_t pos = offsets[blockIdx.x];
+  for (int r = 0; r < TILE_ITEMS; ++r) {
+    const int64_t i = t0 + r * TILE_THREADS + threadIdx.x;
+    const uint64_t k = i < N ? keys[i] : SIR_NO_KEY;
+    const bool take = i < N && k <= T;
+    int rank;
+    const int tot = block_scan_flag(take, &rank, warp_tot);
+    if (take) {
+      keys_out[pos + rank] = k;
+      idx_out[pos + rank] = idx_base + i;
+    }
+    pos += tot;
+  }
+}
+
+// Stable LSD radix sort of (key, index) pairs, 8-bit digits: per-tile digit counts (digit-major, so that one
+// exclusive scan gives every tile its output offset per digit), then a scatter that ranks each round of
+// TILE_THREADS pairs by (warp, lane) within its digit - the input order is kept among equal digits.
+constexpr int SORT_BINS = 256;
+
+__global__ void __launch_bounds__(TILE_THREADS) sort_tile_hist_kernel(const uint64_t* __restrict__ keys, int64_t K,
+                                                                      int shift, int64_t nb,
+                                                                      int64_t* __restrict__ counts) {
+  __shared__ int h[SORT_BINS];
+  h[threadIdx.x] = 0;
+  __syncthreads();
+  const int64_t t0 = (int64_t)blockIdx.x * TILE;
+#pragma unroll 4
+  for (int r = 0; r < TILE_ITEMS; ++r) {
+    const int64_t i = t0 + r * TILE_THREADS + threadIdx.x;
+    if (i < K) atomicAdd(&h[(unsigned)(keys[i] >> shift) & (SORT_BINS - 1)], 1);
+  }
+  __syncthreads();
+  counts[(int64_t)threadIdx.x * nb + blockIdx.x] = h[threadIdx.x];
+}
+
+__global__ void __launch_bounds__(TILE_THREADS) sort_scatter_kernel(const uint64_t* __restrict__ keys_in,
+                                                                    const int64_t* __restrict__ idx_in, int64_t K,
+                                                                    int shift, int64_t nb,
+                                                                    const int64_t* __restrict__ offsets,
+                                                                    uint64_t* __restrict__ keys_out,
+                                                                    int64_t* __restrict__ idx_out) {
+  constexpr int WARPS = TILE_THREADS / 32;
+  __shared__ int64_t base[SORT_BINS];
+  __shared__ int warp_cnt[WARPS][SORT_BINS];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  base[t] = offsets[(int64_t)t * nb + blockIdx.x];
+#pragma unroll
+  for (int w = 0; w < WARPS; ++w) warp_cnt[w][t] = 0;
+  __syncthreads();
+  const int64_t t0 = (int64_t)blockIdx.x * TILE;
+  for (int r = 0; r < TILE_ITEMS; ++r) {
+    const int64_t i = t0 + r * TILE_THREADS + t;
+    if (t0 + r * TILE_THREADS >= K) break;              // block-uniform
+    const bool valid = i < K;
+    const uint64_t k = valid ? keys_in[i] : 0;
+    const unsigned dig = valid ? (unsigned)(k >> shift) & (SORT_BINS - 1) : SORT_BINS;
+    const unsigned peers = __match_any_sync(FULL, dig);
+    const int lt = __popc(peers & ((1u << lane) - 1u));
+    if (valid && lt == 0) warp_cnt[warp][dig] = __popc(peers);
+    __syncthreads();
+    if (valid) {
+      int64_t p = base[dig] + lt;
+      for (int w = 0; w < warp; ++w) p += warp_cnt[w][dig];
+      keys_out[p] = k;
+      idx_out[p] = idx_in[i];
+    }
+    __syncthreads();
+    int64_t add = 0;
+#pragma unroll
+    for (int w = 0; w < WARPS; ++w) {
+      add += warp_cnt[w][t];
+      warp_cnt[w][t] = 0;
+    }
+    base[t] += add;
+    __syncthreads();
+  }
+}
+
+__global__ void normalise_kernel(double* __restrict__ w, int64_t N, double total, double fill) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  w[i] = (total != 0.0 && isfinite(total)) ? w[i] / total : fill;
 }
 
 int pack_mvn(int d, const double* mean_host, const double* chol_host, MvnDev* p, double* log_norm) {
@@ -387,6 +598,128 @@ int basq_cleanse_weights(basq_ctx* ctx, double* w, int64_t N, double eps) {
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
   BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  return BASQ_OK;
+}
+
+int basq_weights_sum(basq_ctx* ctx, const double* w, int64_t N, double* total_host) {
+  BASQ_CHECK(ctx && (w || N == 0) && total_host, BASQ_ERR_INVALID, "basq_weights_sum: NULL argument");
+  BASQ_CHECK(N >= 0, BASQ_ERR_INVALID, "basq_weights_sum: negative size");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  *total_host = 0.0;
+  if (N == 0) return BASQ_OK;
+  DevBuf total;
+  BASQ_TRY(total.alloc(ctx, sizeof(double)));
+  BASQ_TRY(sum_device(ctx, w, N, total.as<double>()));
+  BASQ_CUDA(cudaMemcpyAsync(total_host, total.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  return BASQ_OK;
+}
+
+int basq_weights_normalise(basq_ctx* ctx, double* w, int64_t N_loc, double total, int64_t N_glob) {
+  BASQ_CHECK(ctx && (w || N_loc == 0), BASQ_ERR_INVALID, "basq_weights_normalise: NULL argument");
+  BASQ_CHECK(N_loc >= 0 && N_glob >= N_loc && N_glob >= 1, BASQ_ERR_INVALID,
+             "basq_weights_normalise: bad sizes (N_loc %lld, N_glob %lld)", (long long)N_loc, (long long)N_glob);
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  if (N_loc == 0) return BASQ_OK;
+  normalise_kernel<<<(unsigned)ceil_div64(N_loc, 256), 256, 0, ctx->stream>>>(w, N_loc, total, 1.0 / (double)N_glob);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+int basq_weights_cleanse(basq_ctx* ctx, double* w, int64_t N, double eps) {
+  BASQ_CHECK(ctx && (w || N == 0), BASQ_ERR_INVALID, "basq_weights_cleanse: NULL argument");
+  BASQ_CHECK(N >= 0, BASQ_ERR_INVALID, "basq_weights_cleanse: negative size");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  if (N == 0) return BASQ_OK;
+  cleanse_kernel<<<(unsigned)ceil_div64(N, 256), 256, 0, ctx->stream>>>(w, N, eps);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+int basq_sir_keys(basq_ctx* ctx, const double* w, int64_t N_loc, uint64_t seed, int64_t idx_base, uint64_t* keys_out) {
+  BASQ_CHECK(ctx && ((w && keys_out) || N_loc == 0), BASQ_ERR_INVALID, "basq_sir_keys: NULL argument");
+  BASQ_CHECK(N_loc >= 0 && idx_base >= 0, BASQ_ERR_INVALID, "basq_sir_keys: negative size or index base");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  if (N_loc == 0) return BASQ_OK;
+  sir_race_keys_kernel<<<(unsigned)ceil_div64(N_loc, 256), 256, 0, ctx->stream>>>(w, N_loc, seed, idx_base, keys_out);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+int basq_sir_histogram(basq_ctx* ctx, const uint64_t* keys, int64_t N_loc, uint64_t mask, uint64_t bits, int shift,
+                       int64_t* hist_host) {
+  BASQ_CHECK(ctx && (keys || N_loc == 0) && hist_host, BASQ_ERR_INVALID, "basq_sir_histogram: NULL argument");
+  BASQ_CHECK(N_loc >= 0 && shift >= 0 && shift < 64, BASQ_ERR_INVALID, "basq_sir_histogram: bad size or shift");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  for (int b = 0; b < SIR_BINS; ++b) hist_host[b] = 0;
+  if (N_loc == 0) return BASQ_OK;
+  DevBuf hist;
+  BASQ_TRY(hist.alloc(ctx, sizeof(unsigned long long) * SIR_BINS));
+  BASQ_CUDA(cudaMemsetAsync(hist.p, 0, sizeof(unsigned long long) * SIR_BINS, ctx->stream));
+  const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div64(N_loc, 1024), 2 * std::max(ctx->num_sms, 1));
+  sir_histogram_kernel<<<blocks, 1024, 0, ctx->stream>>>(keys, N_loc, mask, bits, shift,
+                                                          hist.as<unsigned long long>());
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  BASQ_CUDA(cudaMemcpyAsync(hist_host, hist.p, sizeof(int64_t) * SIR_BINS, cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  return BASQ_OK;
+}
+
+int basq_sir_collect(basq_ctx* ctx, const uint64_t* keys, int64_t N_loc, uint64_t T, int64_t idx_base, int64_t cap,
+                     uint64_t* keys_out, int64_t* idx_out, int64_t* n_out_host) {
+  BASQ_CHECK(ctx && (keys || N_loc == 0) && ((keys_out && idx_out) || cap == 0) && n_out_host, BASQ_ERR_INVALID,
+             "basq_sir_collect: NULL argument");
+  BASQ_CHECK(N_loc >= 0 && cap >= 0 && idx_base >= 0, BASQ_ERR_INVALID, "basq_sir_collect: negative argument");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  *n_out_host = 0;
+  if (N_loc == 0) return BASQ_OK;
+  const int64_t nb = ceil_div64(N_loc, TILE);
+  DevBuf offs, total;
+  BASQ_TRY(offs.alloc(ctx, sizeof(int64_t) * nb));
+  BASQ_TRY(total.alloc(ctx, sizeof(int64_t)));
+  sir_tile_count_kernel<<<(unsigned)nb, TILE_THREADS, 0, ctx->stream>>>(keys, N_loc, T, offs.as<int64_t>());
+  exclusive_scan_kernel<<<1, 1024, 0, ctx->stream>>>(offs.as<int64_t>(), nb, total.as<int64_t>());
+  ctx->launches += 2;
+  BASQ_CUDA(cudaGetLastError());
+  int64_t n = 0;
+  BASQ_CUDA(cudaMemcpyAsync(&n, total.p, sizeof(n), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  BASQ_CHECK(n <= cap, BASQ_ERR_INVALID, "basq_sir_collect: %lld keys <= T, room for %lld", (long long)n,
+             (long long)cap);
+  *n_out_host = n;
+  if (n == 0) return BASQ_OK;
+  sir_collect_kernel<<<(unsigned)nb, TILE_THREADS, 0, ctx->stream>>>(keys, N_loc, T, idx_base, offs.as<int64_t>(),
+                                                                     keys_out, idx_out);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+int basq_sir_sort(basq_ctx* ctx, uint64_t* keys, int64_t* idx, int64_t K) {
+  BASQ_CHECK(ctx && ((keys && idx) || K == 0), BASQ_ERR_INVALID, "basq_sir_sort: NULL argument");
+  BASQ_CHECK(K >= 0, BASQ_ERR_INVALID, "basq_sir_sort: negative size");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  if (K <= 1) return BASQ_OK;
+  const int64_t nb = ceil_div64(K, TILE);
+  DevBuf kt, it, counts;
+  BASQ_TRY(kt.alloc(ctx, sizeof(uint64_t) * K));
+  BASQ_TRY(it.alloc(ctx, sizeof(int64_t) * K));
+  BASQ_TRY(counts.alloc(ctx, sizeof(int64_t) * SORT_BINS * nb));
+  uint64_t* kb[2] = {keys, kt.as<uint64_t>()};
+  int64_t* ib[2] = {idx, it.as<int64_t>()};
+  for (int pass = 0; pass < 8; ++pass) {      // even number of passes: the result lands back in keys / idx
+    const int src = pass & 1, shift = 8 * pass;
+    sort_tile_hist_kernel<<<(unsigned)nb, TILE_THREADS, 0, ctx->stream>>>(kb[src], K, shift, nb, counts.as<int64_t>());
+    exclusive_scan_kernel<<<1, 1024, 0, ctx->stream>>>(counts.as<int64_t>(), SORT_BINS * nb, nullptr);
+    sort_scatter_kernel<<<(unsigned)nb, TILE_THREADS, 0, ctx->stream>>>(kb[src], ib[src], K, shift, nb,
+                                                                        counts.as<int64_t>(), kb[1 - src], ib[1 - src]);
+    ctx->launches += 3;
+    BASQ_CUDA(cudaGetLastError());
+  }
   return BASQ_OK;
 }
 

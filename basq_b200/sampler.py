@@ -17,11 +17,13 @@ from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import _lib, ops
 
 _F = {torch.float32: _lib.F32, torch.float64: _lib.F64}
+SIR_DIGIT_BITS = 11    # BASQ_SIR_DIGIT_BITS
 
 
 def _mvn_params(mean, cov=None, scale_tril=None):
@@ -115,6 +117,61 @@ def sir_indices(weights, n_return, seed=0):
 def SIR(X, weights, n_return, seed=0):
     """UncertaintySampler.SIR (BASQ/_sampler.py:104-118): ``X[torch.multinomial(weights, n_return)]``."""
     return X[sir_indices(weights, n_return, seed=seed)]
+
+
+class ShardEngine:
+    """Rank-local steps of the candidate side over a row-sharded set (basq_weights_*, basq_sir_*), the engine of
+    the functions in basq_b200.sharded, which sum the host results over the ranks between the calls.  Weights
+    are fp64 device tensors; SIR keys are int64 tensors that hold the uint64 key bits."""
+
+    def __init__(self, device):
+        self.device = torch.device(device)
+        self.ctx = _lib.context_for(self.device)
+
+    def candidate_weights(self, kernel, X, ratio):
+        """calc_weights before normalisation."""
+        if len(X) == 0:
+            return torch.empty(0, dtype=torch.float64, device=self.device)
+        mean, var = ops.gp_predict(kernel, X, space=0, want_var=True)
+        return _weights(0, ratio, False, mean, var, False)
+
+    def weights_sum(self, w) -> float:
+        out = C.c_double(0.0)
+        _lib.check(_lib.lib.basq_weights_sum(self.ctx.handle, w.data_ptr(), w.numel(), C.byref(out)))
+        return float(out.value)
+
+    def weights_normalise(self, w, total, N_glob):
+        _lib.check(_lib.lib.basq_weights_normalise(self.ctx.handle, w.data_ptr(), w.numel(), float(total), int(N_glob)))
+
+    def weights_cleanse(self, w, eps):
+        _lib.check(_lib.lib.basq_weights_cleanse(self.ctx.handle, w.data_ptr(), w.numel(), float(eps)))
+
+    def sir_keys(self, w, seed, idx_base):
+        keys = torch.empty(w.numel(), dtype=torch.int64, device=self.device)
+        _lib.check(_lib.lib.basq_sir_keys(self.ctx.handle, w.data_ptr(), w.numel(), C.c_uint64(int(seed) & (2 ** 64 - 1)),
+                                          int(idx_base), keys.data_ptr()))
+        return keys
+
+    def sir_histogram(self, keys, mask, bits, shift):
+        hist = np.zeros(1 << SIR_DIGIT_BITS, dtype=np.int64)
+        _lib.check(_lib.lib.basq_sir_histogram(self.ctx.handle, keys.data_ptr(), keys.numel(), C.c_uint64(mask),
+                                               C.c_uint64(bits), int(shift), hist.ctypes.data))
+        return hist
+
+    def sir_collect(self, keys, T, idx_base, cap):
+        ks = torch.empty(cap, dtype=torch.int64, device=self.device)
+        ids = torch.empty(cap, dtype=torch.int64, device=self.device)
+        n = C.c_int64(0)
+        _lib.check(_lib.lib.basq_sir_collect(self.ctx.handle, keys.data_ptr(), keys.numel(), C.c_uint64(T), int(idx_base),
+                                             int(cap), ks.data_ptr(), ids.data_ptr(), C.byref(n)))
+        return ks[: n.value], ids[: n.value]
+
+    def sir_sort(self, keys, idx):
+        """Stable sort of the pairs by key, in place (contiguous tensors); returns idx."""
+        if not (keys.is_contiguous() and idx.is_contiguous() and keys.numel() == idx.numel()):
+            raise ValueError("sir_sort: keys and idx must be contiguous and of the same length")
+        _lib.check(_lib.lib.basq_sir_sort(self.ctx.handle, keys.data_ptr(), idx.data_ptr(), keys.numel()))
+        return idx
 
 
 class PriorSampler:

@@ -1,4 +1,5 @@
-"""Recombination of a candidate set sharded over ranks (one process per GPU).
+"""Recombination of a candidate set sharded over ranks (one process per GPU), and the stages around it on the
+same shards: the Nystrom basis, the weighted double sums and the candidate side (acquisition weights, SIR).
 
 Per Tchernychova-Lyons pass every rank forms the barycentre numerators of ITS points
 (cell = global position mod F*S) in one sweep of kernel evaluations; for each of the pass's
@@ -332,3 +333,135 @@ def kernel_quadform_sharded(kernel, X_local, a_local, group=None) -> float:
     s = torch.tensor([total], dtype=torch.float64, device=X_local.device if nccl else "cpu")
     dist.all_reduce(s, group=group)
     return float(s.item())
+
+
+# ---- candidate side: acquisition weights, cleansing, SIR and the quadrature over a sharded candidate set ----
+# Each function runs the rank-local steps on `engine` (sampler.ShardEngine by default; tests substitute an oracle)
+# and sums their host results over the ranks.  Without a process group it degenerates to one shard.
+
+SIR_SHIFTS = (53, 42, 31, 20, 9, 0)    # radix-select passes of BASQ_SIR_DIGIT_BITS = 11 bits, from the top
+
+
+def _ranks(group):
+    on = dist.is_initialized() and dist.get_world_size(group) > 1
+    if not on:
+        return False, 1, 0, False
+    return True, dist.get_world_size(group), dist.get_rank(group), dist.get_backend(group) == "nccl"
+
+
+def _engine(engine, t):
+    if engine is not None:
+        return engine
+    from .sampler import ShardEngine
+    return ShardEngine(t.device)
+
+
+def _fold_sum(x, group, device):
+    """Sum of the per-rank values x, folded in rank order on every rank: every rank holds the same bits."""
+    on, world, _, nccl = _ranks(group)
+    if not on:
+        return float(x)
+    t = torch.tensor([float(x)], dtype=torch.float64, device=device if nccl else "cpu")
+    parts = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(parts, t, group=group)
+    total = 0.0
+    for p in parts:
+        total += float(p.item())
+    return total
+
+
+def _normalised(eng, w, N_glob, group):
+    eng.weights_normalise(w, _fold_sum(eng.weights_sum(w), group, w.device), N_glob)
+    return w
+
+
+def calc_weights_sharded(kernel, pts_rec_local, ratio, N_glob, group=None, engine=None):
+    """sampler.calc_weights for the rows pts_rec_local of a candidate set of N_glob rows sharded over the ranks:
+    this rank's weights, normalised by the sum over every rank (uniform 1 / N_glob when that is 0 or not finite)."""
+    eng = _engine(engine, pts_rec_local)
+    return _normalised(eng, eng.candidate_weights(kernel, pts_rec_local, ratio), N_glob, group)
+
+
+def cleansing_weights_sharded(w_local, N_glob, eps=float(torch.finfo(torch.float32).eps), group=None, engine=None):
+    """sampler.cleansing_weights of this rank's shard of N_glob weights (SOBER/_weights.py:21-38): the replacements
+    are per weight, the normalisation uses the sum over every rank.  Returns a new tensor."""
+    eng = _engine(engine, w_local)
+    w = w_local.detach().to(torch.float64).clone().contiguous()
+    eng.weights_cleanse(w, eps)
+    return _normalised(eng, w, N_glob, group)
+
+
+def _sum_hist(h, group, device):
+    on, _, _, nccl = _ranks(group)
+    if not on:
+        return h.copy()
+    t = torch.from_numpy(h.copy())
+    if nccl:
+        t = t.to(device)
+    dist.all_reduce(t, group=group)
+    return t.cpu().numpy()
+
+
+def sir_indices_sharded(w_local, n_return, seed=0, idx_base=0, group=None, engine=None):
+    """sampler.sir_indices over a weight vector sharded by rows: this rank holds rows [idx_base, idx_base + len)
+    and the ranks' rows follow each other in rank order.  Returns the global indices of the draws in draw order,
+    the same on every rank and equal, index for index, to sampler.sir_indices on the concatenated weights.
+
+    Every key is computed from its global row, so it has the same bits as on one GPU.  A radix select over the key
+    bits (histograms summed over the ranks, BASQ_SIR_DIGIT_BITS per pass) finds the m-th smallest key T,
+    m = min(n_return, #keys), and how many keys <= T every rank holds; the ranks gather their (key, index) pairs
+    <= T in rank order, each ascending in index, and a stable sort by key orders them by (key, index)."""
+    eng = _engine(engine, w_local)
+    on, _, _, nccl = _ranks(group)
+    w = w_local.detach().to(torch.float64).contiguous()
+    keys = eng.sir_keys(w, seed, idx_base)
+    mask = bits = below = mine = 0
+    m = None
+    for shift in SIR_SHIFTS:
+        h_loc = eng.sir_histogram(keys, mask, bits, shift)
+        if m is None:                       # first pass: the last bin holds the rows without a key
+            h_loc[-1] = 0
+        h = _sum_hist(h_loc, group, w.device)
+        if m is None:
+            m = min(int(n_return), int(h.sum()))
+            if m <= 0:
+                return torch.empty(0, dtype=torch.int64, device=w.device)
+        cum = np.cumsum(h)
+        d = int(np.searchsorted(cum, m - below))   # the digit of the m-th key: cum[d - 1] < m - below <= cum[d]
+        below += int(cum[d - 1]) if d else 0
+        mine += int(h_loc[:d].sum())
+        mask |= ((h.size - 1) << shift) & (2 ** 64 - 1)
+        bits |= d << shift
+    mine += int(h_loc[d])                   # keys equal to T
+    ks, ids = eng.sir_collect(keys, bits, idx_base, mine)
+    if len(ks) != mine:
+        raise RuntimeError(f"sir_indices_sharded: collected {len(ks)} keys, the histograms counted {mine}")
+    if on:
+        ks = torch.cat(_all_gather_var(ks, group, nccl))
+        ids = torch.cat(_all_gather_var(ids, group, nccl))
+    return eng.sir_sort(ks.contiguous(), ids.contiguous())[:m]
+
+
+def SIR_sharded(X_local, w_local, n_return, seed=0, idx_base=0, group=None, engine=None):
+    """UncertaintySampler.SIR over sharded candidates without moving any: each rank keeps the drawn rows it owns.
+    Returns (X_drawn_local, N_new_glob, new_idx_base, src_global_idx): the drawn set is numbered rank-major (this
+    rank's rows, in draw order, are rows [new_idx_base, new_idx_base + len(X_drawn_local)) of N_new_glob), ready
+    for recombination_sharded; src_global_idx are their indices in the old set."""
+    idx = sir_indices_sharded(w_local, n_return, seed=seed, idx_base=idx_base, group=group, engine=engine)
+    idx = idx.to(X_local.device)
+    mine = (idx >= idx_base) & (idx < idx_base + len(X_local))
+    src = idx[mine]
+    return X_local[src - idx_base], len(idx), int((idx < idx_base).sum()), src
+
+
+def full_quadrature_sharded(X_local, w_local, kernel, group=None):
+    """gp.full_quadrature over rows sharded across the ranks: (EZy, VarZy), EZy = w . m(X) folded over the ranks
+    in rank order, VarZy = w^T K(X, X) w from kernel_quadform_sharded.  Every rank returns the same values."""
+    from . import ops
+
+    w64 = w_local.to(device=X_local.device, dtype=torch.float64)
+    ez = 0.0
+    if len(X_local):
+        mean, _ = ops.gp_predict(kernel, X_local, space=1, want_var=False)
+        ez = float(w64 @ mean)
+    return _fold_sum(ez, group, X_local.device), kernel_quadform_sharded(kernel, X_local, w64, group=group)

@@ -328,6 +328,40 @@ int basq_cleanse_weights(basq_ctx* ctx, double* w, int64_t N, double eps);
 int basq_sir_resample(basq_ctx* ctx, const double* w, int64_t N, int64_t n_out, uint64_t seed,
                       int64_t* idx_out_host, int64_t* n_drawn_host);
 
+/* ---- candidate side over a set sharded by rows across ranks (one process per GPU) ------------ */
+/* Rank-local primitives; the caller sums their host results over the ranks between the calls
+   (basq_b200/sharded.py).  A rank holds rows [idx_base, idx_base + N_loc) of the global set.
+   Weights: *total_host = sum of w[N] in a fixed order (same inputs, same bits; 0 for N = 0; synchronises).
+   normalise divides w[N_loc] by `total` (the sum over every rank), or fills 1 / N_glob when total is 0 or
+   not finite - basq_candidate_weights(normalise = 1) and basq_cleanse_weights on one shard of the set.
+   cleanse applies the three replacements of basq_cleanse_weights (w < eps -> 0, inf / nan -> eps) without
+   normalising. */
+int basq_weights_sum(basq_ctx* ctx, const double* w, int64_t N, double* total_host);
+int basq_weights_normalise(basq_ctx* ctx, double* w, int64_t N_loc, double total, int64_t N_glob);
+int basq_weights_cleanse(basq_ctx* ctx, double* w, int64_t N, double eps);
+/* The race of basq_sir_resample over a sharded set, selected exactly on the device.
+   keys: keys_out[N_loc] = the bits (as uint64) of key_i = -log(u(seed; idx_base + i)) / w_i, the key
+         basq_sir_resample gives global row idx_base + i; rows without a key (!(w_i > 0), or a key of +inf,
+         which basq_sir_resample never draws) get ~0.  Non-negative doubles order like their bits.
+   histogram: radix select of the n-th smallest key, BASQ_SIR_DIGIT_BITS bits per pass from the top:
+         hist_host[2^BASQ_SIR_DIGIT_BITS] (HOST) = counts of the keys k with (k & mask) == bits by digit
+         (k >> shift) mod 2^BASQ_SIR_DIGIT_BITS; synchronises.  Shifts 53, 42, 31, 20, 9, 0 fix every bit;
+         after summing a pass over the ranks the caller picks the digit that holds the n-th key and adds
+         it to (mask, bits).  In the first pass (mask 0, shift 53) the keyless rows, and only they, fall
+         into the last bin.  The result is the threshold T and the number of keys <= T on every rank.
+   collect: keys_out / idx_out[n] = every (key, idx_base + i) with key <= T, ascending in i; *n_out_host = n
+         (BASQ_ERR_INVALID when n > cap).  The count is known when the call returns, the write is queued.
+   sort: stable LSD radix sort of (keys[K], idx[K]) by key, in place.  Sorting the collected pairs of all
+         ranks in rank order gives the draws of basq_sir_resample on the whole set: (key, index) ascending. */
+#define BASQ_SIR_DIGIT_BITS 11
+int basq_sir_keys(basq_ctx* ctx, const double* w, int64_t N_loc, uint64_t seed, int64_t idx_base,
+                  uint64_t* keys_out);
+int basq_sir_histogram(basq_ctx* ctx, const uint64_t* keys, int64_t N_loc, uint64_t mask, uint64_t bits,
+                       int shift, int64_t* hist_host);
+int basq_sir_collect(basq_ctx* ctx, const uint64_t* keys, int64_t N_loc, uint64_t T, int64_t idx_base,
+                     int64_t cap, uint64_t* keys_out, int64_t* idx_out, int64_t* n_out_host);
+int basq_sir_sort(basq_ctx* ctx, uint64_t* keys, int64_t* idx, int64_t K);
+
 /* ---- small dense helper exposed for tests ---------------------------------------------------- */
 /* C[m,n] = alpha * op(A) op(B) + beta * C, fp64 row-major; op = transpose when the flag is set. */
 int basq_dgemm(basq_ctx* ctx, int transA, int transB, int m, int n, int k, double alpha,
