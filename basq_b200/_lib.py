@@ -83,11 +83,17 @@ def _load():
         "basq_session_level_fold": (I, [P, I, I, P, P, L]),
         "basq_session_level_project": (I, [P, I, I, P, P, P, P, L, I, I, P]),
         "basq_session_apply_cells": (I, [P, L, L, I, P, C.POINTER(L)]),
+        "basq_session_reproducible": (I, [P, C.POINTER(I)]),
+        "basq_session_grid_maxima": (I, [P, P]),
+        "basq_session_set_grid": (I, [P, L, P]),
+        "basq_session_level_fold_exact": (I, [P, I, I, P, P, L]),
+        "basq_session_level_project_exact": (I, [P, I, I, P, P, P, P, L, P]),
         "basq_sample_mvn": (I, [P, C.c_uint64, L, L, I, I, P, P, P]),
         "basq_standard_normals": (I, [P, C.c_uint64, L, L, I, P]),
         "basq_ctx_set_seed": (I, [P, C.c_uint64]),
         "basq_ctx_memory": (I, [P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(L)]),
         "basq_ctx_allow_f32_eval": (I, [P, I, C.POINTER(L)]),
+        "basq_ctx_reproducible": (I, [P, I]),
         "basq_mvn_logpdf": (I, [P, P, L, I, I, P, P, P]),
         "basq_candidate_weights": (I, [P, I, D, I, P, P, L, I, P]),
         "basq_cleanse_weights": (I, [P, P, L, D]),
@@ -95,6 +101,8 @@ def _load():
         "basq_weights_sum": (I, [P, P, L, C.POINTER(D)]),
         "basq_weights_normalise": (I, [P, P, L, D, L]),
         "basq_weights_cleanse": (I, [P, P, L, D]),
+        "basq_weights_max": (I, [P, P, L, C.POINTER(D)]),
+        "basq_weights_sum_grid": (I, [P, P, L, D, L, P]),
         "basq_sir_keys": (I, [P, P, L, C.c_uint64, L, P]),
         "basq_sir_histogram": (I, [P, P, L, C.c_uint64, C.c_uint64, I, P]),
         "basq_sir_collect": (I, [P, P, L, C.c_uint64, L, L, P, P, C.POINTER(L)]),
@@ -125,6 +133,7 @@ class Context:
         h = C.c_void_p()
         check(lib.basq_ctx_create(int(device_index), C.c_void_p(stream_ptr or None), C.byref(h)))
         self.handle = h
+        self.is_reproducible = False      # basq_ctx_reproducible's default; only reproducible() changes it
         self.device_index = device_index
         self.stream_ptr = stream_ptr
 
@@ -157,6 +166,12 @@ class Context:
         n = C.c_int64(0)
         check(lib.basq_ctx_allow_f32_eval(self.handle, -1 if on is None else int(bool(on)), C.byref(n)))
         return int(n.value)
+
+    def reproducible(self, on: bool):
+        """Reproducible mode for the sessions created afterwards (basq_ctx_reproducible): the same rule, bit for
+        bit, on one GPU and sharded over any number of ranks."""
+        check(lib.basq_ctx_reproducible(self.handle, int(bool(on))))
+        self.is_reproducible = bool(on)
 
     def set_seed(self, seed: int):
         """Key of the library's own Gaussian draws (basq_ctx_set_seed)."""

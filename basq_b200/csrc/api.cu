@@ -254,6 +254,15 @@ struct basq_session {
   double kappa = 0.0;
   int64_t idx_base = 0;
   bool scale_wf = true;
+  // reproducible mode (basq_ctx_reproducible at creation): the next pass sums on the grids set by
+  // session_set_grid for grid_R live points - set sums, masses, objective (1.5 * 2^52 * Q each, grid_round)
+  bool repro = false;
+  double szmax = 0.0;   // max_m |sz_m| (non-linear modes): enters the bound of the set sums
+  int64_t grid_R = -1;
+  double grid_m[3] = {0.0, 0.0, 0.0};
+  double grid_m2[3] = {0.0, 0.0, 0.0};  // the finer grids of the remainders of fp64 terms (hi / lo, set_grid)
+  DevBuf G2, cellmass2, cellobj2;      // the sums of those remainders (G2: fp64 records only)
+  DevBuf Gc;                           // [Mtot + 2, S] hi + lo of the summed exact columns (project_exact)
   std::vector<double> omega_host;
   std::vector<int> rank_host;
 };
@@ -261,10 +270,14 @@ struct basq_session {
 namespace basq {
 namespace {
 
-// G[:, 0..ncols) for local records [p_lo, p_hi), set index = (off + p) mod S
-int session_set_sums(basq_session* s, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg) {
+// G[:, 0..ncols) for local records [p_lo, p_hi), set index = (off + p) mod S; grid_m != 0: on that grid
+int session_set_sums(basq_session* s, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg,
+                     double grid_m = 0.0, double grid_m2 = 0.0, double* G2 = nullptr) {
   basq_ctx* ctx = s->ctx;
   SetSumArgs a;
+  a.grid_m = grid_m;
+  a.grid_m2 = grid_m2;
+  a.G2 = G2;
   a.pool = &s->pool;
   a.lm = s->lm.view();
   a.off_glob = off;
@@ -344,18 +357,20 @@ int nl_sweep_prepare(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams&
 int nl_sweep_sums(basq_ctx* ctx, const KParams& kp, int nl, NlSweep* w, const RecPool& pool, const LmView& lmz,
                   const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg,
                   SetSumArgs* a) {
-  if (w->use_nls) return nls_set_sums(ctx, kp, nl, &w->nlop, pool, lmz, lmobs, off, S, p_lo, p_hi, G, ldg);
+  if (w->use_nls) return nls_set_sums(ctx, kp, nl, &w->nlop, pool, lmz, lmobs, off, S, p_lo, p_hi, G, ldg, a->grid_m);
   // non-linear kernels need C_h(z_m, x_p) = k(z_m, x_p) - (K_ZX W) k(Xobs, x_p) per pair: build the
   // correction for a chunk of points with two GEMM-shaped steps, then accumulate.
   const int n_obs = lmobs.count;
   BASQ_CUDA(cudaMemsetAsync(G, 0, sizeof(double) * (size_t)lmz.count * ldg, ctx->stream));
+  if (a->G2) BASQ_CUDA(cudaMemsetAsync(a->G2, 0, sizeof(double) * (size_t)lmz.count * ldg, ctx->stream));
   for (int64_t c0 = p_lo; c0 < p_hi; c0 += w->chunkP) {
     const int64_t c1 = std::min(p_hi, c0 + w->chunkP);
     const int64_t cnt = c1 - c0;
     BASQ_TRY(base_gram_records(ctx, kp, lmobs, pool, c0, c1, w->V.as<double>(), w->chunkP));
-    // corrT[p, m] = sum_o V[o, p] * Az[m, o]
+    // corrT[p, m] = sum_o V[o, p] * Az[m, o]; in reproducible sessions a point's correction must not depend on
+    // the chunk it falls into (the chunk sizes depend on the shard), so the GEMM runs in a fixed summation order
     BASQ_TRY(dgemm(ctx, true, true, (int)cnt, w->M, n_obs, 1.0, w->V.as<double>(), w->chunkP, w->Az, n_obs, 0.0,
-                   w->corrT.as<double>(), w->M));
+                   w->corrT.as<double>(), w->M, false, false, false, false, a->grid_m != 0.0));
     a->p_lo = c0;
     a->p_hi = c1;
     a->corrT = w->corrT.as<double>();
@@ -383,6 +398,7 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
   s->rows = s->n;
   s->S = S_override > 0 ? S_override : 2 * (q + 1);
   s->idx_base = idx_base;
+  s->repro = ctx->reproducible;
   const int mode = desc->mode;
   const int n_obs = (mode == BASQ_PLAIN) ? 0 : desc->n_obs;
   const bool nonlin = (mode == BASQ_WSABI_M || mode == BASQ_MMLT_G);
@@ -421,6 +437,13 @@ int session_create_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void*
     BASQ_TRY(warp_factor(ctx, desc, s->kp, s->lmobs.view(), Z, M, s->sz.as<double>()));
     BASQ_TRY(sx.alloc(ctx, sizeof(double) * std::max<int64_t>(N_loc, 1)));
     BASQ_TRY(warp_factor(ctx, desc, s->kp, s->lmobs.view(), X, N_loc, sx.as<double>()));
+    if (s->repro && nonlin) {   // replicated landmark data: the same maximum on every rank
+      std::vector<double> h((size_t)M);
+      BASQ_CUDA(cudaMemcpyAsync(h.data(), s->sz.p, sizeof(double) * M, cudaMemcpyDeviceToHost, ctx->stream));
+      BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+      for (double v : h) s->szmax = std::max(s->szmax, fabs(v));
+      BASQ_CHECK(isfinite(s->szmax), BASQ_ERR_NUMERIC, "session: non-finite warp factor of a landmark");
+    }
   }
 
   // projection matrix U' [q, Mtot]
@@ -470,6 +493,14 @@ int session_reserve_cells(basq_session* s, int cells) {
   s->cellobj.release();
   BASQ_TRY(s->cellmass.alloc(ctx, sizeof(double) * (size_t)cells));
   BASQ_TRY(s->cellobj.alloc(ctx, sizeof(double) * (size_t)cells));
+  if (s->repro) {
+    s->G2.release();
+    s->cellmass2.release();
+    s->cellobj2.release();
+    if (s->pool.dtype == BASQ_F64) BASQ_TRY(s->G2.alloc(ctx, sizeof(double) * (size_t)s->Mtot * s->ldg));
+    BASQ_TRY(s->cellmass2.alloc(ctx, sizeof(double) * (size_t)cells));
+    BASQ_TRY(s->cellobj2.alloc(ctx, sizeof(double) * (size_t)cells));
+  }
   s->omega_host.resize(cells);
   s->rank_host.resize(cells);
   return BASQ_OK;
@@ -488,10 +519,14 @@ int session_pass_begin(basq_session* s, int64_t R_glob, int64_t off, int F) {
   BASQ_CHECK(off >= 0 && off + s->pool.count <= R_glob, BASQ_ERR_INVALID,
              "pass: offset %lld + local %lld exceeds global %lld", (long long)off, (long long)s->pool.count,
              (long long)R_glob);
+  BASQ_CHECK(!s->repro || s->grid_R == R_glob, BASQ_ERR_INVALID,
+             "pass: a reproducible session needs the grids of this pass first (basq_session_set_grid)");
   const int c_eff = (int)std::min<int64_t>(cells, R_glob);
   BASQ_TRY(session_reserve_cells(s, cells));
   if (!s->Gf.p) {
-    BASQ_TRY(s->Gf.alloc(ctx, sizeof(double) * (size_t)s->Mtot * s->S));
+    // reproducible sessions: hi and lo parts of the set sums, masses and objective sums (session_level_fold_exact)
+    BASQ_TRY(s->Gf.alloc(ctx, sizeof(double) * (size_t)(s->repro ? 2 * (s->Mtot + 2) : s->Mtot) * s->S));
+    if (s->repro) BASQ_TRY(s->Gc.alloc(ctx, sizeof(double) * (size_t)(s->Mtot + 2) * s->S));
     for (int i = 0; i < 2; ++i) BASQ_TRY(s->raw[i].alloc(ctx, sizeof(double) * (size_t)(s->n + 1) * s->S));
     BASQ_TRY(s->lnode.alloc(ctx, sizeof(int) * s->S));
     BASQ_TRY(s->lppos.alloc(ctx, sizeof(int) * s->S));
@@ -501,9 +536,14 @@ int session_pass_begin(basq_session* s, int64_t R_glob, int64_t off, int F) {
   s->pass_R = R_glob;
   s->pass_off = off;
   PhaseTimer t(ctx, PH_SETSUM);
-  BASQ_TRY(set_masses(ctx, s->pool, off, cells, c_eff, s->cellmass.as<double>()));
-  if (s->obj) BASQ_TRY(cell_objective(ctx, s->pool, off, cells, c_eff, s->obj, s->cellobj.as<double>()));
-  BASQ_TRY(session_set_sums(s, off, cells, 0, s->pool.count, s->G.as<double>(), s->ldg));
+  BASQ_TRY(set_masses(ctx, s->pool, off, cells, c_eff, s->cellmass.as<double>(), s->grid_m[1], s->grid_m2[1],
+                      s->cellmass2.as<double>()));
+  if (s->obj)
+    BASQ_TRY(cell_objective(ctx, s->pool, off, cells, c_eff, s->obj, s->cellobj.as<double>(), s->grid_m[2],
+                            s->grid_m2[2], s->cellobj2.as<double>()));
+  BASQ_TRY(session_set_sums(s, off, cells, 0, s->pool.count, s->G.as<double>(), s->ldg, s->grid_m[0], s->grid_m2[0],
+                            s->G2.as<double>()));
+  s->grid_R = -1;   // the grids belong to this pass
   return BASQ_OK;
 }
 
@@ -575,9 +615,11 @@ int session_level_fold(basq_session* s, int lvl, int K, const int* node_host, do
   return BASQ_OK;   // no synchronisation: node_host was copied into the pinned ring
 }
 
+// exact: Gf_rows holds all Mtot + 2 rows of session_level_fold_exact summed over the ranks; masses and
+// objective sums come from its last two rows instead of this rank's cells
 int session_level_project(basq_session* s, int lvl, int K, const int* node_host, const int* ppos_host,
                           const double* fpar_host, const double* Gf_rows, int64_t ld_gf, int row0, int nrows,
-                          double* A_out) {
+                          double* A_out, bool exact = false) {
   basq_ctx* ctx = s->ctx;
   const int n = s->n, S = s->S, F = s->pass_F, rows = s->rows;
   BASQ_TRY(session_level_check(s, lvl, K, node_host, ppos_host));
@@ -602,11 +644,19 @@ int session_level_project(basq_session* s, int lvl, int K, const int* node_host,
   BASQ_CUDA(cudaMemsetAsync(A_out, 0, sizeof(double) * (size_t)rows * S, ctx->stream));
   double* raw = s->raw[s->raw_cur].as<double>();
   const double* prev = s->raw[s->raw_cur ^ 1].as<double>();
-  fold_cols_kernel<<<(unsigned)ceil_div64(K, 256), 256, 0, ctx->stream>>>(s->cellmass.as<double>(), 0, 1, K,
-                                                                          s->lnode.as<int>(), stride, cnt, raw, S);
-  ctx->launches++;
-  BASQ_CUDA(cudaGetLastError());
-  if (s->obj) {  // objective row (SOBER/_rchq.py:138-146), folded like the masses
+  if (exact) {
+    BASQ_CUDA(cudaMemcpyAsync(raw, Gf_rows + (int64_t)s->Mtot * ld_gf, sizeof(double) * K, cudaMemcpyDeviceToDevice,
+                              ctx->stream));
+    if (s->obj)
+      BASQ_CUDA(cudaMemcpyAsync(raw + (int64_t)n * S, Gf_rows + (int64_t)(s->Mtot + 1) * ld_gf, sizeof(double) * K,
+                                cudaMemcpyDeviceToDevice, ctx->stream));
+  } else {
+    fold_cols_kernel<<<(unsigned)ceil_div64(K, 256), 256, 0, ctx->stream>>>(s->cellmass.as<double>(), 0, 1, K,
+                                                                            s->lnode.as<int>(), stride, cnt, raw, S);
+    ctx->launches++;
+    BASQ_CUDA(cudaGetLastError());
+  }
+  if (s->obj && !exact) {  // objective row (SOBER/_rchq.py:138-146), folded like the masses
     fold_cols_kernel<<<(unsigned)ceil_div64(K, 256), 256, 0, ctx->stream>>>(s->cellobj.as<double>(), 0, 1, K,
                                                                             s->lnode.as<int>(), stride, cnt,
                                                                             raw + (int64_t)n * S, S);
@@ -630,8 +680,71 @@ int session_level_project(basq_session* s, int lvl, int K, const int* node_host,
   return BASQ_OK;
 }
 
+// Reproducible sessions: the level's grid-exact columns of this rank, Gf_out[2 (Mtot + 2), K] (ld = ld_gf): rows
+// 0 .. Mtot-1 the folded set sums, row Mtot the masses, row Mtot + 1 the objective sums (0 without objective), on
+// the pass's grids; rows Mtot + 2 .. 2 Mtot + 3 the same for the remainders on the finer grids (0 where a sum has
+// one grid: set sums of fp32 records).  Every entry is a multiple of its grid and far from overflowing it, so the
+// fold, and any sum of these arrays over ranks in any order, is exact.
+int session_level_fold_exact(basq_session* s, int lvl, int K, const int* node_host, double* Gf_out, int64_t ld_gf) {
+  basq_ctx* ctx = s->ctx;
+  BASQ_CHECK(s->repro, BASQ_ERR_INVALID, "level_fold_exact: the session is not reproducible (basq_ctx_reproducible)");
+  BASQ_TRY(session_level_fold(s, lvl, K, node_host, Gf_out, ld_gf));   // also copies node_host to s->lnode
+  const int stride = s->S << lvl, cnt = s->pass_F >> lvl, Mtot = s->Mtot;
+  double* lo = Gf_out + (int64_t)(Mtot + 2) * ld_gf;
+  auto fold = [&](const DevBuf& src, int rows, int64_t ldsrc, double* dst) {
+    fold_cols_kernel<<<(unsigned)ceil_div64((int64_t)rows * K, 256), 256, 0, ctx->stream>>>(
+        src.as<double>(), ldsrc, rows, K, s->lnode.as<int>(), stride, cnt, dst, ld_gf);
+    ctx->launches++;
+  };
+  auto zero = [&](int rows, double* dst) {
+    return cudaMemset2DAsync(dst, sizeof(double) * ld_gf, 0, sizeof(double) * K, rows, ctx->stream);
+  };
+  fold(s->cellmass, 1, 0, Gf_out + (int64_t)Mtot * ld_gf);
+  fold(s->cellmass2, 1, 0, lo + (int64_t)Mtot * ld_gf);
+  if (s->obj) {
+    fold(s->cellobj, 1, 0, Gf_out + (int64_t)(Mtot + 1) * ld_gf);
+    fold(s->cellobj2, 1, 0, lo + (int64_t)(Mtot + 1) * ld_gf);
+  } else {
+    BASQ_CUDA(zero(1, Gf_out + (int64_t)(Mtot + 1) * ld_gf));
+    BASQ_CUDA(zero(1, lo + (int64_t)(Mtot + 1) * ld_gf));
+  }
+  if (s->G2.p) fold(s->G2, Mtot, s->ldg, lo);
+  else BASQ_CUDA(zero(Mtot, lo));
+  BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+// out[r, i] = hi[r, i] + lo[r, i]: the one rounding from the exact hi and lo sums to the columns that are projected
+__global__ void add_parts_kernel(const double* __restrict__ hi, const double* __restrict__ lo, int64_t ld, int rows,
+                                 int K, double* __restrict__ out, int64_t ldo) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (int64_t)rows * K) return;
+  const int r = (int)(t / K), i = (int)(t % K);
+  out[(int64_t)r * ldo + i] = __dadd_rn(hi[(int64_t)r * ld + i], lo[(int64_t)r * ld + i]);
+}
+
+// Reproducible sessions: the level system from the columns of session_level_fold_exact summed over every rank -
+// the whole projection on every rank, with the same function and shapes as a single-GPU session.
+int session_level_project_exact(basq_session* s, int lvl, int K, const int* node_host, const int* ppos_host,
+                                const double* fpar_host, const double* Gf, int64_t ld_gf, double* A_out) {
+  BASQ_CHECK(s->repro && s->Gc.p, BASQ_ERR_INVALID,
+             "level_project_exact: the session is not reproducible (basq_ctx_reproducible) or has no pass");
+  basq_ctx* ctx = s->ctx;
+  const int rows = s->Mtot + 2;
+  add_parts_kernel<<<(unsigned)ceil_div64((int64_t)rows * K, 256), 256, 0, ctx->stream>>>(
+      Gf, Gf + (int64_t)rows * ld_gf, ld_gf, rows, K, s->Gc.as<double>(), K);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  return session_level_project(s, lvl, K, node_host, ppos_host, fpar_host, s->Gc.as<double>(), K, 0, s->Mtot, A_out,
+                               true);
+}
+
 int session_level(basq_session* s, int lvl, int K, const int* node_host, const int* ppos_host,
                   const double* fpar_host, double* A_out) {
+  if (s->repro) {
+    BASQ_TRY(session_level_fold_exact(s, lvl, K, node_host, s->Gf.as<double>(), s->S));
+    return session_level_project_exact(s, lvl, K, node_host, ppos_host, fpar_host, s->Gf.as<double>(), s->S, A_out);
+  }
   const int cnt = s->pass_F >> lvl;
   bool identity = (cnt == 1 && lvl == 0);  // plain round: the sets ARE the cells, project G as it is
   for (int i = 0; identity && i < K; ++i) identity = node_host[i] == i;
@@ -836,6 +949,7 @@ int session_apply_impl(basq_session* s, int64_t R_glob, int64_t off, int F, cons
 // waste slots) plus (1 + L/2) projections of S columns, and replaces L + 1 rounds: pick the F with
 // the lowest cost per level.  One evaluation ~ 4.4 fp64-GEMM flop at the measured kernel rates.
 int choose_cell_factor(const basq_session* s, int64_t R_glob, int64_t R_loc_max) {
+  if (s->repro) R_loc_max = R_glob;   // the cells must not depend on how the points are split over ranks
   static const int forced = [] { const char* e = getenv("BASQ_CELL_FACTOR"); return e ? atoi(e) : 0; }();
   const int64_t S = s->S;
   auto fits = [&](int f) { return R_glob >= (int64_t)4 * f * S; };
@@ -863,6 +977,37 @@ int choose_cell_factor(const basq_session* s, int64_t R_glob, int64_t R_loc_max)
     if (F == 1 || cost < best_cost) { best = F; best_cost = cost; }
   }
   return best;
+}
+
+// Grids of a reproducible pass over R_glob live points from the maxima over every rank of |wf|, |mu| and |mu obj|
+// (record_maxima, max-reduced over the ranks: exact).  A bound B on the sum of |terms| of every set sum, mass and
+// objective sum gives Q = 2^(ceil(log2 B) - 51): every term is below 2^51 Q and every partial sum below 2^53 Q.
+//   linear modes: |wf_p k| <= |wf_p| sigma_f^2          (wf = mu, or mu m(x) for WSABI-L)
+//   WSABI-M:      |mu_p (sz C sx_p + C^2 / 2)| <= |mu_p| (max|sz| sigma_f^2 |sx_p| + sigma_f^4 / 2)   (|C| <= sigma_f^2)
+//   MMLT:         |mu_p sz sx_p expm1(C)| <= |mu_p| max|sz| |sx_p| max(expm1(sigma_f^2), 1)
+int session_set_grid(basq_session* s, int64_t R_glob, const double* mx) {
+  BASQ_CHECK(s->repro, BASQ_ERR_INVALID, "set_grid: the session is not reproducible (basq_ctx_reproducible)");
+  BASQ_CHECK(R_glob >= 1, BASQ_ERR_INVALID, "set_grid: R_glob must be positive");
+  const double os = s->kp.outputscale, R = (double)R_glob;
+  double B[3];
+  if (s->nl == NL_WSABIM) B[0] = R * mx[1] * (s->szmax * os * mx[0] + 0.5 * os * os);
+  else if (s->nl == NL_MMLT) B[0] = R * mx[1] * s->szmax * mx[0] * std::max(expm1(os), 1.0);
+  else B[0] = R * mx[0] * os;
+  B[1] = R * mx[1];
+  B[2] = R * mx[2];
+  // Second grids for the remainders term - hi (each below Q / 2, so their sum is below R Q / 2): the fp64 terms,
+  // masses and objective sums keep their fp64 accuracy, about 2^-103 R^2 B absolute.
+  for (int i = 0; i < 3; ++i) {
+    BASQ_CHECK(isfinite(B[i]) && B[i] < 0x1p1000, BASQ_ERR_NUMERIC, "set_grid: weights or factors out of range");
+    grid_pair(B[i], R, &s->grid_m[i], &s->grid_m2[i]);
+  }
+  s->grid_R = R_glob;
+  return BASQ_OK;
+}
+
+int session_grid_local(basq_session* s, double* max_host) {
+  BASQ_CHECK(s->repro, BASQ_ERR_INVALID, "grid_maxima: the session is not reproducible (basq_ctx_reproducible)");
+  return record_maxima(s->ctx, s->pool, s->obj, max_host);
 }
 
 // Phi[p_lo..p_hi, q] for the session's live records
@@ -904,6 +1049,11 @@ int recombine_impl(basq_ctx* ctx, const basq_kernel_desc* desc, const void* X, i
     BASQ_CHECK(++rounds <= 256, BASQ_ERR_NUMERIC, "recombine: no convergence after 256 passes");
     const int F = choose_cell_factor(s.get(), R, R);
     factor.resize((size_t)F * S);
+    if (s->repro) {
+      double mx[3];
+      BASQ_TRY(session_grid_local(s.get(), mx));
+      BASQ_TRY(session_set_grid(s.get(), R, mx));
+    }
     BASQ_TRY(session_pass_begin(s.get(), R, 0, F));
     trace_point(ctx, "  pass: set sums");
     BASQ_TRY(session_pass_levels(s.get(), A.as<double>(), omega.as<double>(), factor.data()));
@@ -1022,6 +1172,12 @@ int basq_ctx_allow_f32_eval(basq_ctx* ctx, int on, int64_t* demotions_host) {
   BASQ_CHECK(ctx, BASQ_ERR_INVALID, "basq_ctx_allow_f32_eval: NULL context");
   if (on >= 0) ctx->eval_f32 = on != 0;
   if (demotions_host) *demotions_host = ctx->demotions;
+  return BASQ_OK;
+}
+
+int basq_ctx_reproducible(basq_ctx* ctx, int on) {
+  BASQ_CHECK(ctx, BASQ_ERR_INVALID, "basq_ctx_reproducible: NULL context");
+  if (on >= 0) ctx->reproducible = on != 0;
   return BASQ_OK;
 }
 
@@ -1552,6 +1708,38 @@ int basq_session_level(basq_session* s, int lvl, int K, const int* node_host, co
   BASQ_CHECK(s && node_host && fpar_host && A_out && (lvl == 0 || ppos_host), BASQ_ERR_INVALID, "NULL argument");
   BASQ_CUDA(cudaSetDevice(s->ctx->device));
   return session_level(s, lvl, K, node_host, ppos_host, fpar_host, A_out);
+}
+
+int basq_session_reproducible(const basq_session* s, int* on_host) {
+  BASQ_CHECK(s && on_host, BASQ_ERR_INVALID, "NULL argument");
+  *on_host = s->repro ? 1 : 0;
+  return BASQ_OK;
+}
+
+int basq_session_grid_maxima(basq_session* s, double* max_host) {
+  BASQ_CHECK(s && max_host, BASQ_ERR_INVALID, "NULL argument");
+  BASQ_CUDA(cudaSetDevice(s->ctx->device));
+  return session_grid_local(s, max_host);
+}
+
+int basq_session_set_grid(basq_session* s, int64_t R_glob, const double* max_host) {
+  BASQ_CHECK(s && max_host, BASQ_ERR_INVALID, "NULL argument");
+  return session_set_grid(s, R_glob, max_host);
+}
+
+int basq_session_level_fold_exact(basq_session* s, int lvl, int K, const int* node_host, double* Gf_out,
+                                  int64_t ld_gf) {
+  BASQ_CHECK(s && node_host && Gf_out && ld_gf >= K, BASQ_ERR_INVALID, "basq_session_level_fold_exact: bad argument");
+  BASQ_CUDA(cudaSetDevice(s->ctx->device));
+  return session_level_fold_exact(s, lvl, K, node_host, Gf_out, ld_gf);
+}
+
+int basq_session_level_project_exact(basq_session* s, int lvl, int K, const int* node_host, const int* ppos_host,
+                                     const double* fpar_host, const double* Gf, int64_t ld_gf, double* A_out) {
+  BASQ_CHECK(s && node_host && fpar_host && A_out && Gf && (lvl == 0 || ppos_host) && ld_gf >= K, BASQ_ERR_INVALID,
+             "basq_session_level_project_exact: bad argument");
+  BASQ_CUDA(cudaSetDevice(s->ctx->device));
+  return session_level_project_exact(s, lvl, K, node_host, ppos_host, fpar_host, Gf, ld_gf, A_out);
 }
 
 int basq_session_apply(basq_session* s, int64_t R_glob, int64_t off_glob, const double* omega,

@@ -187,6 +187,92 @@ __global__ void scale_or_fill_kernel(double* __restrict__ w, int64_t N, const do
   w[i] = (t != 0.0 && isfinite(t)) ? w[i] / t : 1.0 / (double)N;
 }
 
+// ---- reproducible weight totals (basq_ctx_reproducible) ----
+// max |w| (a NaN wins: its canonical bit pattern exceeds every non-negative double's); out must be zeroed
+__global__ void abs_max_kernel(const double* __restrict__ w, int64_t N, unsigned long long* __restrict__ out) {
+  double m = 0.0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
+    const double v = fabs(w[i]);
+    if (!(v <= m) && m == m) m = v;
+  }
+  if (m != m) m = __longlong_as_double(0x7ff8000000000000ll);
+  for (int o = 16; o > 0; o >>= 1) {
+    const double u = __shfl_down_sync(0xffffffffu, m, o);
+    if (__double_as_longlong(u) > __double_as_longlong(m)) m = u;
+  }
+  if ((threadIdx.x & 31) == 0) atomicMax(out, (unsigned long long)__double_as_longlong(m));
+}
+// hilo[0] += sum of w rounded to the grid of gm, hilo[1] += sum of the remainders on the grid of gm2: both exact,
+// so the order of the atomic additions does not matter
+__global__ void grid_sum_kernel(const double* __restrict__ w, int64_t N, double gm, double gm2, double* __restrict__ hilo) {
+  double s = 0.0, s2 = 0.0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
+    const double hi = grid_round(w[i], 1.0, gm);
+    s += hi;
+    s2 += grid_round(w[i] - hi, 1.0, gm2);
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    s += __shfl_down_sync(0xffffffffu, s, o);
+    s2 += __shfl_down_sync(0xffffffffu, s2, o);
+  }
+  if ((threadIdx.x & 31) == 0) {
+    atomicAdd(hilo, s);
+    atomicAdd(hilo + 1, s2);
+  }
+}
+__global__ void add_two_kernel(const double* __restrict__ hilo, double* __restrict__ total) { *total = hilo[0] + hilo[1]; }
+
+int weights_abs_max(basq_ctx* ctx, const double* w, int64_t N, double* max_host) {
+  *max_host = 0.0;
+  if (N == 0) return BASQ_OK;
+  DevBuf d;
+  BASQ_TRY(d.alloc(ctx, sizeof(double)));
+  BASQ_CUDA(cudaMemsetAsync(d.p, 0, sizeof(double), ctx->stream));
+  abs_max_kernel<<<(unsigned)std::min<int64_t>(ceil_div64(N, 256), 4 * (int64_t)ctx->num_sms), 256, 0, ctx->stream>>>(
+      w, N, d.as<unsigned long long>());
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  BASQ_CUDA(cudaMemcpyAsync(max_host, d.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  return BASQ_OK;
+}
+
+// hilo_dev[2] = the exact hi / lo sums of w[N] on the grids of N_glob weights of magnitude <= wmax (the maximum over
+// every rank).  A non-finite or huge wmax makes both parts wmax: the total is not finite, as a plain sum's would be.
+int weights_grid_sum(basq_ctx* ctx, const double* w, int64_t N, double wmax, int64_t N_glob, double* hilo_dev) {
+  const double B = wmax * (double)N_glob;
+  if (!(isfinite(B) && B < 0x1p1000)) {
+    const double h[2] = {wmax == wmax ? INFINITY : wmax, 0.0};
+    BASQ_CUDA(cudaMemcpyAsync(hilo_dev, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
+    BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+    return BASQ_OK;
+  }
+  double gm, gm2;
+  grid_pair(B, (double)N_glob, &gm, &gm2);
+  BASQ_CUDA(cudaMemsetAsync(hilo_dev, 0, 2 * sizeof(double), ctx->stream));
+  if (N > 0) {
+    grid_sum_kernel<<<(unsigned)std::min<int64_t>(ceil_div64(N, 256), 4 * (int64_t)ctx->num_sms), 256, 0, ctx->stream>>>(
+        w, N, gm, gm2, hilo_dev);
+    ctx->launches++;
+    BASQ_CUDA(cudaGetLastError());
+  }
+  return BASQ_OK;
+}
+
+// total_dev = the reproducible total of w[N] on one GPU: hi + lo of weights_grid_sum with the maximum of w itself
+int weights_total_repro(basq_ctx* ctx, const double* w, int64_t N, double* total_dev) {
+  double wmax = 0.0;
+  BASQ_TRY(weights_abs_max(ctx, w, N, &wmax));
+  DevBuf hilo;
+  BASQ_TRY(hilo.alloc(ctx, 2 * sizeof(double)));
+  BASQ_TRY(weights_grid_sum(ctx, w, N, wmax, N, hilo.as<double>()));
+  add_two_kernel<<<1, 1, 0, ctx->stream>>>(hilo.as<double>(), total_dev);
+  ctx->launches++;
+  BASQ_CUDA(cudaGetLastError());
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));   // hilo goes out of scope
+  return BASQ_OK;
+}
+
 // Sequential importance resampling without replacement (torch.multinomial(weights, n), as
 // UncertaintySampler.SIR, BASQ/_sampler.py:104-118) as an exponential race (Efraimidis-Spirakis):
 // key_i = -log(u_i) / w_i with u_i uniform; the n smallest keys, in increasing order, are distributed
@@ -523,7 +609,8 @@ int basq_candidate_weights(basq_ctx* ctx, int kind, double ratio, int log_out, c
   if (normalise) {
     DevBuf total;
     BASQ_TRY(total.alloc(ctx, sizeof(double)));
-    BASQ_TRY(sum_device(ctx, w_out, N, total.as<double>()));
+    if (ctx->reproducible) BASQ_TRY(weights_total_repro(ctx, w_out, N, total.as<double>()));
+    else BASQ_TRY(sum_device(ctx, w_out, N, total.as<double>()));
     scale_or_fill_kernel<<<blocks, 256, 0, ctx->stream>>>(w_out, N, total.as<double>());
     ctx->launches++;
     BASQ_CUDA(cudaGetLastError());
@@ -593,7 +680,8 @@ int basq_cleanse_weights(basq_ctx* ctx, double* w, int64_t N, double eps) {
   ctx->launches++;
   DevBuf total;
   BASQ_TRY(total.alloc(ctx, sizeof(double)));
-  BASQ_TRY(sum_device(ctx, w, N, total.as<double>()));
+  if (ctx->reproducible) BASQ_TRY(weights_total_repro(ctx, w, N, total.as<double>()));
+  else BASQ_TRY(sum_device(ctx, w, N, total.as<double>()));
   scale_or_fill_kernel<<<blocks, 256, 0, ctx->stream>>>(w, N, total.as<double>());
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
@@ -611,6 +699,24 @@ int basq_weights_sum(basq_ctx* ctx, const double* w, int64_t N, double* total_ho
   BASQ_TRY(total.alloc(ctx, sizeof(double)));
   BASQ_TRY(sum_device(ctx, w, N, total.as<double>()));
   BASQ_CUDA(cudaMemcpyAsync(total_host, total.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
+  return BASQ_OK;
+}
+
+int basq_weights_max(basq_ctx* ctx, const double* w, int64_t N, double* max_host) {
+  BASQ_CHECK(ctx && (w || N == 0) && max_host && N >= 0, BASQ_ERR_INVALID, "basq_weights_max: bad argument");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  return weights_abs_max(ctx, w, N, max_host);
+}
+
+int basq_weights_sum_grid(basq_ctx* ctx, const double* w, int64_t N, double wmax, int64_t N_glob, double* hilo_host) {
+  BASQ_CHECK(ctx && (w || N == 0) && hilo_host && N >= 0 && N_glob >= N && N_glob >= 1, BASQ_ERR_INVALID,
+             "basq_weights_sum_grid: bad argument");
+  BASQ_CUDA(cudaSetDevice(ctx->device));
+  DevBuf hilo;
+  BASQ_TRY(hilo.alloc(ctx, 2 * sizeof(double)));
+  BASQ_TRY(weights_grid_sum(ctx, w, N, wmax, N_glob, hilo.as<double>()));
+  BASQ_CUDA(cudaMemcpyAsync(hilo_host, hilo.p, 2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
   return BASQ_OK;
 }

@@ -149,6 +149,7 @@ struct basq_ctx {
   double* staged_mu = nullptr;
   cudaEvent_t side_ev[2] = {nullptr, nullptr};
   bool eval_f32 = false;           // basq_ctx_allow_f32_eval: fp64 inputs may be evaluated on the fp32 tensor-core path
+  bool reproducible = false;       // basq_ctx_reproducible: sessions sum on a grid, the same bits for any split over ranks
   int64_t demotions = 0;
   uint64_t seed = 0;               // basq_ctx_set_seed: key of the library's own Gaussian draws (Nystrom test matrix)
   uint64_t draws = 0;              // test matrices drawn since the seed was set (each call uses key seed + draws)
@@ -330,6 +331,25 @@ __device__ __forceinline__ double f2d_pos(float k) {
   return __hiloint2double((int)((u >> 3) + 0x38000000u), (int)(u << 29));
 }
 
+// Reproducible mode, host side: the grids of sums of at most R terms whose |sum| is bounded by B.  gm = 1.5 * 2^52 Q
+// with Q = 2^(ceil(log2 B) - 51) (every term below 2^51 Q, every partial sum below 2^53 Q); gm2 the grid of the
+// remainders term - hi, each below Q / 2, so their sum is below R Q / 2.  B must be finite and below 2^1000.
+inline void grid_pair(double B, double R, double* gm, double* gm2) {
+  int e = -1000;
+  if (B > 0.0) frexp(B, &e);                 // B <= 2^e
+  e = e < -800 ? -800 : e;
+  *gm = ldexp(1.5, e - 51 + 52);
+  int e2 = 0;
+  frexp(R * ldexp(0.5, e - 51), &e2);        // R Q / 2 <= 2^e2
+  *gm2 = ldexp(1.5, e2 - 51 + 52);
+}
+
+// Reproducible mode: the term a * b rounded to the grid Q of gm = 1.5 * 2^52 * Q (exact for |a b| < 2^51 Q: gm + a b
+// then lies in [2^52 Q, 2^53 Q), where the spacing of doubles is Q).  Sums of such terms are multiples of Q and
+// exact while they stay below 2^53 Q, so they do not depend on the order of the additions, on the tiling or on
+// how the terms are split over ranks and all-reduced.
+__device__ __forceinline__ double grid_round(double a, double b, double gm) { return __dsub_rn(__fma_rn(a, b, gm), gm); }
+
 // One kernel evaluation in fp32 from prepared operands.  Every fp32 kernel in the library goes
 // through the same operation sequence (acc = a + b; acc = fma(x_i, zz_i, acc) for i ascending;
 // finish_f32) with the same operand roles, so k(z, x) is bit-identical wherever it is recomputed
@@ -478,9 +498,14 @@ struct RecPool {
 int build_records(basq_ctx* ctx, const KParams& kp, int dtype, const void* X, int64_t N, double uniform_w,
                   const double* mu, const double* factor, bool factor_in_weight, RecPool* pool,
                   bool round_buffer = true);
-int set_masses(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, double* mass_out);
+// grid_m != 0: reproducible sums, every term rounded to the grid of grid_m (grid_round)
+// (masses and objective terms are fp64: the remainders of the terms go to the grid of grid_m2, summed into *_out2)
+int set_masses(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, double* mass_out,
+               double grid_m = 0.0, double grid_m2 = 0.0, double* mass_out2 = nullptr);
 int cell_objective(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, const double* obj,
-                   double* out);
+                   double* out, double grid_m = 0.0, double grid_m2 = 0.0, double* out2 = nullptr);
+// max_host[3] = maxima over the live records of |wf|, |mu| and |mu obj[idx]| (obj may be NULL); synchronises
+int record_maxima(basq_ctx* ctx, const RecPool& pool, const double* obj, double* max_host);
 int apply_round(basq_ctx* ctx, RecPool* pool, int64_t off_glob, int S, const double* omega, const int* rank_excl,
                 int K, bool scale_wf, int64_t dest_base, int64_t new_count);
 int extract_result(basq_ctx* ctx, const RecPool& pool, int64_t idx_base, int64_t* idx_out, double* w_out);
@@ -499,6 +524,9 @@ struct SetSumArgs {
   double* G;            // [lm->count, ldg]
   int64_t ldg;
   bool accumulate;
+  double grid_m = 0.0;  // != 0: reproducible instances, terms rounded to the grid of 1.5 * 2^52 * Q (grid_round)
+  double grid_m2 = 0.0; // fp64 records in reproducible instances: grid of the remainders term - hi, summed into G2
+  double* G2 = nullptr; // [lm->count, ldg]
 };
 int set_sums(basq_ctx* ctx, const KParams& kp, const SetSumArgs& a);
 
@@ -513,7 +541,8 @@ struct NlOperands {
 int nls_prepare(basq_ctx* ctx, const KParams& kp, const double* Az, int M, int n_obs, const double* sz,
                 NlOperands* op);
 int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const RecPool& pool, const LmView& lmz,
-                 const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg);
+                 const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg,
+                 double grid_m = 0.0);
 
 // gpvar.cu: fused posterior variance on the tensor cores (fp32 inputs)
 // mean_out != NULL: the fused kernel also writes the posterior mean (*mean_done tells whether it did)
@@ -526,7 +555,8 @@ int gp_variance_tc(basq_ctx* ctx, const basq_kernel_desc* desc, const KParams& k
 // dgemm.cu
 int dgemm(basq_ctx* ctx, bool ta, bool tb, int m, int n, int k, double alpha, const double* A, int64_t lda,
           const double* B, int64_t ldb, double beta, double* C, int64_t ldc, bool b_lower_tri = false,
-          bool a_lower_tri = false, bool c_symmetric = false, bool c_lower_only = false);
+          bool a_lower_tri = false, bool c_symmetric = false, bool c_lower_only = false, bool fixed_order = false);
+// fixed_order: one tile shape, no split-K - an element's k-sum does not depend on m or n (reproducible sessions)
 // b_lower_tri (with tb): B is lower triangular, C = A B^T only visits k <= column
 // a_lower_tri (without ta): A is lower triangular, C = A B only visits k <= row
 // c_symmetric (m == n, beta == 0; e.g. A^T A): only the tiles that touch the lower triangle are computed, the

@@ -203,7 +203,7 @@ __global__ void mirror_lower_kernel(double* __restrict__ C, int N, int64_t ldc) 
 
 template <bool TA, bool TB, int WM, int WN, int MF, int NF>
 int launch_pipe(basq_ctx* ctx, int m, int n, int k, double alpha, const double* A, int64_t lda, const double* B,
-                int64_t ldb, double beta, double* C, int64_t ldc, int tri_k, int sym) {
+                int64_t ldb, double beta, double* C, int64_t ldc, int tri_k, int sym, bool fixed_order = false) {
   constexpr int BM = WM * 8 * MF, BNN = WN * 8 * NF;
   constexpr int A_EL = TA ? PK * (BM + 4) : BM * (PK + 4);
   constexpr int B_EL = TB ? BNN * (PK + 4) : PK * (BNN + 4);
@@ -220,7 +220,7 @@ int launch_pipe(basq_ctx* ctx, int m, int n, int k, double alpha, const double* 
     for (unsigned by = 0; by < grid.y; ++by) tiles += std::min<int64_t>(grid.x, ceil_div64((int64_t)(by + 1) * BM, BNN));
   }
   int splits = 1;
-  if (sym != 2 && tri_k == 0 && tiles * 2 <= ctx->num_sms && k >= 16 * PK)
+  if (!fixed_order && sym != 2 && tri_k == 0 && tiles * 2 <= ctx->num_sms && k >= 16 * PK)
     splits = (int)std::min<int64_t>(ctx->num_sms / tiles, k / (8 * PK));
   if (splits <= 1) {
     kern<<<grid, WM * WN * 32, SMEM, ctx->stream>>>(m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, a16, b16, 0,
@@ -247,7 +247,11 @@ int launch_pipe(basq_ctx* ctx, int m, int n, int k, double alpha, const double* 
 // tile shape that needs the fewest SM-waves of work for an m x n output
 template <bool TA, bool TB>
 int launch_best(basq_ctx* ctx, int m, int n, int k, double alpha, const double* A, int64_t lda, const double* B,
-                int64_t ldb, double beta, double* C, int64_t ldc, int tri_k, int sym) {
+                int64_t ldb, double beta, double* C, int64_t ldc, int tri_k, int sym, bool fixed_order) {
+  // fixed_order: one tile shape and no split-K, so that every output element sums its k terms in the same order
+  // whatever m and n are
+  if (fixed_order)
+    return launch_pipe<TA, TB, 2, 4, 8, 4>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym, true);
   auto cost = [&](int bm, int bn) {
     const int64_t tiles = (int64_t)ceil_div(m, bm) * ceil_div(n, bn);
     return (double)ceil_div64(tiles, ctx->num_sms) * bm * bn;
@@ -264,7 +268,7 @@ int launch_best(basq_ctx* ctx, int m, int n, int k, double alpha, const double* 
 
 int dgemm(basq_ctx* ctx, bool ta, bool tb, int m, int n, int k, double alpha, const double* A, int64_t lda,
           const double* B, int64_t ldb, double beta, double* C, int64_t ldc, bool b_lower_tri, bool a_lower_tri,
-          bool c_symmetric, bool c_lower_only) {
+          bool c_symmetric, bool c_lower_only, bool fixed_order) {
   BASQ_CHECK(!c_symmetric || (m == n && beta == 0.0 && !b_lower_tri && !a_lower_tri), BASQ_ERR_INVALID,
              "dgemm: c_symmetric needs a square output, beta = 0 and dense operands");
   BASQ_CHECK(!c_lower_only || (m == n && !c_symmetric && !b_lower_tri && !a_lower_tri), BASQ_ERR_INVALID,
@@ -277,10 +281,10 @@ int dgemm(basq_ctx* ctx, bool ta, bool tb, int m, int n, int k, double alpha, co
   if (m <= 0 || n <= 0) return BASQ_OK;
   BASQ_CHECK(k >= 0, BASQ_ERR_INVALID, "dgemm: negative k");
   BASQ_CHECK(ceil_div(m, 64) <= 65535, BASQ_ERR_UNSUPPORTED, "dgemm: m=%d too large for one launch", m);
-  if (!ta && !tb) BASQ_TRY((launch_best<false, false>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym)));
-  else if (ta && !tb) BASQ_TRY((launch_best<true, false>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym)));
-  else if (!ta && tb) BASQ_TRY((launch_best<false, true>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym)));
-  else BASQ_TRY((launch_best<true, true>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym)));
+  if (!ta && !tb) BASQ_TRY((launch_best<false, false>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym, fixed_order)));
+  else if (ta && !tb) BASQ_TRY((launch_best<true, false>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym, fixed_order)));
+  else if (!ta && tb) BASQ_TRY((launch_best<false, true>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym, fixed_order)));
+  else BASQ_TRY((launch_best<true, true>(ctx, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, tri_k, sym, fixed_order)));
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
   return BASQ_OK;

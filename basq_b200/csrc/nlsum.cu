@@ -64,7 +64,8 @@ int nls_prepare(basq_ctx* ctx, const KParams& kp, const double* Az, int M, int n
 
 // G[:, 0..S) = set sums of local records [p_lo, p_hi), set of a record = (off + p) mod S.
 int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const RecPool& pool, const LmView& lmz,
-                 const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg) {
+                 const LmView& lmobs, int64_t off, int S, int64_t p_lo, int64_t p_hi, double* G, int64_t ldg,
+                 double grid_m) {
   BASQ_CHECK(pool.dtype == BASQ_F32 && lmz.dtype == BASQ_F32, BASQ_ERR_INVALID, "nlsum: fp32 records only");
   BASQ_CHECK(lmz.count == op->M && lmobs.count == op->n_obs, BASQ_ERR_INVALID, "nlsum: operand mismatch");
   BASQ_CHECK(p_lo >= 0 && p_hi <= pool.count && p_lo <= p_hi && S >= 1, BASQ_ERR_INVALID, "nlsum: bad range");
@@ -73,8 +74,9 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
     return BASQ_OK;
   }
   ctx->pair_evals += (int64_t)op->M * (p_hi - p_lo);
-  // every cell has at most one member of the range: one column per cell (GRAM); else 8 sets x 32 members
-  const bool gram = (p_hi - p_lo) <= (int64_t)S;
+  // every cell has at most one member of the range: one column per cell (GRAM); else 8 sets x 32 members.
+  // Reproducible sums round every term to the grid, which only the set-sum mode does.
+  const bool gram = grid_m == 0.0 && (p_hi - p_lo) <= (int64_t)S;
   const int JT = gram ? NLS_NT : NLS_JT, EC = NLS_NT / JT;
   const int n_jg_total = ceil_div(S, JT);
   // tile stride: an upper bound of any group's tile count.  The kernels start group g at
@@ -122,7 +124,7 @@ int nls_set_sums(basq_ctx* ctx, const KParams& kp, int nl, NlOperands* op, const
     d.kxh = kx.kxh; d.kxl = kx.kxl; d.trec = kx.trec; d.KP = op->KP;
     d.zz = reinterpret_cast<const float*>(lmz.zz); d.bz = lmz.b; d.szf = op->szf.as<float>();
     d.M = op->M; d.n_mtiles = op->n_mtiles; d.os_f = kp.os_f;
-    d.G = G; d.ldg = ldg;
+    d.G = G; d.ldg = ldg; d.grid_m = grid_m;
     BASQ_TRY(launch_nlsum(ctx, kp.family, nl, kp.dp, d, gram ? 1 : 0));
   }
   return BASQ_OK;

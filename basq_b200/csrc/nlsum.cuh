@@ -76,6 +76,7 @@ struct NlsDev {
   float os_f;
   double* G;
   int64_t ldg;
+  double grid_m;  // reproducible instances: 1.5 * 2^52 * Q of the pass's grid Q (grid_round, common.cuh)
 };
 
 template <int DP>
@@ -142,7 +143,7 @@ __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64
 // Epilogue of one 128 x 256 tile for one thread (TMEM lane = landmark row m, column half `half`):
 // correction from TMEM, k(z_m, x_p) with the library's operation sequence, C, the non-linearity, fp64
 // accumulation per set (MODE 0) or one store per column (MODE 1).
-template <int FAM, int DP, int NL, int MODE>
+template <int FAM, int DP, int NL, int MODE, bool REPRO>
 __device__ __forceinline__ void nls_epilogue_tile(const NlsDev& a, const unsigned char* recs, uint32_t taddr, int half,
                                                   const float (&zr)[DP], float bm, float szm, float ainv,
                                                   double (&acc)[NLS_JT], int m, bool mok, int j0) {
@@ -169,7 +170,8 @@ __device__ __forceinline__ void nls_epilogue_tile(const NlsDev& a, const unsigne
       const float cv = __fsub_rn(k, __fmul_rn(__uint_as_float(v[c]), ainv));
       float val = nl_apply_f32<NL>(cv, __fmul_rn(szm, (float)hw.x));
       val = (hw.y != 0.0) ? val : 0.f;
-      if (MODE == 0) acc[c % NLS_JT] = fma(f2d_signed(val), hw.y, acc[c % NLS_JT]);
+      if (MODE == 0 && REPRO) acc[c % NLS_JT] += grid_round(f2d_signed(val), hw.y, a.grid_m);
+      else if (MODE == 0) acc[c % NLS_JT] = fma(f2d_signed(val), hw.y, acc[c % NLS_JT]);
       else out[c] = f2d_signed(val) * hw.y;
     }
     if (MODE == 1 && mok) {
@@ -185,7 +187,8 @@ __device__ __forceinline__ void nls_epilogue_tile(const NlsDev& a, const unsigne
 }
 
 // MODE 0: SETSUM (accumulate per set, write once per work item) ; MODE 1: GRAM (one column = one cell)
-template <int FAM, int DP, int NL, int MODE>
+// REPRO (MODE 0): every term is rounded to the pass's grid before it is added (see setsum_mma.cuh)
+template <int FAM, int DP, int NL, int MODE, bool REPRO>
 __global__ void __launch_bounds__(NLS_THREADS, 1) nlsum_kernel(const NlsDev a) {
   using Cfg = NlsCfg<DP>;
   constexpr int NSTAGE = Cfg::NSTAGE, NT = NLS_NT;
@@ -254,7 +257,7 @@ __global__ void __launch_bounds__(NLS_THREADS, 1) nlsum_kernel(const NlsDev a) {
         mma::mbar_wait(&t_full[buf], ph);
         mma::tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + buf * NT + half * (NT / 2);
-        nls_epilogue_tile<FAM, DP, NL, MODE>(a, sRec, taddr, half, zr, bm, szm, ainv, acc, m, mok, j0);
+        nls_epilogue_tile<FAM, DP, NL, MODE, REPRO>(a, sRec, taddr, half, zr, bm, szm, ainv, acc, m, mok, j0);
         mma::tc_fence_before();
         __syncwarp();
         if (lane == 0) {
@@ -553,12 +556,15 @@ int launch_nlsum_dp(basq_ctx* ctx, const NlsDev& dev, int mode) {
   const int64_t n_items = (int64_t)dev.n_mtiles * dev.n_jg;
   const int grid = (int)std::min<int64_t>(ctx->num_sms, n_items);
   if (grid <= 0) return BASQ_OK;
-  if (mode == 0) {
-    BASQ_CUDA(cudaFuncSetAttribute(nlsum_kernel<FAM, DP, NL, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    nlsum_kernel<FAM, DP, NL, 0><<<grid, NLS_THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+  if (mode == 0 && dev.grid_m != 0.0) {
+    BASQ_CUDA(cudaFuncSetAttribute(nlsum_kernel<FAM, DP, NL, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    nlsum_kernel<FAM, DP, NL, 0, true><<<grid, NLS_THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+  } else if (mode == 0) {
+    BASQ_CUDA(cudaFuncSetAttribute(nlsum_kernel<FAM, DP, NL, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    nlsum_kernel<FAM, DP, NL, 0, false><<<grid, NLS_THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
   } else {
-    BASQ_CUDA(cudaFuncSetAttribute(nlsum_kernel<FAM, DP, NL, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    nlsum_kernel<FAM, DP, NL, 1><<<grid, NLS_THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+    BASQ_CUDA(cudaFuncSetAttribute(nlsum_kernel<FAM, DP, NL, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    nlsum_kernel<FAM, DP, NL, 1, false><<<grid, NLS_THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
   }
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());

@@ -166,27 +166,49 @@ int build_records(basq_ctx* ctx, const KParams& kp, int dtype, const void* X, in
 // ---------------------------------------------------------------------------------------------
 // set masses: mass[j] = sum of mu over local points whose global position = j (mod S)
 // ---------------------------------------------------------------------------------------------
+// REPRO: every mass is rounded to the grid of gm before it is added (grid_round, common.cuh), its remainder to the
+// finer grid of gm2 and summed into mass2
+template <bool REPRO>
 __global__ void set_mass_kernel(const unsigned char* __restrict__ recs, int rec_bytes, int64_t count, int64_t off,
-                                int S, int S_eff, double* __restrict__ mass) {
+                                int S, int S_eff, double* __restrict__ mass, double gm, double gm2,
+                                double* __restrict__ mass2) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= S) return;
-  double s = 0.0;
+  double s = 0.0, s2 = 0.0;
   if (warp < S_eff) {
     int64_t p0 = ((int64_t)warp - off) % S;
     if (p0 < 0) p0 += S;
-    for (int64_t p = p0 + (int64_t)lane * S; p < count; p += (int64_t)32 * S)
-      s += reinterpret_cast<const double*>(recs + p * rec_bytes)[1];
+    for (int64_t p = p0 + (int64_t)lane * S; p < count; p += (int64_t)32 * S) {
+      const double m = reinterpret_cast<const double*>(recs + p * rec_bytes)[1];
+      if (REPRO) {
+        const double hi = grid_round(m, 1.0, gm);
+        s += hi;
+        s2 += grid_round(m - hi, 1.0, gm2);
+      } else {
+        s += m;
+      }
+    }
   }
   for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+  if (REPRO)
+    for (int o = 16; o > 0; o >>= 1) s2 += __shfl_down_sync(0xffffffffu, s2, o);
   if (lane == 0) mass[warp] = s;
+  if (REPRO && lane == 0) mass2[warp] = s2;
 }
 
-int set_masses(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, double* mass_out) {
+int set_masses(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, double* mass_out, double grid_m,
+               double grid_m2, double* mass_out2) {
   const int threads = 256;
   const int blocks = ceil_div((int64_t)S * 32, threads);
-  set_mass_kernel<<<blocks, threads, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
-                                                       pool.count, off_glob, S, S_eff, mass_out);
+  if (grid_m != 0.0)
+    set_mass_kernel<true><<<blocks, threads, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
+                                                               pool.count, off_glob, S, S_eff, mass_out, grid_m,
+                                                               grid_m2, mass_out2);
+  else
+    set_mass_kernel<false><<<blocks, threads, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
+                                                                pool.count, off_glob, S, S_eff, mass_out, 0.0, 0.0,
+                                                                nullptr);
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
   return BASQ_OK;
@@ -195,35 +217,96 @@ int set_masses(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int 
 // cell objective sums: out[j] = sum of mu_p * obj[idx_p] over local points in cell j (the extra row
 // of the objective-aware recombination, SOBER/_rchq.py:138-146); obj is indexed by the candidate's
 // original local row, which every record carries
+template <bool REPRO>
 __global__ void cell_obj_kernel(const unsigned char* __restrict__ recs, int rec_bytes, int f64, int64_t count,
                                 int64_t off, int S, int S_eff, const double* __restrict__ obj,
-                                double* __restrict__ out) {
+                                double* __restrict__ out, double gm, double gm2, double* __restrict__ out2) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= S) return;
-  double s = 0.0;
+  double s = 0.0, s2 = 0.0;
   if (warp < S_eff) {
     int64_t p0 = ((int64_t)warp - off) % S;
     if (p0 < 0) p0 += S;
     for (int64_t p = p0 + (int64_t)lane * S; p < count; p += (int64_t)32 * S) {
       const unsigned char* rec = recs + p * rec_bytes;
       const int64_t idx = f64 ? reinterpret_cast<const int64_t*>(rec)[2] : (int64_t) reinterpret_cast<const int*>(rec)[4];
-      s = fma(reinterpret_cast<const double*>(rec)[1], obj[idx], s);
+      const double m = reinterpret_cast<const double*>(rec)[1];
+      if (REPRO) {
+        const double hi = grid_round(m, obj[idx], gm);
+        s += hi;
+        s2 += grid_round(__fma_rn(m, obj[idx], -hi), 1.0, gm2);
+      } else {
+        s = fma(m, obj[idx], s);
+      }
     }
   }
   for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+  if (REPRO)
+    for (int o = 16; o > 0; o >>= 1) s2 += __shfl_down_sync(0xffffffffu, s2, o);
   if (lane == 0) out[warp] = s;
+  if (REPRO && lane == 0) out2[warp] = s2;
 }
 
 int cell_objective(basq_ctx* ctx, const RecPool& pool, int64_t off_glob, int S, int S_eff, const double* obj,
-                   double* out) {
+                   double* out, double grid_m, double grid_m2, double* out2) {
   const int threads = 256;
   const int blocks = ceil_div((int64_t)S * 32, threads);
-  cell_obj_kernel<<<blocks, threads, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
-                                                       pool.dtype == BASQ_F64 ? 1 : 0, pool.count, off_glob, S, S_eff,
-                                                       obj, out);
+  if (grid_m != 0.0)
+    cell_obj_kernel<true><<<blocks, threads, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
+                                                               pool.dtype == BASQ_F64 ? 1 : 0, pool.count, off_glob, S,
+                                                               S_eff, obj, out, grid_m, grid_m2, out2);
+  else
+    cell_obj_kernel<false><<<blocks, threads, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
+                                                                pool.dtype == BASQ_F64 ? 1 : 0, pool.count, off_glob, S,
+                                                                S_eff, obj, out, 0.0, 0.0, nullptr);
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
+  return BASQ_OK;
+}
+
+// Maxima over the live records of |wf|, |mu| and |mu obj[idx]| (obj may be NULL: 0), the inputs of the grids of
+// a reproducible pass.  out[3] must be zeroed; non-negative doubles order like their bit patterns.
+__global__ void record_maxima_kernel(const unsigned char* __restrict__ recs, int rec_bytes, int f64, int64_t count,
+                                     const double* __restrict__ obj, unsigned long long* __restrict__ out) {
+  // NaN inputs: fmax would drop them, so !(x <= m) takes them over; a NaN bound makes session_set_grid fail
+  auto take = [](double& m, double x) { if (!(x <= m)) m = x; };
+  double m[3] = {0.0, 0.0, 0.0};
+  for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < count; p += (int64_t)gridDim.x * blockDim.x) {
+    const unsigned char* rec = recs + p * rec_bytes;
+    const double* h = reinterpret_cast<const double*>(rec);
+    if (m[0] == m[0]) take(m[0], fabs(h[0]));
+    if (m[1] == m[1]) take(m[1], fabs(h[1]));
+    if (obj && m[2] == m[2]) {
+      const int64_t idx = f64 ? reinterpret_cast<const int64_t*>(rec)[2] : (int64_t) reinterpret_cast<const int*>(rec)[4];
+      take(m[2], fabs(h[1] * obj[idx]));
+    }
+  }
+  for (int i = 0; i < 3; ++i) {
+    // a NaN becomes the canonical quiet NaN, whose bit pattern exceeds every non-negative double's
+    double v = m[i] == m[i] ? m[i] : __longlong_as_double(0x7ff8000000000000ll);
+    for (int o = 16; o > 0; o >>= 1) {
+      const double u = __shfl_down_sync(0xffffffffu, v, o);
+      if (__double_as_longlong(u) > __double_as_longlong(v)) v = u;
+    }
+    if ((threadIdx.x & 31) == 0) atomicMax(out + i, (unsigned long long)__double_as_longlong(v));
+  }
+}
+
+int record_maxima(basq_ctx* ctx, const RecPool& pool, const double* obj, double* max_host) {
+  DevBuf d;
+  BASQ_TRY(d.alloc(ctx, 3 * sizeof(double)));
+  BASQ_CUDA(cudaMemsetAsync(d.p, 0, 3 * sizeof(double), ctx->stream));
+  if (pool.count > 0) {
+    const int blocks = (int)std::min<int64_t>(ceil_div64(pool.count, 256), 4 * (int64_t)ctx->num_sms);
+    record_maxima_kernel<<<blocks, 256, 0, ctx->stream>>>(pool.buf[pool.cur].as<unsigned char>(), pool.rec_bytes,
+                                                          pool.dtype == BASQ_F64 ? 1 : 0, pool.count, obj,
+                                                          d.as<unsigned long long>());
+    ctx->launches++;
+    BASQ_CUDA(cudaGetLastError());
+  }
+  BASQ_CUDA(cudaMemcpyAsync(max_host, d.p, 3 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  BASQ_CUDA(cudaStreamSynchronize(ctx->stream));
   return BASQ_OK;
 }
 

@@ -32,6 +32,9 @@ int set_sums(basq_ctx* ctx, const KParams& kp, const SetSumArgs& a) {
   dev.G = a.G;
   dev.ldg = a.ldg;
   dev.accumulate = a.accumulate ? 1 : 0;
+  dev.grid_m = a.grid_m;
+  dev.grid_m2 = a.grid_m2;
+  dev.G2 = a.G2;
   if (pool.dtype == BASQ_F32 && a.nl == NL_LIN && lm.lmA != nullptr) {
     // fp32 linear modes: argument tiles on the tensor cores (setsum_mma.cuh)
     SetSumMmaDev md;
@@ -48,6 +51,7 @@ int set_sums(basq_ctx* ctx, const KParams& kp, const SetSumArgs& a) {
     md.G = dev.G;
     md.ldg = dev.ldg;
     md.accumulate = dev.accumulate;
+    md.grid_m = a.grid_m;
     switch (kp.family) {
       case BASQ_RBF: return launch_setsum_mma_rbf(ctx, kp.dp, md);
       case BASQ_MATERN15: return launch_setsum_mma_m15(ctx, kp.dp, md);

@@ -35,6 +35,9 @@ struct SetSumDev {
   double* G;
   int64_t ldg;
   int accumulate;
+  double grid_m;  // reproducible instances: 1.5 * 2^52 * Q of the pass's grid Q (grid_round, common.cuh)
+  double grid_m2; // reproducible fp64 instances: the grid of the remainders term - hi, summed into G2
+  double* G2;
 };
 
 __device__ __forceinline__ void cp_async16_zfill(void* smem_dst, const void* gmem_src, bool valid) {
@@ -63,7 +66,8 @@ struct SetSumCfg {
   static constexpr int SMEM_BYTES = NSTAGE * STAGE_BYTES;
 };
 
-template <typename T, int FAM, int DP, bool NONLIN>
+// REPRO: every term is rounded to the pass's grid before it is added (see setsum_mma.cuh)
+template <typename T, int FAM, int DP, bool NONLIN, bool REPRO>
 __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
   using Cfg = SetSumCfg<T, DP>;
   constexpr int TM = Cfg::TM, JT = Cfg::JT, EC = Cfg::EC, NSTAGE = Cfg::NSTAGE, RB = Cfg::RB;
@@ -93,11 +97,26 @@ __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
     }
   }
 
+  // fp64 inputs in reproducible instances: two grids, so that the fp64 accuracy of the terms survives - acc sums
+  // the terms rounded to the grid of grid_m, acc2 their remainders rounded to the finer grid of grid_m2
+  constexpr bool TWO = REPRO && sizeof(T) == 8;
   double acc[TM][JT];
+  double acc2[TWO ? TM : 1][TWO ? JT : 1];
 #pragma unroll
   for (int t = 0; t < TM; ++t)
 #pragma unroll
     for (int jj = 0; jj < JT; ++jj) acc[t][jj] = 0.0;
+#pragma unroll
+  for (int t = 0; t < (TWO ? TM : 1); ++t)
+#pragma unroll
+    for (int jj = 0; jj < (TWO ? JT : 1); ++jj) acc2[t][jj] = 0.0;
+  // term a * b on the two grids
+  // (the remainder x y - hi is below Q / 2 and is rounded once by the fma)
+  auto add2 = [&](int t, int jj, double x, double y) {
+    const double hi = grid_round(x, y, a.grid_m);
+    acc[t][jj] += hi;
+    if constexpr (TWO) acc2[t][jj] += grid_round(__fma_rn(x, y, -hi), 1.0, a.grid_m2);
+  };
 
   // ---- member range of this CTA: local p = j + e*S - off  in [p_lo, p_hi)
   const int64_t S = a.S;
@@ -158,7 +177,8 @@ __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
 #pragma unroll
             for (int t = 0; t < TM; ++t) {
               const float k = pair_eval_f32<FAM, DP>(&f[2], pa, reinterpret_cast<const float*>(zreg[t]), breg[t], a.os_f);
-              acc[t][jj] = fma(f2d_pos(k), hw.x, acc[t][jj]);
+              if (REPRO) add2(t, jj, f2d_pos(k), hw.x);
+              else acc[t][jj] = fma(f2d_pos(k), hw.x, acc[t][jj]);
             }
           } else {
             const int64_t e = e_lo + c * EC + ei;
@@ -172,7 +192,8 @@ __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
                 if (m < a.Mtot) {
                   const float k = pair_eval_f32<FAM, DP>(&f[2], pa, reinterpret_cast<const float*>(zreg[t]), breg[t], a.os_f);
                   const double cv = f2d_pos(k) - crow[m];
-                  acc[t][jj] = fma(nl_apply(a.nl, cv, szreg[t], hw.x), hw.y, acc[t][jj]);
+                  if (REPRO) add2(t, jj, nl_apply(a.nl, cv, szreg[t], hw.x), hw.y);
+                  else acc[t][jj] = fma(nl_apply(a.nl, cv, szreg[t], hw.x), hw.y, acc[t][jj]);
                 }
               }
             }
@@ -190,7 +211,8 @@ __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
 #pragma unroll
             for (int t = 0; t < TM; ++t) {
               const double k = pair_eval_f64<FAM, DP>(&g[1], reinterpret_cast<const double*>(zreg[t]), a.os_d);
-              acc[t][jj] = fma(k, hw.x, acc[t][jj]);
+              if (REPRO) add2(t, jj, k, hw.x);
+              else acc[t][jj] = fma(k, hw.x, acc[t][jj]);
             }
           } else {
             const int64_t e = e_lo + c * EC + ei;
@@ -204,7 +226,8 @@ __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
                 if (m < a.Mtot) {
                   const double k = pair_eval_f64<FAM, DP>(&g[1], reinterpret_cast<const double*>(zreg[t]), a.os_d);
                   const double cv = k - crow[m];
-                  acc[t][jj] = fma(nl_apply(a.nl, cv, szreg[t], hw.x), hw.y, acc[t][jj]);
+                  if (REPRO) add2(t, jj, nl_apply(a.nl, cv, szreg[t], hw.x), hw.y);
+                  else acc[t][jj] = fma(nl_apply(a.nl, cv, szreg[t], hw.x), hw.y, acc[t][jj]);
                 }
               }
             }
@@ -226,6 +249,10 @@ __global__ void __launch_bounds__(128) setsum_kernel(const SetSumDev a) {
       if (j >= a.S) continue;
       double* dst = a.G + (int64_t)m * a.ldg + j;
       *dst = a.accumulate ? (*dst + acc[t][jj]) : acc[t][jj];
+      if constexpr (TWO) {
+        double* dst2 = a.G2 + (int64_t)m * a.ldg + j;
+        *dst2 = a.accumulate ? (*dst2 + acc2[t][jj]) : acc2[t][jj];
+      }
     }
   }
 }
@@ -236,10 +263,15 @@ int launch_setsum_dp(basq_ctx* ctx, const SetSumDev& dev) {
   using Cfg = SetSumCfg<T, DP>;
   dim3 grid((unsigned)ceil_div(dev.Mtot, Cfg::THREADS * Cfg::TM), (unsigned)ceil_div(dev.S, Cfg::JT));
   BASQ_CHECK(grid.y <= 65535, BASQ_ERR_UNSUPPORTED, "set_sums: %d sets exceed the grid limit", dev.S);
-  if (dev.nl == NL_LIN)
-    setsum_kernel<T, FAM, DP, false><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+  const bool repro = dev.grid_m != 0.0;
+  if (dev.nl == NL_LIN && !repro)
+    setsum_kernel<T, FAM, DP, false, false><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+  else if (!repro)
+    setsum_kernel<T, FAM, DP, true, false><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+  else if (dev.nl == NL_LIN)
+    setsum_kernel<T, FAM, DP, false, true><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
   else
-    setsum_kernel<T, FAM, DP, true><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+    setsum_kernel<T, FAM, DP, true, true><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
   return BASQ_OK;

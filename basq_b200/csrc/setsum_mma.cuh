@@ -50,6 +50,7 @@ struct SetSumMmaDev {
   double* G;
   int64_t ldg;
   int accumulate;
+  double grid_m;     // reproducible instances: 1.5 * 2^52 * Q of the pass's grid Q (grid_round, common.cuh)
 };
 
 template <int DP>
@@ -258,7 +259,9 @@ __global__ void build_lmA_kernel(const float* __restrict__ zz, const float* __re
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
-template <int FAM, int DP>
+// REPRO: every term w_p k is rounded to the pass's grid before it is added, so that the sums are exact and do
+// not depend on the tiling or on how the points are split over ranks (DESIGN.md, reproducible mode)
+template <int FAM, int DP, bool REPRO>
 __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(const SetSumMmaDev a) {
   using Cfg = MmaCfg<DP>;
   constexpr int KA = Cfg::KA, NT = Cfg::NT, MT = Cfg::MT, JT = Cfg::JT, EC = Cfg::EC, NSTAGE = Cfg::NSTAGE,
@@ -365,10 +368,17 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
                 const float u11 = __uint_as_float(h ? vb[4 * k + 3] : va[4 * k + 3]);
                 const float k00 = finish_f32(FAM, u00, a.os_f), k01 = finish_f32(FAM, u01, a.os_f);
                 const float k10 = finish_f32(FAM, u10, a.os_f), k11 = finish_f32(FAM, u11, a.os_f);
-                acc[mt][2 * h][0] = fma(f2d_pos(k00), w2.x, acc[mt][2 * h][0]);
-                acc[mt][2 * h][1] = fma(f2d_pos(k01), w2.y, acc[mt][2 * h][1]);
-                acc[mt][2 * h + 1][0] = fma(f2d_pos(k10), w2.x, acc[mt][2 * h + 1][0]);
-                acc[mt][2 * h + 1][1] = fma(f2d_pos(k11), w2.y, acc[mt][2 * h + 1][1]);
+                if (REPRO) {
+                  acc[mt][2 * h][0] += grid_round(f2d_pos(k00), w2.x, a.grid_m);
+                  acc[mt][2 * h][1] += grid_round(f2d_pos(k01), w2.y, a.grid_m);
+                  acc[mt][2 * h + 1][0] += grid_round(f2d_pos(k10), w2.x, a.grid_m);
+                  acc[mt][2 * h + 1][1] += grid_round(f2d_pos(k11), w2.y, a.grid_m);
+                } else {
+                  acc[mt][2 * h][0] = fma(f2d_pos(k00), w2.x, acc[mt][2 * h][0]);
+                  acc[mt][2 * h][1] = fma(f2d_pos(k01), w2.y, acc[mt][2 * h][1]);
+                  acc[mt][2 * h + 1][0] = fma(f2d_pos(k10), w2.x, acc[mt][2 * h + 1][0]);
+                  acc[mt][2 * h + 1][1] = fma(f2d_pos(k11), w2.y, acc[mt][2 * h + 1][1]);
+                }
               }
             }
           }
@@ -599,8 +609,8 @@ __global__ void __launch_bounds__(MmaCfg<DP>::THREADS, 1) setsum_mma_kernel(cons
   }
 }
 
-template <int FAM, int DP>
-int launch_setsum_mma_dp(basq_ctx* ctx, SetSumMmaDev dev) {
+template <int FAM, int DP, bool REPRO>
+int launch_setsum_mma_inst(basq_ctx* ctx, SetSumMmaDev dev) {
   using Cfg = MmaCfg<DP>;
   dev.n_mgroups = ceil_div(dev.Mtot, Cfg::MT * 128);
   dev.n_jgroups = ceil_div(dev.S, Cfg::JT);
@@ -608,13 +618,18 @@ int launch_setsum_mma_dp(basq_ctx* ctx, SetSumMmaDev dev) {
   BASQ_CHECK(n_items < (1ll << 31), BASQ_ERR_UNSUPPORTED, "set_sums: too many work items");
   BASQ_CHECK((size_t)Cfg::SMEM_BYTES <= ctx->smem_optin, BASQ_ERR_UNSUPPORTED,
              "set_sums: kernel needs %d B shared memory (limit %zu)", Cfg::SMEM_BYTES, ctx->smem_optin);
-  BASQ_CUDA(cudaFuncSetAttribute(setsum_mma_kernel<FAM, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  BASQ_CUDA(cudaFuncSetAttribute(setsum_mma_kernel<FAM, DP, REPRO>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  Cfg::SMEM_BYTES));
   const int grid = (int)std::min<int64_t>(ctx->num_sms, n_items);
-  setsum_mma_kernel<FAM, DP><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
+  setsum_mma_kernel<FAM, DP, REPRO><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, ctx->stream>>>(dev);
   ctx->launches++;
   BASQ_CUDA(cudaGetLastError());
   return BASQ_OK;
+}
+
+template <int FAM, int DP>
+int launch_setsum_mma_dp(basq_ctx* ctx, const SetSumMmaDev& dev) {
+  return dev.grid_m != 0.0 ? launch_setsum_mma_inst<FAM, DP, true>(ctx, dev) : launch_setsum_mma_inst<FAM, DP, false>(ctx, dev);
 }
 
 template <int FAM>

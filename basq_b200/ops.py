@@ -284,6 +284,15 @@ def stage_candidates(X_host, mu_host=None, device="cuda"):
     return len(X_host), X_host.dtype
 
 
+def reproducible(on: bool, device=None):
+    """Switch the reproducible mode of the context on `device`'s current stream (basq_ctx_reproducible): sessions
+    created afterwards - recombine, recombine_host, Session, recombination_sharded - sum on a power-of-two grid,
+    so that one GPU and any number of ranks with any split of the candidates return the same (idx, w) bit for bit.
+    Results differ from the default mode's by the grid rounding (DESIGN.md)."""
+    dev = torch.device(device if device is not None else "cuda")
+    _lib.context_for(dev).reproducible(on)
+
+
 class Session:
     """Staged recombination over a rank-local shard (basq_session_* in the C ABI)."""
 
@@ -323,10 +332,15 @@ class Session:
         if obj_loc is not None:
             objd = _prep(obj_loc, device, torch.float64)
             assert objd.shape == (n_loc,)
+            if n_loc == 0:      # an empty shard still carries the objective row: NULL would switch it off
+                objd = torch.zeros(1, dtype=torch.float64, device=device)
             self._keep.append(objd)
             _lib.check(_lib.lib.basq_session_set_objective(h, objd.data_ptr()))
             self.rows = self.n + 1
         self.has_obj = obj_loc is not None
+        on = C.c_int(0)
+        _lib.check(_lib.lib.basq_session_reproducible(h, C.byref(on)))
+        self.reproducible = bool(on.value)
 
     def close(self):
         h, self.handle = getattr(self, "handle", None), None
@@ -396,6 +410,35 @@ class Session:
         _lib.check(_lib.lib.basq_session_level_project(self.handle, int(lvl), K, nd.ctypes.data, pp.ctypes.data,
                                                        fp.ctypes.data, Gf_rows.data_ptr(), K, int(row0), int(nrows),
                                                        A.data_ptr()))
+
+    # --- reproducible sessions: grids per pass, grid-exact columns summed over the ranks, full projection --------
+    def grid_maxima(self) -> np.ndarray:
+        """This rank's maxima of |wf|, |mu|, |mu obj| over its live points (basq_session_grid_maxima)."""
+        mx = np.zeros(3, dtype=np.float64)
+        _lib.check(_lib.lib.basq_session_grid_maxima(self.handle, mx.ctypes.data))
+        return mx
+
+    def set_grid(self, R_glob, maxima):
+        mx = np.ascontiguousarray(maxima, dtype=np.float64)
+        _lib.check(_lib.lib.basq_session_set_grid(self.handle, int(R_glob), mx.ctypes.data))
+
+    def level_fold_exact(self, lvl, node, Gf: torch.Tensor):
+        """This rank's grid-exact columns of the level, Gf [2 (Mtot + 2), K]: set sums, masses, objective sums on the
+        pass's grids, then the sums of their remainders on the finer grids (basq_session_level_fold_exact)."""
+        K = len(node)
+        assert Gf.dtype == torch.float64 and Gf.is_contiguous() and Gf.numel() >= 2 * (self.landmarks() + 2) * K
+        nd = np.ascontiguousarray(node, dtype=np.int32)
+        _lib.check(_lib.lib.basq_session_level_fold_exact(self.handle, int(lvl), K, nd.ctypes.data, Gf.data_ptr(), K))
+
+    def level_project_exact(self, lvl, node, ppos, fpar, Gf: torch.Tensor, A: torch.Tensor):
+        """Level system A [rows, S] from the columns of level_fold_exact summed over every rank."""
+        assert A.dtype == torch.float64 and A.is_contiguous() and A.shape == (self.rows, self.S)
+        K = len(node)
+        nd = np.ascontiguousarray(node, dtype=np.int32)
+        pp = np.ascontiguousarray(ppos if lvl > 0 else np.zeros(K), dtype=np.int32)
+        fp = np.ascontiguousarray(fpar, dtype=np.float64)
+        _lib.check(_lib.lib.basq_session_level_project_exact(self.handle, int(lvl), K, nd.ctypes.data, pp.ctypes.data,
+                                                             fp.ctypes.data, Gf.data_ptr(), K, A.data_ptr()))
 
     def car(self, A: torch.Tensor, C_cols: int, omega: torch.Tensor):
         if self.has_obj:

@@ -140,6 +140,21 @@ class ShardEngine:
         _lib.check(_lib.lib.basq_weights_sum(self.ctx.handle, w.data_ptr(), w.numel(), C.byref(out)))
         return float(out.value)
 
+    @property
+    def reproducible(self) -> bool:
+        return self.ctx.is_reproducible
+
+    def weights_max(self, w) -> float:
+        out = C.c_double(0.0)
+        _lib.check(_lib.lib.basq_weights_max(self.ctx.handle, w.data_ptr(), w.numel(), C.byref(out)))
+        return float(out.value)
+
+    def weights_sum_grid(self, w, wmax, N_glob) -> np.ndarray:
+        hilo = np.zeros(2, dtype=np.float64)
+        _lib.check(_lib.lib.basq_weights_sum_grid(self.ctx.handle, w.data_ptr(), w.numel(), float(wmax), int(N_glob),
+                                                  hilo.ctypes.data))
+        return hilo
+
     def weights_normalise(self, w, total, N_glob):
         _lib.check(_lib.lib.basq_weights_normalise(self.ctx.handle, w.data_ptr(), w.numel(), float(total), int(N_glob)))
 

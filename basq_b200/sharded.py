@@ -10,8 +10,14 @@ so the collectives on the data path are that all-reduce (SURVEY 8e) and, under N
 reduce-scatter of the level's folded set-sum columns by landmark rows in front of it, which lets
 every rank project 1/G of the rows instead of repeating the whole fp64 projection.
 
+Reproducible sessions (ops.reproducible) take another route to the same rule on any number of ranks: every
+term of the cell sums is rounded to a power-of-two grid fixed per pass from maxima over every rank (one
+all-reduce MAX of three numbers), so the ranks' grid-exact level columns sum exactly, in any order; after one
+all-reduce of those columns every rank projects all of them, as one GPU does, and no sum of A follows.
+
 The loop is written against a tiny engine interface so the host logic can be exercised on CPU with
-gloo and an oracle-backed engine (tests/test_sharded_gloo.py); the product engine is ops.Session.
+gloo and an oracle-backed engine (tests/test_sharded_gloo.py, tests/test_reproducible_gloo.py); the product
+engine is ops.Session.
 """
 from __future__ import annotations
 
@@ -79,7 +85,11 @@ def recombine_sharded(engine, n, S, group=None, device=None, max_rounds=256):
 
     A pass over F*S cells (cell = global position mod F*S, set j = cells j, j+S, ...) costs ONE
     sweep of kernel evaluations; each of its log2(F)+1 Caratheodory levels all-reduces one small
-    [n, S] system, and the candidates shrink by 2F."""
+    [n, S] system, and the candidates shrink by 2F.
+
+    An engine with `reproducible` set takes the exact branch: grid_maxima / set_grid before every pass
+    (all-reduce MAX), and per level level_fold_exact, an all-reduce of the [2 (Mtot + 2), K] grid-exact columns
+    and level_project_exact on every rank - the same bits as one GPU for any world size and split."""
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     device = device if device is not None else getattr(engine, "device", "cpu")
@@ -92,6 +102,11 @@ def recombine_sharded(engine, n, S, group=None, device=None, max_rounds=256):
     # BASQ_SHARE_PROJECTION=0 keeps every rank projecting its own cell sums.
     share_projection = (world > 1 and hasattr(engine, "level_fold") and dist.get_backend(group) == "nccl"
                         and os.environ.get("BASQ_SHARE_PROJECTION", "1") != "0")
+    exact = bool(getattr(engine, "reproducible", False))
+    if exact:
+        share_projection = False
+        Gx = torch.zeros(2 * (engine.landmarks() + 2) * S, dtype=torch.float64, device=device)
+        nccl = world > 1 and dist.get_backend(group) == "nccl"
     A = torch.zeros(getattr(engine, "rows", n), S, dtype=torch.float64, device=device)   # n + 1 rows with an objective
     omega = torch.zeros(S, dtype=torch.float64, device=device)
     rounds = 0
@@ -103,13 +118,27 @@ def recombine_sharded(engine, n, S, group=None, device=None, max_rounds=256):
         off = sum(counts[:rank])
         F = engine.cell_factor(R, max(counts))          # same inputs on every rank -> same F
         cells = F * S
+        if exact:
+            mx = torch.from_numpy(np.asarray(engine.grid_maxima(), dtype=np.float64).copy())
+            if world > 1:
+                mx = mx.to(device) if nccl else mx
+                dist.all_reduce(mx, op=dist.ReduceOp.MAX, group=group)
+            engine.set_grid(R, mx.cpu().numpy())
         engine.pass_begin(R, off, F)
         factor = torch.zeros(cells, dtype=torch.float64)
         tree = LevelTree(S, F, R)
         while True:
             C = tree.columns()
             if C > n or tree.lvl < tree.L:
-                if share_projection:
+                if exact:
+                    # grid-exact columns: their sum over the ranks is exact in any order
+                    K = len(tree.node)
+                    Gv = Gx[: (Gx.numel() // S) * K]
+                    engine.level_fold_exact(tree.lvl, tree.node, Gv)
+                    if world > 1:
+                        dist.all_reduce(Gv, group=group)
+                    engine.level_project_exact(tree.lvl, tree.node, tree.ppos, tree.fpar, Gv, A)
+                elif share_projection:
                     # fold locally, reduce-scatter the folded columns by landmark rows, project 1/world
                     # of the rows here; the all-reduce of A below completes the sum over row blocks
                     K = len(tree.node)
@@ -123,7 +152,7 @@ def recombine_sharded(engine, n, S, group=None, device=None, max_rounds=256):
                 else:
                     engine.level(tree.lvl, tree.node, tree.ppos, tree.fpar, A)
             if C > n:
-                if world > 1:
+                if world > 1 and not exact:
                     dist.all_reduce(A, group=group)
                 engine.car(A, C, omega)                   # identical system -> identical factors on every rank
                 om = omega[:C].cpu().numpy()
@@ -371,7 +400,19 @@ def _fold_sum(x, group, device):
 
 
 def _normalised(eng, w, N_glob, group):
-    eng.weights_normalise(w, _fold_sum(eng.weights_sum(w), group, w.device), N_glob)
+    if getattr(eng, "reproducible", False):
+        # grid-exact totals: the grids from the maximum over every rank (exact), hi and lo sums exact in any order,
+        # one fixed rounding hi + lo - the total of basq_candidate_weights / basq_cleanse_weights on one GPU
+        on, _, _, nccl = _ranks(group)
+        mx = torch.tensor([eng.weights_max(w)], dtype=torch.float64)
+        if on:
+            mx = mx.to(w.device) if nccl else mx
+            dist.all_reduce(mx, op=dist.ReduceOp.MAX, group=group)
+        hl = eng.weights_sum_grid(w, float(mx.item()), N_glob)
+        total = _fold_sum(hl[0], group, w.device) + _fold_sum(hl[1], group, w.device)
+    else:
+        total = _fold_sum(eng.weights_sum(w), group, w.device)
+    eng.weights_normalise(w, total, N_glob)
     return w
 
 

@@ -114,6 +114,16 @@ int basq_ctx_conditioning(basq_ctx* ctx, double kappa_max, double* last_kappa_ho
    BASQ_F64_EVAL_F32=1).  on < 0 leaves the setting unchanged; demotions_host (may be NULL) receives the
    number of sessions demoted so far. */
 int basq_ctx_allow_f32_eval(basq_ctx* ctx, int on, int64_t* demotions_host);
+/* Reproducible mode: with on != 0, sessions created afterwards (basq_recombine*, basq_session_create*) sum on a
+   power-of-two grid - every term w_p k(z_m, x_p), mass and objective term is rounded to a grid Q before it is added,
+   so that every set sum, fold and sum over ranks is exact - and project each level from the columns summed over
+   every rank.  Given the same X (as global rows), Z, U, mu, obj and descriptor, basq_recombine on one GPU and the
+   sharded loop (basq_session_set_grid, basq_session_level_fold_exact, basq_session_level_project_exact) over any
+   number of ranks and any contiguous split then return bit-identical idx and w.  It costs one extra add per term
+   and a synchronising reduction per pass; results differ from the default mode's by the grid rounding (DESIGN.md).
+   Default off; on < 0 leaves the setting unchanged.  Does not apply to basq_gram, basq_features, basq_gp_predict,
+   basq_kernel_quadform or basq_kernel_bilinear. */
+int basq_ctx_reproducible(basq_ctx* ctx, int on);
 /* Key of the library's own Gaussian draws (the Nystrom test matrix when the caller passes none); the
    k-th draw after this call uses the Philox key seed + k.  Default 0. */
 int basq_ctx_set_seed(basq_ctx* ctx, uint64_t seed);
@@ -290,6 +300,23 @@ int basq_session_level_fold(basq_session* s, int lvl, int K, const int* node_hos
 int basq_session_level_project(basq_session* s, int lvl, int K, const int* node_host, const int* ppos_host,
                                const double* fpar_host, const double* Gf_rows, int64_t ld_gf, int row0,
                                int nrows, double* A_out);
+/* Reproducible sessions (basq_ctx_reproducible at creation; *on_host = 1).  Before every pass_begin:
+   basq_session_grid_maxima writes max_host[3] = this rank's maxima over its live points of |wf|, |mu| and
+   |mu obj| (synchronises); the caller takes the element-wise maximum over the ranks and hands it to
+   basq_session_set_grid with the pass's R_glob on every rank, which fixes the pass's grids.  The cell factor
+   then depends on R_glob alone.  Per level, fold_exact writes this rank's grid-exact columns Gf_out[2 (Mtot + 2), K]
+   (ld = ld_gf): rows 0 .. Mtot-1 the folded set sums, row Mtot the masses, row Mtot + 1 the objective sums, and
+   rows Mtot + 2 .. 2 Mtot + 3 the same for the remainders of the fp64 terms on finer grids (zero for the set sums
+   of fp32 inputs); the caller sums them over the ranks in fp64 (exact in any order) and project_exact builds the
+   whole level system A_out[rows, S] from hi + lo of the summed columns on every rank - no sum of A follows.  basq_session_level on a
+   reproducible session does both for one rank. */
+int basq_session_reproducible(const basq_session* s, int* on_host);
+int basq_session_grid_maxima(basq_session* s, double* max_host);
+int basq_session_set_grid(basq_session* s, int64_t R_glob, const double* max_host);
+int basq_session_level_fold_exact(basq_session* s, int lvl, int K, const int* node_host, double* Gf_out,
+                                  int64_t ld_gf);
+int basq_session_level_project_exact(basq_session* s, int lvl, int K, const int* node_host, const int* ppos_host,
+                                     const double* fpar_host, const double* Gf, int64_t ld_gf, double* A_out);
 /* Rescale the kept cells by factor_host[F*S] (HOST; product of the level factors along each cell's
    path, 0 = dropped), drop the rest, compact.  New local count out. */
 int basq_session_apply_cells(basq_session* s, int64_t R_glob, int64_t off_glob, int F,
@@ -339,6 +366,15 @@ int basq_sir_resample(basq_ctx* ctx, const double* w, int64_t N, int64_t n_out, 
 int basq_weights_sum(basq_ctx* ctx, const double* w, int64_t N, double* total_host);
 int basq_weights_normalise(basq_ctx* ctx, double* w, int64_t N_loc, double total, int64_t N_glob);
 int basq_weights_cleanse(basq_ctx* ctx, double* w, int64_t N, double eps);
+/* Reproducible totals (basq_ctx_reproducible).  On one GPU, basq_candidate_weights(normalise = 1) and
+   basq_cleanse_weights divide by the total of basq_weights_sum_grid(w, N, max|w|, N), computed as hi + lo.  Over
+   ranks: basq_weights_max gives this rank's max |w[N]| (a NaN wins; 0 for N = 0; synchronises).  The caller takes
+   the maximum over the ranks, and basq_weights_sum_grid writes hilo_host[2], the sums of this rank's weights on the
+   two grids fixed by that maximum and N_glob.  Both sums are exact.  Their sums over the ranks, added as
+   total = hi + lo, give the one-GPU total bit for bit: pass it to basq_weights_normalise.  A non-finite wmax gives
+   a non-finite total. */
+int basq_weights_max(basq_ctx* ctx, const double* w, int64_t N, double* max_host);
+int basq_weights_sum_grid(basq_ctx* ctx, const double* w, int64_t N, double wmax, int64_t N_glob, double* hilo_host);
 /* The race of basq_sir_resample over a sharded set, selected exactly on the device.
    keys: keys_out[N_loc] = the bits (as uint64) of key_i = -log(u(seed; idx_base + i)) / w_i, the key
          basq_sir_resample gives global row idx_base + i; rows without a key (!(w_i > 0), or a key of +inf,
